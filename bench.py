@@ -26,6 +26,10 @@ through enough distinct input batches that the footprint exceeds 2x L2 (126 MB).
 The `e2e` leg calls go1mpc_control_tick_host_async with pinned HOST buffers (H2D of the tick's
 arguments, both ticks, compact result rows) and, for N > 1, gathers the result rows of every rank to
 rank 0 over NCCL once per batch; rank 0 reads the gathered rows back to host memory.
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) so that two builds can be compared
+output for output: the inputs depend only on the arguments.  The run writes nothing else to disk outside a
+temporary directory, so it can run from a read-only tree.
 """
 import argparse
 import ctypes
@@ -40,6 +44,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # no __pycache__ in the tree the bench runs from
 
 METRIC = "batched MPC QP solves/sec"
 UNIT = "solves/s"
@@ -70,7 +75,33 @@ def parse():
                     help="e2e, N > 1: how the result rows reach rank 0 -- NVLink peer-memory stores + flags (csrc/peer_gather.cu) or torch.distributed.gather")
     ap.add_argument("--e2e-no-graph", action="store_true", help="e2e: enqueue every step's calls from the host instead of replaying one captured graph per batch slot")
     ap.add_argument("--e2e-no-gather", action="store_true", help="DIAGNOSTIC: leave the gather to rank 0 out of the e2e leg (the number is then not the e2e metric)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float64; a fixed sample of the robots when "
+                         "they exceed 64 MB)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
+    return a
+
+
+DUMP_BYTES = 63 * 10 ** 6      # --dump-outputs: data of all files of all ranks, under 64 MB with the .npy headers
+DUMP_SEED = 0xB2000D
+
+
+def dump_outputs(path, rows, first, budget, suffix=""):
+    """Writes the per-robot results of one step, rows = {name: [B, k] host array}, as path/<name><suffix>.npy in float64
+    (the int diagnostics convert exactly), plus robot<suffix>.npy: the robots' indices in the global batch (first = index
+    of row 0).  All B robots when they fit in `budget` bytes, else a sorted sample drawn with the fixed DUMP_SEED."""
+    B = len(next(iter(rows.values())))
+    per_robot = 8 * (1 + sum(v.shape[1] for v in rows.values()))
+    n = min(B, budget // per_robot)
+    idx = np.arange(B) if n == B else np.sort(np.random.default_rng(DUMP_SEED).choice(B, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"robot{suffix}.npy"), (first + idx).astype(np.float64))
+    for name, v in rows.items():
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), np.ascontiguousarray(v[idx], dtype=np.float64))
 
 
 def shard_range(B, rank, world):
@@ -197,7 +228,7 @@ def run_reference(a):
         return
     cores = os.cpu_count() or 1
     run, solves, close, B = cpu_pool(a, cores)
-    steps = min(a.steps, 200)
+    steps = a.steps
     W = min(max(a.warmup, 1), 5)
     run(W)
     times = [run(1) for _ in range(steps)]
@@ -437,6 +468,15 @@ def run_b200(a):
     e1.synchronize()
     torch.cuda.synchronize()
     barrier()
+    if a.dump_outputs:
+        # what the caller of both ticks receives from the last timed step (K - 1: slot r on lane ln), taken before the legs
+        # below overwrite those buffers: body output records and diagnostics [B, stride], planner Vec38, state after the tick
+        # and diagnostics (transposed from the planner's field-major layout to [B, fields])
+        r, ln = (K - 1) % nrot, (K - 1) % L
+        dump_outputs(a.dump_outputs, {"body_out": out_d[r].cpu().numpy(), "body_diag": diag_d[r].cpu().numpy(),
+                                      "step_out": so_d[r].cpu().numpy().T, "step_state": st_w[ln].cpu().numpy().T,
+                                      "step_diag": sd_d[r].cpu().numpy().T},
+                     lo if p["name"] == "cfg3" else rank * B, DUMP_BYTES // world, "" if world == 1 else f"_rank{rank}")
     launches = (mpc.launch_count - l0) if a.no_graph else launches_per_K
     total_ms = e0.elapsed_time(e1)
     solves_timed = float(sum(B + sqp_solves[i % nrot] for i in range(K)))
@@ -501,7 +541,7 @@ def run_b200(a):
     e2e = None
     if not a.no_e2e:
         from quadrupedal_loco_b200 import sharding
-        Ke = min(K, 200)
+        Ke = K
         Le = min(L, 4)
         CD = q.COMPACT_DOUBLES
         tx_np, xw_np, tick_np = q.split_body_record(nh, rec.reshape(nrot * B, in_s))

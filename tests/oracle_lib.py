@@ -3,7 +3,9 @@ reference build (oracle/_ref/*.so).  Test infrastructure: nothing in the product
 package imports this module."""
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -47,15 +49,24 @@ STEP_STATE, STEP_IN, STEP_OUT = 202, 20, 38
 
 
 def build_oracle(fast=False):
-    """liboracle.so: -O2 -ffp-contract=off (the checker).  fast=True: liboracle_fast.so, the same
-    sources at -O3 -march=native for the CPU-baseline timing; always rebuilt on the machine that
-    times it (it is never shipped: -march=native code may not run elsewhere)."""
-    name = "liboracle_fast.so" if fast else "liboracle.so"
-    so = os.path.join(ORC_DIR, name)
+    """liboracle.so: -O2 -ffp-contract=off (the checker), built in oracle/ when missing or older than its
+    sources.  fast=True: liboracle_fast.so, the same sources at -O3 -march=native for the CPU-baseline
+    timing, always built afresh on the machine that times it (-march=native code may not run elsewhere)
+    and into a new temporary directory (the tree may be read-only there); the caller removes it."""
+    env = {k: v for k, v in os.environ.items() if k not in ("CC", "CXX")}
+    if fast:
+        tmp = tempfile.mkdtemp(prefix="go1mpc_oracle_")
+        so = os.path.join(tmp, "liboracle_fast.so")
+        try:
+            subprocess.run(["make", "-s", "-C", ORC_DIR, f"FAST_SO={so}", so], check=True, env=env, capture_output=True)
+        except BaseException:
+            shutil.rmtree(tmp, ignore_errors=True)
+            raise
+        return so
+    so = os.path.join(ORC_DIR, "liboracle.so")
     srcs = [os.path.join(ORC_DIR, f) for f in os.listdir(ORC_DIR) if f.endswith((".c", ".h"))]
-    if fast or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        env = {k: v for k, v in os.environ.items() if k not in ("CC", "CXX")}
-        subprocess.run(["make", "-B" if fast else "-s", "-C", ORC_DIR, name], check=True, env=env, capture_output=True)
+    if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
+        subprocess.run(["make", "-s", "-C", ORC_DIR, "liboracle.so"], check=True, env=env, capture_output=True)
     return so
 
 
@@ -66,7 +77,10 @@ def ref_path(name):
 
 class Oracle:
     def __init__(self, fast=False):
-        self.lib = ctypes.CDLL(build_oracle(fast))
+        so = build_oracle(fast)
+        self.lib = ctypes.CDLL(so)
+        if fast:
+            shutil.rmtree(os.path.dirname(so))      # the loaded library stays mapped
 
     def qp_solve(self, n, p, m, G, g0, CE, ce0, CI, ci0, x0=None):
         """Column-major flat inputs for ONE problem.  Returns dict."""
