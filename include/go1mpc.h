@@ -631,6 +631,54 @@ int go1mpc_rt_node_tick_msgs_batch(go1mpc_t *h, int nh, int B, double *state_d, 
 int go1mpc_rt_node_tick_batch_host(go1mpc_t *h, int nh, int B, double *state, const double *msg, const int *ctrl,
                                    const double *bodyangle_state, double *body_out, double *out100);
 
+/* ---------------------------------------------------------------------------
+ * Gait stack tick: both nodes above behind ONE host call per 100 Hz tick for B robots that share one clock -- the call a
+ * controller farm makes every 10 ms.  The sensor slots the nodes read go up, the result slots the servo consumes come down;
+ * everything the reference keeps as node members (and both nodes' messages) stays in HBM, in one SoA state [row][B]:
+ *   [GO1MPC_STACK_ROW_NLP, +go1mpc_nlp_node_state_doubles())   the planner node's state
+ *   [GO1MPC_STACK_ROW_GAIT, +100)      /MPC/Gait                  [GO1MPC_STACK_ROW_RT2NRT, +25)  /rt2nrt/state
+ *   GO1MPC_STACK_ROW_WALKDTIME         the planner's tick counter walkdtime (exact integer)
+ *   [GO1MPC_STACK_ROW_TRAJ, +100)      /rtMPC/traj                [GO1MPC_STACK_ROW_RT, +go1mpc_rt_node_state_doubles(nh))  the 100 Hz node
+ * go1mpc_gait_stack_default_state gives one robot's initial column; a robot is reset by rewriting its column, a batch is
+ * checkpointed by a memcpy.  One call enqueues on `stream`:
+ *   1. H2D of sensor (and, when planner = 1, of cmd / start if given)
+ *   2. planner = 1: walkdtime += 1, then go1mpc_nlp_node_tick_batch on the state with rfoot_fb / lfoot_fb = rows 22..24 / 19..21
+ *      of the resident /rt2nrt/state (the foot feedback the previous fast tick forwarded, as the reference's ROS graph wires it)
+ *   3. the sensor rows into their slots of a /control2rtmpc/state buffer (its other 14 slots 0), then
+ *      go1mpc_rt_node_tick_msgs_batch writing /rtMPC/traj and /rt2nrt/state into the state
+ *   4. the n_slots selected slots of both messages -> rows_d [B][n_slots]; D2H into rows when given
+ * Results are bit-identical to calling the two node entries in that order.  The reference's clock (planner every 25 ms,
+ * fast node every 10 ms): the fast tick at 10k ms sets planner = 1 when a multiple of 25 lies in (10(k-1), 10k], k = 0, 3, 5,
+ * 8, 10, ...  The body-MPC input records and all staging are per-stream workspace owned by the handle, allocated on the
+ * first call with a given (stream, B): later calls with that pair allocate nothing, so a warmed-up schedule can be captured
+ * with go1mpc_graph_capture_*.  Host buffers should be pinned and stay untouched until the stream has passed the call.
+ * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer, n_slots outside 1..64, a slot outside 0..199,
+ * body_out_d not 16-byte or rows_d not 8-byte aligned; GO1MPC_E_UNSUPPORTED for nh outside 3..40 or cfg.step.ext_height set.
+ * ------------------------------------------------------------------------ */
+#define GO1MPC_STACK_SENSOR_ROWS 11   /* /control2rtmpc/state slots 0 | 10 11 13 14 | 19 20 21 | 22 23 24 */
+#define GO1MPC_STACK_SLOTS_MAX 64
+#define GO1MPC_STACK_ROW_NLP 0
+#define GO1MPC_STACK_ROW_GAIT 480
+#define GO1MPC_STACK_ROW_RT2NRT 580
+#define GO1MPC_STACK_ROW_WALKDTIME 605
+#define GO1MPC_STACK_ROW_TRAJ 606
+#define GO1MPC_STACK_ROW_RT 706
+typedef struct {
+  int nh;                    /* body-MPC horizon, 3..40 */
+  int planner;               /* 1: the 40 Hz planner node ticks first in this call */
+  const double *sensor;      /* host [11][B] SoA: control flag, body angles / rates, L foot xyz, R foot xyz */
+  const int *cmd, *start;    /* host [B] or NULL; read only when planner = 1 (as go1mpc_nlp_node_tick_batch) */
+  double *state_d;           /* device [go1mpc_gait_stack_state_doubles(nh)][B] SoA, in/out */
+  double *body_out_d;        /* device [B][go1mpc_body_out_stride(nh)], in/out, zero-initialised, 16-byte aligned */
+  int n_slots;
+  int slots[GO1MPC_STACK_SLOTS_MAX];   /* 0..99 = /MPC/Gait slot, 100..199 = /rtMPC/traj slot - 100 */
+  double *rows_d;            /* device [B][n_slots], caller-owned (e.g. go1mpc_gather_dest with row_doubles = n_slots) */
+  double *rows;              /* host [B][n_slots] or NULL: copy of rows_d */
+} Go1GaitStackTick;
+int go1mpc_gait_stack_state_doubles(int nh);
+int go1mpc_gait_stack_default_state(go1mpc_t *h, int nh, double *column);
+int go1mpc_gait_stack_tick_host_async(go1mpc_t *h, int B, const Go1GaitStackTick *t, void *stream);
+
 /* Per-kernel timing of the three-launch body tick (measurement aid for bench.py's roofline): while enabled, each
  * go1mpc_body_mpc_step_batch call on that path records CUDA events around its setup / solve / merge launches;
  * go1mpc_body_phase_ms waits for the last such call and returns the three durations in milliseconds.  Do not enable

@@ -9,7 +9,8 @@ from .binding import (  # noqa: F401
     Go1Mpc, Go1MpcError, load_library, library_path, body_in_stride, body_out_stride,
     body_diag_stride, pack_body_inputs, EXPORTED_SYMBOLS, QP_ITERS, BODY_DIAG_ACTIVE,
     STEP_STATE, STEP_IN, STEP_OUT, STEP_DIAG, BODY_TICK_OUT, body_tick_in_stride, split_body_record,
-    ControlTick, COMPACT_DOUBLES, lpf_coefficients,
+    ControlTick, COMPACT_DOUBLES, lpf_coefficients, GaitStackTick, STACK_SENSOR_ROWS, STACK_SLOTS_MAX, STACK_ROW_NLP,
+    STACK_ROW_GAIT, STACK_ROW_RT2NRT, STACK_ROW_WALKDTIME, STACK_ROW_TRAJ, STACK_ROW_RT,
 )
 from ._build import build  # noqa: F401
 
@@ -18,4 +19,6 @@ __all__ = [
     "body_out_stride", "body_diag_stride", "pack_body_inputs", "EXPORTED_SYMBOLS", "QP_ITERS",
     "BODY_DIAG_ACTIVE", "STEP_STATE", "STEP_IN", "STEP_OUT", "STEP_DIAG", "BODY_TICK_OUT", "body_tick_in_stride",
     "split_body_record", "ControlTick", "COMPACT_DOUBLES", "lpf_coefficients",
+    "GaitStackTick", "STACK_SENSOR_ROWS", "STACK_SLOTS_MAX", "STACK_ROW_NLP", "STACK_ROW_GAIT", "STACK_ROW_RT2NRT",
+    "STACK_ROW_WALKDTIME", "STACK_ROW_TRAJ", "STACK_ROW_RT",
 ]

@@ -33,6 +33,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_nlp_node_state_doubles", "go1mpc_nlp_node_default_state", "go1mpc_nlp_walkdtime_max", "go1mpc_nlp_t_end_footstep",
     "go1mpc_nlp_node_tick_batch", "go1mpc_foot_trajectory_stop_batch", "go1mpc_nlp_node_tick_batch_host", "go1mpc_rt_node_tick_batch_host", "go1mpc_foot_trajectory_stop_batch_host",
     "go1mpc_grf_force_opt_batch_host", "go1mpc_grf_force_distribution_batch_host", "go1mpc_grf_joint_torques_batch_host", "go1mpc_leg_fk_batch_host", "go1mpc_leg_ik_batch_host",
+    "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
 ]
 
 
@@ -163,6 +164,9 @@ def load_library():
     lib.go1mpc_graph_destroy.argtypes = [vp, vp]
     lib.go1mpc_leg_fk_batch_host.argtypes = [vp, ctypes.c_int] + [vp] * 6
     lib.go1mpc_leg_ik_batch_host.argtypes = [vp, ctypes.c_int] + [vp] * 8
+    lib.go1mpc_gait_stack_state_doubles.argtypes = [ctypes.c_int]
+    lib.go1mpc_gait_stack_default_state.argtypes = [vp, ctypes.c_int, vp]
+    lib.go1mpc_gait_stack_tick_host_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackTick), vp]
     _LIB = lib
     return lib
 
@@ -249,6 +253,20 @@ class ControlTick(ctypes.Structure):
                 ("tx_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p), ("compact_d", ctypes.c_void_p),
                 ("compact", ctypes.c_void_p), ("out38", ctypes.c_void_p), ("step_diag", ctypes.c_void_p),
                 ("body_diag", ctypes.c_void_p), ("step_in_rows", ctypes.c_int)]
+
+
+STACK_SENSOR_ROWS = 11   # GO1MPC_STACK_SENSOR_ROWS: /control2rtmpc/state slots 0 | 10 11 13 14 | 19 20 21 | 22 23 24
+STACK_SLOTS_MAX = 64     # GO1MPC_STACK_SLOTS_MAX
+# GO1MPC_STACK_ROW_*: first row of each block of the gait stack state
+STACK_ROW_NLP, STACK_ROW_GAIT, STACK_ROW_RT2NRT, STACK_ROW_WALKDTIME, STACK_ROW_TRAJ, STACK_ROW_RT = 0, 480, 580, 605, 606, 706
+
+
+class GaitStackTick(ctypes.Structure):
+    """Go1GaitStackTick of include/go1mpc.h."""
+    _fields_ = [("nh", ctypes.c_int), ("planner", ctypes.c_int), ("sensor", ctypes.c_void_p), ("cmd", ctypes.c_void_p),
+                ("start", ctypes.c_void_p), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p),
+                ("n_slots", ctypes.c_int), ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p),
+                ("rows", ctypes.c_void_p)]
 
 
 def _ptr(a):
@@ -540,6 +558,29 @@ class Go1Mpc:
         self._check(self.lib.go1mpc_rt_node_tick_msgs_batch(self.h, nh, B, _ptr(state_d), _ptr(gait_msg_d), _ptr(ctl_msg_d), _ptr(body_in_d),
                                                             _ptr(body_out_d), _ptr(body_diag_d), _ptr(traj_msg_d), _ptr(rt2nrt_msg_d),
                                                             stream), "rt_node_tick_msgs_batch")
+
+    # --- gait stack tick: both nodes behind one host call ---
+    def gait_stack_state_doubles(self, nh):
+        return int(self.lib.go1mpc_gait_stack_state_doubles(nh))
+
+    def gait_stack_default_state(self, nh):
+        s = np.zeros(self.gait_stack_state_doubles(nh))
+        self._check(self.lib.go1mpc_gait_stack_default_state(self.h, nh, _ptr(s)), "gait_stack_default_state")
+        return s
+
+    def gait_stack_tick_struct(self, nh, planner, sensor, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None):
+        """Go1GaitStackTick for the given buffers (host: sensor [11][B], cmd / start [B] int32, rows [B][len(slots)])."""
+        t = GaitStackTick(nh, 1 if planner else 0, _ptr(sensor), _ptr(cmd), _ptr(start), _ptr(state_d), _ptr(body_out_d), len(slots))
+        for k, v in enumerate(slots[:STACK_SLOTS_MAX]):
+            t.slots[k] = int(v)
+        t.rows_d = _ptr(rows_d)
+        t.rows = _ptr(rows)
+        return t
+
+    def gait_stack_tick_host_async(self, B, t, stream=None):
+        """go1mpc_gait_stack_tick_host_async with a GaitStackTick (gait_stack_tick_struct); returns after enqueueing on `stream`
+        (None = the handle's)."""
+        self._check(self.lib.go1mpc_gait_stack_tick_host_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_host_async")
 
     def measure_dfma_peak(self, ms=200):
         g = ctypes.c_double(0.0)

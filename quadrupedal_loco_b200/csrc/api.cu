@@ -71,6 +71,10 @@ struct go1mpc {
   double* squat_d = nullptr;       // X_CoM_position_squat table of the planner node (host libm), built on first use
   struct NlpWs { DevBuf b[7]; };   // workspace of go1mpc_nlp_node_tick_batch, one per caller stream
   std::map<cudaStream_t, NlpWs> nlp_ws;
+  // workspace of go1mpc_gait_stack_tick_host_async, one per caller stream (grown on demand): sensor | /control2rtmpc/state |
+  // walkdtime ints | cmd | start | body-MPC input records
+  struct StackWs { DevBuf b[6]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
+  std::map<cudaStream_t, StackWs> stack_ws;
   double* trtab_d = nullptr;       // remaining-time bound table of the planner tick (host libm), built on first use
   std::vector<cudaEvent_t> ev_pool;   // go1mpc_stream_wait: events, reused round-robin
   unsigned ev_next = 0;
@@ -330,6 +334,7 @@ void go1mpc_destroy(go1mpc_t* h) {
   if (h->squat_d) cudaFree(h->squat_d);
   for (cudaEvent_t e : h->phase_ev) if (e) cudaEventDestroy(e);
   for (auto& kv : h->nlp_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
+  for (auto& kv : h->stack_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
   for (auto& L : h->lanes) {
     for (DevBuf& b : L.stage) if (b.p) cudaFree(b.p);
     if (L.stream) cudaStreamDestroy(L.stream);
@@ -1398,6 +1403,86 @@ int go1mpc_rt_node_tick_batch_host(go1mpc_t* h, int nh, int B, double* state, co
   CU(h, cudaMemcpyAsync(body_out, dbo, bob, cudaMemcpyDeviceToHost, st));
   CU(h, cudaMemcpyAsync(out100, dout, mb, cudaMemcpyDeviceToHost, st));
   CU(h, cudaStreamSynchronize(st));
+  return GO1MPC_OK;
+}
+
+// ------------------------------------------------------------------ gait stack tick: both nodes behind one host call
+static_assert(GO1MPC_STACK_ROW_GAIT == GO1MPC_STACK_ROW_NLP + NLP_NODE_DOUBLES && GO1MPC_STACK_ROW_RT2NRT == GO1MPC_STACK_ROW_GAIT + 100 &&
+              GO1MPC_STACK_ROW_WALKDTIME == GO1MPC_STACK_ROW_RT2NRT + 25 && GO1MPC_STACK_ROW_TRAJ == GO1MPC_STACK_ROW_WALKDTIME + 1 &&
+              GO1MPC_STACK_ROW_RT == GO1MPC_STACK_ROW_TRAJ + 100, "gait stack state layout");
+static_assert(GO1MPC_STACK_SENSOR_ROWS == GAIT_STACK_SENSOR_ROWS && GO1MPC_STACK_SLOTS_MAX == GAIT_STACK_SLOTS_MAX, "gait stack sizes");
+int go1mpc_gait_stack_state_doubles(int nh) { return GO1MPC_STACK_ROW_RT + go1mpc_rt_node_state_doubles(nh); }
+int go1mpc_gait_stack_default_state(go1mpc_t* h, int nh, double* s) {
+  if (!h || !s) return GO1MPC_E_INVALID;
+  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_default_state: 3 <= nh <= 40");
+  memset(s, 0, sizeof(double) * GO1MPC_STACK_ROW_RT);
+  int rc = go1mpc_nlp_node_default_state(h, s + GO1MPC_STACK_ROW_NLP);
+  if (rc) return rc;
+  return go1mpc_rt_node_default_state(h, nh, s + GO1MPC_STACK_ROW_RT);
+}
+
+int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick* t, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
+  if (!t || !t->sensor || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: bad argument");
+  const int nh = t->nh, n = t->n_slots;
+  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_tick_host_async: 3 <= nh <= 40");
+  if (h->cfg.step.ext_height)
+    return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_tick_host_async: cfg.step.ext_height must be 0 (the planner node owns CoM_height_solve)");
+  if (n < 1 || n > GO1MPC_STACK_SLOTS_MAX) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: 1 <= n_slots <= 64");
+  GaitStackSlots S;
+  S.n = n;
+  for (int k = 0; k < GO1MPC_STACK_SLOTS_MAX; k++) {
+    S.slot[k] = k < n ? t->slots[k] : 0;
+    if (S.slot[k] < 0 || S.slot[k] >= 200) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: slots must lie in 0..199");
+  }
+  // the body kernels read and write body_out_d with 16-byte loads / TMA; the pack kernel stores doubles into rows_d
+  if (((uintptr_t)t->body_out_d & 15) || ((uintptr_t)t->rows_d & 7))
+    return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: body_out_d must be 16-byte and rows_d 8-byte aligned");
+  CU(h, cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
+    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
+  go1mpc::StackWs& W = h->stack_ws[st];
+  const size_t b = (size_t)B;
+  const size_t bytes[6] = {b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), b * 25 * sizeof(double), b * sizeof(int), b * sizeof(int),
+                           b * sizeof(int), b * go1mpc_body_in_stride(nh) * sizeof(double)};
+  void* d[6];
+  int rc;
+  for (int k = 0; k < 6; k++) {
+    const bool grow = bytes[k] > W.b[k].cap;
+    if (grow) CU(h, cudaStreamSynchronize(st));     // growing: earlier work on this stream may still use the old buffer
+    if ((rc = stage_buf2(h, W.b[k], bytes[k], &d[k]))) return rc;
+    if (grow && k == 1) W.zero_B = -1;
+  }
+  double* ctl = (double*)d[1];
+  if (W.zero_B != B) {
+    // the 14 slots of /control2rtmpc/state the stack does not upload read as zero: cleared once per batch size
+    CU(h, cudaMemsetAsync(ctl, 0, bytes[1], st));
+    W.zero_B = B;
+  }
+  double* state = t->state_d;
+  CU(h, cudaMemcpyAsync(d[0], t->sensor, bytes[0], cudaMemcpyHostToDevice, st));
+  const int* cmd_d = nullptr;
+  const int* start_d = nullptr;
+  if (t->planner && t->cmd) { CU(h, cudaMemcpyAsync(d[3], t->cmd, bytes[3], cudaMemcpyHostToDevice, st)); cmd_d = (const int*)d[3]; }
+  if (t->planner && t->start) { CU(h, cudaMemcpyAsync(d[4], t->start, bytes[4], cudaMemcpyHostToDevice, st)); start_d = (const int*)d[4]; }
+  CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl, h->sms, st));
+  h->launches++;
+  double* gait = state + GO1MPC_STACK_ROW_GAIT * b;
+  double* rt2nrt = state + GO1MPC_STACK_ROW_RT2NRT * b;
+  double* traj = state + GO1MPC_STACK_ROW_TRAJ * b;
+  if (t->planner &&
+      (rc = go1mpc_nlp_node_tick_batch(h, B, state + GO1MPC_STACK_ROW_NLP * b, (const int*)d[2], start_d, cmd_d, rt2nrt + 22 * b,
+                                       rt2nrt + 19 * b, gait, st)))
+    return rc;
+  if ((rc = rt_node_enqueue(h, nh, B, state + GO1MPC_STACK_ROW_RT * b, gait, nullptr, nullptr, ctl, (double*)d[5], t->body_out_d, nullptr,
+                            traj, rt2nrt, nullptr, st)))
+    return rc;
+  CU(h, gait_stack_pack_launch(S, B, gait, traj, t->rows_d, h->sms, st));
+  h->launches++;
+  if (t->rows) CU(h, cudaMemcpyAsync(t->rows, t->rows_d, b * n * sizeof(double), cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
 }
 

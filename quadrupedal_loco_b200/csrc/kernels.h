@@ -244,6 +244,17 @@ struct RtKParams {
 cudaError_t rt_pre_launch(RtKParams P, cudaStream_t st);
 cudaError_t rt_post_launch(RtKParams P, cudaStream_t st);
 
+// ---- the gait stack tick around both nodes (gait_stack.cu) ----
+constexpr int GAIT_STACK_SENSOR_ROWS = 11, GAIT_STACK_SLOTS_MAX = 64;
+struct GaitStackSlots {
+  int n;
+  int slot[GAIT_STACK_SLOTS_MAX];   // 0..99 /MPC/Gait slot, 100..199 /rtMPC/traj slot + 100
+};
+cudaError_t gait_stack_pre_launch(int B, int planner, double* walkdtime_row, int* walkdtime_i, const double* sensor, double* ctl,
+                                  int sms, cudaStream_t st);
+cudaError_t gait_stack_pack_launch(const GaitStackSlots& S, int B, const double* gait, const double* traj, double* rows, int sms,
+                                   cudaStream_t st);
+
 // register-resident DFMA loop: flops executed are returned through *flops
 cudaError_t dfma_peak_launch(int grid, int block, int iters, double* sink, cudaStream_t st);
 

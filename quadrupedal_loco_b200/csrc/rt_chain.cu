@@ -26,6 +26,7 @@ constexpr int NS = 27;
 constexpr int N_LOOP = 0, N_MPC = 1, N_CNT = 2, N_TINT = 3, N_FLAGOLD = 4, N_COM = 5, N_COMV = 17, N_ACC = 20, N_ZMP = 32, N_DCM = 44, N_INTER = 56;
 // swing-foot layout (oracle/rt_foot.c), relative to its base
 constexpr int F_TS = 0, F_FX = 27, F_LIFT = 108, F_RY = 135, F_BJXX = 136, F_BJX1 = 137, F_ARR = 138;
+constexpr int NH_MAX = 40, W_MAX = NH_MAX + 2;   // GO1MPC_BODY_NH_MAX; window width nh + 2
 
 __device__ __forceinline__ int ni_of(int nh) { return 9 + 3 * (nh - 1); }
 
@@ -88,6 +89,11 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
   const double flag = MSG(99);
   const bool ctrl = P.ctl_msg ? (P.ctl_msg[b] > 0) : (P.ctrl ? (P.ctrl[b] > 0) : true);
   bool active = false;
+  double cmpc = 0.0;
+  // the step table _ts: read once, written back once (the message may re-time one step)
+  double ts[NS];
+#pragma unroll
+  for (int i = 0; i < NS; i++) ts[i] = FS_(F_TS + i);
   double* rec = P.body_in + (size_t)b * P.in_stride;
   const double* bout = P.body_out + (size_t)b * P.out_stride;
   if (ctrl) {
@@ -97,7 +103,7 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
     N_(N_TINT) = tint;
     if (flag > 0) {
       active = true;
-      const double cmpc = N_(N_MPC) + 1;
+      cmpc = N_(N_MPC) + 1;
       N_(N_MPC) = cmpc;
       // ---- xget_position_interpolation (:113-372) ----
       const double cnt = N_(N_CNT) + 1;
@@ -172,21 +178,35 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
           FS_(F_FX + 54 + bjxx_nrt) = MSG(91); FS_(F_FX + 54 + bjxx_nrt + 1) = MSG(92);
         }
         const int bjxp = (int)MSG(93);
-        if (MSG(94) > 0 && bjxp >= 0 && bjxp < NS) FS_(F_TS + bjxp) = MSG(94);
+        if (MSG(94) > 0 && bjxp >= 0 && bjxp < NS) { ts[bjxp] = MSG(94); FS_(F_TS + bjxp) = ts[bjxp]; }
       }
     }
   }
   // step tables rebuilt from _ts (:1774-1784); _t_end_footstep with 2 tstep (the swing-foot call's)
   double tx[NS];
   tx[0] = 0.0;
-  for (int i = 1; i < NS; i++) { double v = tx[i - 1] + FS_(F_TS + i - 1); tx[i] = round(v / dt_slow) * dt_slow - 0.00001; }
+  for (int i = 1; i < NS; i++) { double v = tx[i - 1] + ts[i - 1]; tx[i] = round(v / dt_slow) * dt_slow - 0.00001; }
   const double t_end = round((tx[NS - 1] - 2 * P.tstep) / dt_fast);
-  if (active && N_(N_MPC) * dt_fast > 1) {
-    const int j_indexx = (int)(N_(N_MPC) - (int)1 / dt_fast);
+  // The swing-foot window, the lift heights and the foot-rotation horizons live in local arrays for the whole horizon loop:
+  // loaded once, stored once.  Same operations in the same order as the reference, so the results are bit-identical.
+  const bool swung = active && cmpc * dt_fast > 1;
+  double arr[6 * W_MAX], rot[6 * NH_MAX];
+  if (swung) {
+    const int j_indexx = (int)(cmpc - (int)1 / dt_fast);
     int bjxx = (int)FS_(F_BJXX), bjx1 = (int)FS_(F_BJX1);
     double ry = FS_(F_RY);
-#define ARR(foot, k, idx) FS_(F_ARR + ((foot) * 3 + (k)) * W + (idx))      /* foot 0 = right, 1 = left */
+    for (int i = 0; i < 6 * W; i++) arr[i] = FS_(F_ARR + i);
+    double lift[NS];
+#pragma unroll
+    for (int i = 0; i < NS; i++) lift[i] = FS_(F_LIFT + i);
+    // the reference zeroes lift heights 24..26 on every horizon step; nothing in the loop sets them, so once is the same
+#pragma unroll
+    for (int it = 24; it < NS; it++) lift[it] = 0.0;
+#define ARR(foot, k, idx) arr[((foot) * 3 + (k)) * W + (idx)]      /* foot 0 = right, 1 = left */
 #define FXYZ(k, idx) FS_(F_FX + 27 * (k) + (idx))
+    FXYZ(1, 0) = -P.stepwidth0;
+    int fx_key = -1000;            // bjxx the footstep cache below belongs to
+    double fq[3], fq2[3];          // FXYZ(k, bq), FXYZ(k, bq2)
     for (int j_index = j_indexx; j_index < j_indexx + nh; j_index++) {
       const int q = j_index - j_indexx;
       if (j_index <= t_end) {
@@ -197,22 +217,26 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
         while (jp < NS && (j_index + 1) * dt_fast >= tx[jp]) jp++;
         bjx1 = (jp - 1) + 1;
       }
-      if (j_index > t_end) for (int it = bjx1 + 1; it < NS; it++) FS_(F_LIFT + it) = 0.0;       // (stop-walking flag: not raised by the node)
-      for (int it = 24; it < NS; it++) FS_(F_LIFT + it) = 0.0;
-      FXYZ(1, 0) = -P.stepwidth0;
+      if (j_index > t_end) for (int it = bjx1 + 1; it < NS; it++) lift[it] = 0.0;       // (stop-walking flag: not raised by the node)
       if (bjx1 >= 2 && j_index <= t_end) {
         const int sup = (bjx1 % 2 == 0) ? 1 : 0, swg = 1 - sup;       // even: left support, right swing
         for (int k = 0; k < 3; k++) { const double v = ARR(sup, k, q); ARR(sup, k, q + 1) = v; ARR(sup, k, q + 2) = v; }
-        const double ts1 = FS_(F_TS + bjx1 - 1), td1 = P.tdsp_ratio * ts1;
+        const double ts1 = ts[bjx1 - 1], td1 = P.tdsp_ratio * ts1;
         const double s0 = round(tx[bjx1 - 1] / dt_fast);
         if ((j_index + 1 - s0) * dt_fast < td1) {
           for (int k = 0; k < 3; k++) { const double v = ARR(swg, k, q); ARR(swg, k, q + 1) = v; ARR(swg, k, q + 2) = v; }
         } else {
           const double t_des = (j_index + 1 - s0 + 1) * dt_fast;
           const double tp[3] = {t_des - dt_fast, (td1 + ts1) / 2 + 0.0001, ts1 - (2 * dt_fast + 0.001)};
-          const int bq = bjxx < NS ? bjxx : NS - 1, bq2 = bjxx - 2 >= 0 ? (bjxx - 2 < NS ? bjxx - 2 : NS - 1) : 0;
+          if (bjxx != fx_key) {
+            const int bq = bjxx < NS ? bjxx : NS - 1, bq2 = bjxx - 2 >= 0 ? (bjxx - 2 < NS ? bjxx - 2 : NS - 1) : 0;
+#pragma unroll
+            for (int k = 0; k < 3; k++) { fq[k] = FXYZ(k, bq); fq2[k] = FXYZ(k, bq2); }
+            fx_key = bjxx;
+          }
           if (fabs(t_des - ts1) <= (dt_fast)) {
-            for (int k = 0; k < 3; k++) { const double v = FXYZ(k, bq); ARR(swg, k, q + 1) = v; ARR(swg, k, q + 2) = v; }
+#pragma unroll
+            for (int k = 0; k < 3; k++) { const double v = fq[k]; ARR(swg, k, q + 1) = v; ARR(swg, k, q + 2) = v; }
           } else {
             double A[16], Ai[16];
             for (int r = 0; r < 3; r++) { A[4 * r] = powi(tp[r], 3); A[4 * r + 1] = powi(tp[r], 2); A[4 * r + 2] = powi(tp[r], 1); A[4 * r + 3] = 1; }
@@ -220,14 +244,15 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
             gj4(A, Ai);
             const double tap[4] = {powi(t_des, 3), powi(t_des, 2), powi(t_des, 1), 1};
             const double tav[4] = {3 * powi(t_des, 2), 2 * powi(t_des, 1), 1, 0};
-            if ((j_index + 1 - s0) * dt_fast < td1 + dt_fast) ry = (FXYZ(1, bq) + FXYZ(1, bq2)) / 2;
+            if ((j_index + 1 - s0) * dt_fast < td1 + dt_fast) ry = (fq[1] + fq2[1]) / 2;
+#pragma unroll
             for (int k = 0; k < 3; k++) {
               double plan[4];
               plan[0] = ARR(swg, k, q);
-              if (k == 0) plan[1] = (FXYZ(0, bq2) + FXYZ(0, bq)) / 2;
+              if (k == 0) plan[1] = (fq2[0] + fq[0]) / 2;
               else if (k == 1) plan[1] = ry;
-              else plan[1] = fmax(FXYZ(2, bq2), FXYZ(2, bq)) + FS_(F_LIFT + bjx1 - 1);
-              plan[2] = FXYZ(k, bq);
+              else plan[1] = fmax(fq2[2], fq[2]) + lift[bjx1 - 1];
+              plan[2] = fq[k];
               plan[3] = 0;
               double co[4];
               for (int r = 0; r < 4; r++) { double a_ = 0.0; for (int m = 0; m < 4; m++) a_ += Ai[4 * r + m] * plan[m]; co[r] = a_; }
@@ -249,9 +274,14 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
     }
     for (int jjj = 0; jjj < nh + 1; jjj++)
       for (int k = 0; k < 3; k++) { N_(o_foot + 6 * jjj + k) = ARR(0, k, jjj + 1); N_(o_foot + 6 * jjj + 3 + k) = ARR(1, k, jjj + 1); }
-    for (int k = 0; k < 3; k++) { ARR(0, k, 0) = ARR(0, k, 1); ARR(1, k, 0) = ARR(1, k, 1); }
+    // column 0 of the stored window takes column 1 (the reference's shift after the horizon); the local copy stays unshifted:
+    // the record below reads columns 1..nh only
+    for (int i = 0; i < 6 * W; i++) FS_(F_ARR + i) = (i % W == 0) ? arr[i + 1] : arr[i];
+#pragma unroll
+    for (int i = 0; i < NS; i++) FS_(F_LIFT + i) = lift[i];
     FS_(F_BJXX) = bjxx; FS_(F_BJX1) = bjx1; FS_(F_RY) = ry;
-    // XGetSolution_Foot_rotation (:2255-2380) with the members Foot_trajectory_solve_mod2 just updated
+    // XGetSolution_Foot_rotation (:2255-2380) with the members Foot_trajectory_solve_mod2 just updated; rot = Rr[3][nh] | Lr[3][nh]
+    for (int i = 0; i < 6 * nh; i++) rot[i] = RS_(2 + i);
     int rbjxx = (int)RS_(0), rbjx1 = (int)RS_(1);
     for (int walktime = j_indexx; walktime < j_indexx + nh; walktime++) {
       const int col = walktime - j_indexx;
@@ -265,31 +295,32 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
       }
       const int k = rbjx1 - 1;
       if (rbjx1 >= 2 && walktime <= t_end) {
-        const double tsk = FS_(F_TS + k), tdk = P.tdsp_ratio * tsk;
+        const double tsk = ts[k], tdk = P.tdsp_ratio * tsk;
         const double t_des = (walktime + 1) * dt_fast - (tx[k] + 2 * tdk / 4);
         const double sarg = t_des + 2 * tdk / 4;
         const int i1 = rbjx1 < NS ? rbjx1 : NS - 1;
         const double dfx = FXYZ(0, i1) - FXYZ(0, rbjx1 - 1);
-        const int base = 2 + ((rbjx1 % 2 == 0) ? 0 : 3 * nh);          // even: the right foot swings
+        const int base = (rbjx1 % 2 == 0) ? 0 : 3 * nh;          // even: the right foot swings
         const double amp = (rbjx1 % 2 == 0) ? -0.065 : 0.075;
-        RS_(base + 0 * nh + col) = amp * (1 - cos(2 * CUDART_PI / tsk * sarg));
+        rot[base + 0 * nh + col] = amp * (1 - cos(2 * CUDART_PI / tsk * sarg));
         if (sarg >= tsk / 2) {
-          if (dfx > 0) RS_(base + 1 * nh + col) = 0.075 * dfx / P.footx_max * (cos(4 * CUDART_PI / tsk * sarg) - 1);
+          if (dfx > 0) rot[base + 1 * nh + col] = 0.075 * dfx / P.footx_max * (cos(4 * CUDART_PI / tsk * sarg) - 1);
         } else {
-          RS_(base + 1 * nh + col) = 0;
+          rot[base + 1 * nh + col] = 0;
         }
       }
-      N_(o_rot + 6 * col + 0) = RS_(2 + 0 * nh + col); N_(o_rot + 6 * col + 1) = RS_(2 + 1 * nh + col); N_(o_rot + 6 * col + 2) = RS_(2 + 2 * nh + 0);
-      N_(o_rot + 6 * col + 3) = RS_(2 + 3 * nh + 0 * nh + col); N_(o_rot + 6 * col + 4) = RS_(2 + 3 * nh + 1 * nh + col); N_(o_rot + 6 * col + 5) = RS_(2 + 3 * nh + 2 * nh + 0);
+      N_(o_rot + 6 * col + 0) = rot[0 * nh + col]; N_(o_rot + 6 * col + 1) = rot[1 * nh + col]; N_(o_rot + 6 * col + 2) = rot[2 * nh + 0];
+      N_(o_rot + 6 * col + 3) = rot[3 * nh + col]; N_(o_rot + 6 * col + 4) = rot[4 * nh + col]; N_(o_rot + 6 * col + 5) = rot[5 * nh + 0];
     }
+    // rows 0, 1 of each foot are the ones the loop writes
+    for (int i = 0; i < 2 * nh; i++) { RS_(2 + i) = rot[i]; RS_(2 + 3 * nh + i) = rot[3 * nh + i]; }
     RS_(0) = rbjxx; RS_(1) = rbjx1;
-#undef ARR
 #undef FXYZ
   }
   if (active) N_(N_ZMP + 8) = 0.0;          // zmpxyz_ref(2) = _Zsc = 0
   // ---- body-MPC input record (:568-620); an inactive robot gets a gated tick (0): its body state stays as it is ----
   for (int k = 0; k < NS; k++) rec[k] = tx[k];
-  rec[27] = active ? N_(N_MPC) : 0.0;
+  rec[27] = active ? cmpc : 0.0;
   for (int k = 0; k < 4; k++) { rec[28 + k] = bout[14 + k]; rec[32 + k] = P.ctl_msg ? P.ctl_msg[(size_t)(k < 2 ? 10 + k : 11 + k) * B + b]       // state_feedback(10, 11, 13, 14), :105-108
                              : (P.bodyangle_state ? P.bodyangle_state[(size_t)k * B + b] : 0.0); }
   for (int k = 0; k < 2 * nh; k++) rec[36 + k] = bout[18 + k];
@@ -299,11 +330,15 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
     for (int jxx = 0; jxx < nh; jxx++) {
       rows[0 * nh + jxx] = (jxx == 0) ? N_(zi + 0) : N_(zi + 8 + 3 * jxx - 2);
       rows[1 * nh + jxx] = (jxx == 0) ? N_(zi + 1) : N_(zi + 8 + 3 * jxx - 1);
-      const double a0 = (N_(o_rot + jxx * 6) + N_(o_rot + jxx * 6 + 3)) / 5, a1 = (N_(o_rot + jxx * 6 + 1) + N_(o_rot + jxx * 6 + 4)) / 5;
+      // the horizons of this tick when the swing section ran, else the stale ones the state holds
+      const double r0 = swung ? rot[jxx] : N_(o_rot + jxx * 6), l0 = swung ? rot[3 * nh + jxx] : N_(o_rot + jxx * 6 + 3);
+      const double r1 = swung ? rot[nh + jxx] : N_(o_rot + jxx * 6 + 1), l1 = swung ? rot[4 * nh + jxx] : N_(o_rot + jxx * 6 + 4);
+      const double a0 = (r0 + l0) / 5, a1 = (r1 + l1) / 5;
       rows[2 * nh + jxx] = a0; rows[3 * nh + jxx] = a1;
-      rows[4 * nh + jxx] = N_(o_foot + jxx * 6 + 1);        // row 0 written twice (x, then y), row 1 never
+      rows[4 * nh + jxx] = swung ? ARR(0, 1, jxx + 1) : N_(o_foot + jxx * 6 + 1);        // row 0 written twice (x, then y), row 1 never
       rows[5 * nh + jxx] = 0.0;
-      rows[6 * nh + jxx] = N_(o_foot + jxx * 6 + 3); rows[7 * nh + jxx] = N_(o_foot + jxx * 6 + 4);
+      rows[6 * nh + jxx] = swung ? ARR(1, 0, jxx + 1) : N_(o_foot + jxx * 6 + 3);
+      rows[7 * nh + jxx] = swung ? ARR(1, 1, jxx + 1) : N_(o_foot + jxx * 6 + 4);
       rows[8 * nh + jxx] = (jxx == 0) ? N_(ai + 2) : N_(ai + 8 + 3 * jxx);
       if (jxx == 0) { N_(o_thx + 0) = a0; N_(o_thx + 1) = a1; }
     }
@@ -312,6 +347,7 @@ __global__ void __launch_bounds__(128) rt_pre_kernel(RtKParams P) {
   }
   if (P.in_stride > 36 + 11 * nh) rec[36 + 11 * nh] = 0.0;
   if (P.active) P.active[b] = active ? 1 : 0;
+#undef ARR
 #undef N_
 #undef MSG
 #undef FS_
