@@ -387,7 +387,7 @@ __global__ void GO1_TRI_BOUNDS(WPC) tri_solve_kernel(BodyKParams P) {
   unsigned inA = 0u;               // bit 4m+s: slot s of own variable m is in the working set
   int cur = -1, h = 0, iq = 0, nout = 0, npass = 0;
   bool fin = true, dead = false, need_l1 = true, flag = false, end_tol = false;
-  double tol = 0.0, f_value = 0.0, psi_end = 0.0, R_norm = 1.0, dq_min = inf;
+  double tol = 0.0, f_value = 0.0, R_norm = 1.0, dq_min = inf;
   int ip = 0, ip_blk = 0, ip_k = 0;
   double sip = 0.0, ip_sgn = 1.0;
   double* res = nullptr;
@@ -402,7 +402,7 @@ __global__ void GO1_TRI_BOUNDS(WPC) tri_solve_kernel(BodyKParams P) {
 #pragma unroll
           for (int m = 0; m < RW; m++) if (valid[m]) res[row[m]] = x[m];
           if (gl == 0) {
-            res[NH] = f_value; res[NH + 1] = psi_end; res[NH + 2] = R_norm; res[NH + 3] = dq_min;
+            res[NH] = f_value; res[NH + 2] = R_norm; res[NH + 3] = dq_min;
             resi[0] = nout; resi[1] = npass; resi[2] = end_tol ? 1 : 0; resi[3] = flag ? 1 : 0;
           }
         }
@@ -439,7 +439,7 @@ __global__ void GO1_TRI_BOUNDS(WPC) tri_solve_kernel(BodyKParams P) {
           resi = res_ints(res, D::RES_D);
           inA = 0u; iq = 0; nout = 0; npass = 0;
           fin = false; need_l1 = true; flag = false; end_tol = false;
-          psi_end = 0.0; R_norm = 1.0; dq_min = inf;
+          R_norm = 1.0; dq_min = inf;
         }
       }
     }
@@ -497,7 +497,7 @@ __global__ void GO1_TRI_BOUNDS(WPC) tri_solve_kernel(BodyKParams P) {
       bi = min(bi, __shfl_xor_sync(FULL_MASK, bi, 2));
       bi = min(bi, __shfl_xor_sync(FULL_MASK, bi, 1));
       if (g1) {
-        psi_end = psi;
+        if (gl == 0) res[NH + 1] = psi;       // psi at the last step 1 of the half: stored as it is found, not held
         if (!(fabs(psi) > tol)) { fin = true; end_tol = true; if (psi != psi) flag = true; }
         else if (!(bv < 0.0)) fin = true;
         else if (nout >= D::OMAX) { fin = true; flag = true; }
