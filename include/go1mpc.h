@@ -679,6 +679,51 @@ int go1mpc_gait_stack_state_doubles(int nh);
 int go1mpc_gait_stack_default_state(go1mpc_t *h, int nh, double *column);
 int go1mpc_gait_stack_tick_host_async(go1mpc_t *h, int B, const Go1GaitStackTick *t, void *stream);
 
+/* ---------------------------------------------------------------------------
+ * Servo stack tick: K consecutive ticks of go1_servo's 1 kHz loop for B robots in ONE call, fed in place from the messages the
+ * gait stack keeps resident -- the call a controller farm makes after each gait stack call (K = 10 per 10 ms period), joint
+ * targets out.  Per robot b and tick k = 1..K:
+ *   filters   9 butterworthLPF objects, go1mpc_lpf_coefficients(1000, 3), on /MPC/Gait slots 0 1 2 6 7 8 9 10 11 (channels
+ *             0..8 in that order), each stepped once per tick on the held message value -- as 9 objects called every 1 kHz tick
+ *   IK        go1mpc_servo_kin_tick_batch's leg mapping and 4 x Inverse_kinematics_g (servo.cpp:935-1051) with
+ *               body position = filtered (slot 0, slot 1 * y_offset, slot 2)
+ *               roll, pitch   = /rtMPC/traj slots 72, 73 (the body MPC's Vec14 [0], [1]), yaw 0 -- the fused tick's wiring
+ *               left / right virtual foot = filtered slots 6 7 8 / 9 10 11
+ *               initial guess = the previous tick's joint angles
+ *             gait_mode (101 pace, 102 trot, 103 gallop) and y_offset as in go1mpc_servo_kin_tick_batch
+ * The result equals K x (go1mpc_lpf_batch on the state's /MPC/Gait block + go1mpc_servo_kin_tick_batch) bit for bit.
+ * Servo state, caller-owned SoA [GO1MPC_SERVO_STATE_ROWS][B]:
+ *   [GO1MPC_SERVO_ROW_Q, +12)       joint angles q (FR, FL, RR, RL), in/out
+ *   [GO1MPC_SERVO_ROW_HOMING, +12)  homing foot positions (input, as go1mpc_servo_kin_tick_batch's homing_d)
+ *   [GO1MPC_SERVO_ROW_LPF, +45)     the 9 filters' state in go1mpc_lpf_batch's [5][C][B] layout, C = 9; zero-initialise
+ * A robot is reset by rewriting its column, a batch is checkpointed by a memcpy.
+ * Not included: the servo's other filter objects (/MPC/Gait 39-41 and 73-75 at 10 Hz, ...) -- their outputs feed nothing here
+ * and go1mpc_lpf_batch runs them on the resident message --, FK of the measured joints (servo.cpp:734-741), the GRF QP and
+ * the torque map: how the servo assembles their inputs from the messages and the state estimator is not documented here.
+ * One kernel launch, plus the D2H copy of q_d when q is given; nothing is allocated, so a warmed-up gait stack + servo period
+ * can be captured with go1mpc_graph_capture_*.  B = 0 is a no-op.
+ * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer, K outside 1..GO1MPC_SERVO_TICKS_MAX, q_d not
+ * 8-byte aligned; GO1MPC_E_UNSUPPORTED for gait_mode outside 101..103.
+ * ------------------------------------------------------------------------ */
+#define GO1MPC_SERVO_TICKS_MAX 10
+#define GO1MPC_SERVO_STATE_ROWS 69
+#define GO1MPC_SERVO_ROW_Q 0
+#define GO1MPC_SERVO_ROW_HOMING 12
+#define GO1MPC_SERVO_ROW_LPF 24
+typedef struct {
+  int K;                        /* 1..GO1MPC_SERVO_TICKS_MAX consecutive 1 kHz ticks */
+  int gait_mode;
+  double y_offset;
+  const double *stack_state_d;  /* the gait stack's state [go1mpc_gait_stack_state_doubles(nh)][B], read only
+                                   (/MPC/Gait at GO1MPC_STACK_ROW_GAIT, /rtMPC/traj at GO1MPC_STACK_ROW_TRAJ) */
+  double *servo_state_d;        /* [GO1MPC_SERVO_STATE_ROWS][B] in/out */
+  double *q_d;                  /* device [B][12*K]: per robot, tick-major joint targets (usable as a gather dest) */
+  double *q;                    /* host [B][12*K] or NULL: D2H copy */
+  double *jac_d, *foot_des_d;   /* last tick's [36][B] / [12][B], or NULL */
+  int *iters_d;                 /* last tick's Newton updates [4][B], or NULL */
+} Go1ServoStackTick;
+int go1mpc_servo_stack_tick_async(go1mpc_t *h, int B, const Go1ServoStackTick *t, void *stream);
+
 /* Per-kernel timing of the three-launch body tick (measurement aid for bench.py's roofline): while enabled, each
  * go1mpc_body_mpc_step_batch call on that path records CUDA events around its setup / solve / merge launches;
  * go1mpc_body_phase_ms waits for the last such call and returns the three durations in milliseconds.  Do not enable

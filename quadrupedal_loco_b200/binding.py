@@ -34,6 +34,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_nlp_node_tick_batch", "go1mpc_foot_trajectory_stop_batch", "go1mpc_nlp_node_tick_batch_host", "go1mpc_rt_node_tick_batch_host", "go1mpc_foot_trajectory_stop_batch_host",
     "go1mpc_grf_force_opt_batch_host", "go1mpc_grf_force_distribution_batch_host", "go1mpc_grf_joint_torques_batch_host", "go1mpc_leg_fk_batch_host", "go1mpc_leg_ik_batch_host",
     "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
+    "go1mpc_servo_stack_tick_async",
 ]
 
 
@@ -167,6 +168,7 @@ def load_library():
     lib.go1mpc_gait_stack_state_doubles.argtypes = [ctypes.c_int]
     lib.go1mpc_gait_stack_default_state.argtypes = [vp, ctypes.c_int, vp]
     lib.go1mpc_gait_stack_tick_host_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackTick), vp]
+    lib.go1mpc_servo_stack_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoStackTick), vp]
     _LIB = lib
     return lib
 
@@ -267,6 +269,20 @@ class GaitStackTick(ctypes.Structure):
                 ("start", ctypes.c_void_p), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p),
                 ("n_slots", ctypes.c_int), ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p),
                 ("rows", ctypes.c_void_p)]
+
+
+SERVO_TICKS_MAX = 10      # GO1MPC_SERVO_TICKS_MAX
+SERVO_STATE_ROWS = 69     # GO1MPC_SERVO_STATE_ROWS
+# GO1MPC_SERVO_ROW_*: joint angles [0,12) | homing foot positions [12,24) | the 9 filters' state [5][9] from row 24
+SERVO_ROW_Q, SERVO_ROW_HOMING, SERVO_ROW_LPF = 0, 12, 24
+SERVO_LPF_SLOTS = [0, 1, 2, 6, 7, 8, 9, 10, 11]   # /MPC/Gait slot of filter channel 0..8: CoM | left foot | right foot
+
+
+class ServoStackTick(ctypes.Structure):
+    """Go1ServoStackTick of include/go1mpc.h."""
+    _fields_ = [("K", ctypes.c_int), ("gait_mode", ctypes.c_int), ("y_offset", ctypes.c_double),
+                ("stack_state_d", ctypes.c_void_p), ("servo_state_d", ctypes.c_void_p), ("q_d", ctypes.c_void_p),
+                ("q", ctypes.c_void_p), ("jac_d", ctypes.c_void_p), ("foot_des_d", ctypes.c_void_p), ("iters_d", ctypes.c_void_p)]
 
 
 def _ptr(a):
@@ -581,6 +597,20 @@ class Go1Mpc:
         """go1mpc_gait_stack_tick_host_async with a GaitStackTick (gait_stack_tick_struct); returns after enqueueing on `stream`
         (None = the handle's)."""
         self._check(self.lib.go1mpc_gait_stack_tick_host_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_host_async")
+
+    # --- servo stack tick: K 1 kHz servo ticks from the gait stack's resident messages ---
+    def servo_stack_tick_struct(self, K, gait_mode, y_offset, stack_state_d, servo_state_d, q_d, q=None, jac_d=None, foot_des_d=None,
+                                iters_d=None):
+        """Go1ServoStackTick for the given buffers (device: stack state, servo state [69][B], q_d [B][12 K]; host q or None)."""
+        return ServoStackTick(int(K), int(gait_mode), float(y_offset), _ptr(stack_state_d), _ptr(servo_state_d), _ptr(q_d), _ptr(q),
+                              _ptr(jac_d), _ptr(foot_des_d), _ptr(iters_d))
+
+    def servo_stack_tick(self, B, K, gait_mode, y_offset, stack_state_d, servo_state_d, q_d, q=None, jac_d=None, foot_des_d=None,
+                         iters_d=None, stream=None):
+        """go1mpc_servo_stack_tick_async: K consecutive 1 kHz servo ticks (filters + leg IK) on the gait stack state; joint
+        targets into q_d [B][12 K] (and the host q when given).  Returns after enqueueing on `stream` (None = the handle's)."""
+        t = self.servo_stack_tick_struct(K, gait_mode, y_offset, stack_state_d, servo_state_d, q_d, q, jac_d, foot_des_d, iters_d)
+        self._check(self.lib.go1mpc_servo_stack_tick_async(self.h, B, ctypes.byref(t), stream), "servo_stack_tick_async")
 
     def measure_dfma_peak(self, ms=200):
         g = ctypes.c_double(0.0)

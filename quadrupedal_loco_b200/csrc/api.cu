@@ -1486,6 +1486,37 @@ int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick
   return GO1MPC_OK;
 }
 
+// ------------------------------------------------------------------ servo stack tick: K 1 kHz servo ticks from the resident messages
+static_assert(GO1MPC_SERVO_TICKS_MAX == SERVO_TICKS_MAX && GO1MPC_SERVO_STATE_ROWS == SERVO_STATE_ROWS &&
+              GO1MPC_SERVO_ROW_Q == SERVO_ROW_Q && GO1MPC_SERVO_ROW_HOMING == SERVO_ROW_HOMING && GO1MPC_SERVO_ROW_LPF == SERVO_ROW_LPF,
+              "servo stack state layout");
+int go1mpc_servo_stack_tick_async(go1mpc_t* h, int B, const Go1ServoStackTick* t, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
+  if (!t || !t->stack_state_d || !t->servo_state_d || !t->q_d) return fail(h, GO1MPC_E_INVALID, "servo_stack_tick_async: bad argument");
+  if (t->K < 1 || t->K > GO1MPC_SERVO_TICKS_MAX) return fail(h, GO1MPC_E_INVALID, "servo_stack_tick_async: 1 <= K <= 10");
+  if ((uintptr_t)t->q_d & 7) return fail(h, GO1MPC_E_INVALID, "servo_stack_tick_async: q_d must be 8-byte aligned");
+  if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, "servo_stack_tick_async: gait_mode 101, 102 or 103");
+  CU(h, cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  const size_t b = (size_t)B;
+  ServoStackKParams P;
+  P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
+  P.half_hip_width = h->cfg.step.half_hip_width; P.y_offset = t->y_offset;
+  double k6[6];
+  go1mpc_lpf_coefficients(1000.0, 3.0, k6);                     // the servo loop's 3 Hz filters at 1 kHz
+  P.coef = LpfCoef{k6[0], k6[1], k6[2], k6[3], k6[4], k6[5]};
+  P.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
+  P.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
+  P.state = t->servo_state_d; P.q_out = t->q_d;
+  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d;
+  CU(h, servo_stack_launch(P, st));
+  h->launches++;
+  if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, b * 12 * t->K * sizeof(double), cudaMemcpyDeviceToHost, st));
+  return GO1MPC_OK;
+}
+
 // ------------------------------------------------------------------ pipelined host entries
 int go1mpc_body_mpc_step_batch_host_async(go1mpc_t* h, int nh, int B, const double* in, double* out, int* diag) {
   if (!h) return GO1MPC_E_INVALID;

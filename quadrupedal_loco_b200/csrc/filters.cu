@@ -9,6 +9,7 @@
 // bound.  Compiled with -fmad=false, the reference's left-to-right sums: bit-identical to the CPU oracle.
 #include <cuda_runtime.h>
 #include "kernels.h"
+#include "servo_math.cuh"   // lpf_step
 
 namespace go1 {
 
@@ -20,16 +21,11 @@ __global__ void __launch_bounds__(256) lpf_kernel(LpfKParams P) {
     const double* in = P.in + (size_t)(P.in_rows ? P.in_rows[c] : c) * B + b;
     double* S = P.state + t;
     const double y = *in;
-    const double i = S[0], y_p = S[CB], y_pp = S[2 * CB], x_p = S[3 * CB], x_pp = S[4 * CB];
-    const LpfCoef k = P.coef[c];
-    double out;
-    if (i > 2) {
-      out = k.b0 * y + k.b1 * y_p + k.b2 * y_pp + k.a1 * x_p + k.a2 * x_pp;
-    } else {
-      out = x_p + k.a * (y - x_p);
-      S[0] = i + 1;
-    }
-    S[2 * CB] = y_p; S[CB] = y; S[4 * CB] = x_p; S[3 * CB] = out;
+    LpfState s{S[0], S[CB], S[2 * CB], S[3 * CB], S[4 * CB]};
+    const bool counting = !(s.i > 2);
+    const double out = lpf_step(P.coef[c], s, y);
+    if (counting) S[0] = s.i;
+    S[2 * CB] = s.y_pp; S[CB] = s.y_p; S[4 * CB] = s.x_pp; S[3 * CB] = s.x_p;
     P.out[t] = out;
   }
 }

@@ -255,6 +255,23 @@ cudaError_t gait_stack_pre_launch(int B, int planner, double* walkdtime_row, int
 cudaError_t gait_stack_pack_launch(const GaitStackSlots& S, int B, const double* gait, const double* traj, double* rows, int sms,
                                    cudaStream_t st);
 
+// ---- the servo stack tick: K consecutive 1 kHz servo ticks from the gait stack's messages (servo_stack.cu) ----
+constexpr int SERVO_TICKS_MAX = 10, SERVO_LPF_CHANNELS = 9;
+constexpr int SERVO_ROW_Q = 0, SERVO_ROW_HOMING = 12, SERVO_ROW_LPF = 24, SERVO_STATE_ROWS = 24 + 5 * SERVO_LPF_CHANNELS;
+struct ServoStackKParams {
+  int B, K, gait_mode;
+  double half_hip_width, y_offset;
+  LpfCoef coef;                 // the 9 channels' filter (3 Hz at 1 kHz)
+  const double* gait;           // [100][B] /MPC/Gait: slots 0 1 2 6 7 8 9 10 11 through the filters
+  const double* traj;           // [100][B] /rtMPC/traj: slots 72, 73 = roll, pitch
+  double* state;                // [SERVO_STATE_ROWS][B] in/out: q | homing | filters [5][9][B]
+  double* q_out;                // [B][12 K] joint targets, tick-major per robot
+  double* jac;                  // [36][B] or null (last tick)
+  double* foot_des;             // [12][B] or null (last tick)
+  int* iters;                   // [4][B] or null (last tick)
+};
+cudaError_t servo_stack_launch(const ServoStackKParams& P, cudaStream_t st);
+
 // register-resident DFMA loop: flops executed are returned through *flops
 cudaError_t dfma_peak_launch(int grid, int block, int iters, double* sink, cudaStream_t st);
 

@@ -14,69 +14,19 @@
 // (FK: 4 + 8*(3+6) B in, 8*12 B out per leg), sincos-bound in practice.
 #include <cuda_runtime.h>
 #include "kernels.h"
+#include "servo_math.cuh"   // fk / Jacobian / Newton step, the servo leg stage
 
 namespace go1 {
 
 namespace {
-constexpr double L_THIGH = -0.213, L_CALF = -0.213;
-
-struct LegC { double ox, oy, ty; };
-__device__ __forceinline__ LegC leg_consts(int leg) {
-  LegC c;
-  c.ox = (leg == 0 || leg == 1) ? 0.1881 : -0.1881;
-  c.oy = (leg == 0 || leg == 2) ? -0.04675 : 0.04675;
-  c.ty = (leg == 0 || leg == 2) ? -0.08 : 0.08;
-  return c;
-}
-__device__ __forceinline__ void fk_hip(const double q[3], const LegC& c, double pos[3], double J[9]) {
-  double s1, c1, s2, c2, s3, c3;
-  sincos(q[0], &s1, &c1); sincos(q[1], &s2, &c2); sincos(q[2], &s3, &c3);
-  const double s23 = c3 * s2 + c2 * s3, c23 = c3 * c2 - s3 * s2;
-  const double K = L_CALF * s23 + L_THIGH * s2;
-  const double L = L_CALF * c23 + L_THIGH * c2;
-  pos[0] = c.ox + K;
-  pos[1] = c.oy + c.ty * c1 - s1 * L;
-  pos[2] = c.ty * s1 + c1 * L;
-  J[0] = 0.0;                     J[1] = L;        J[2] = L_CALF * c23;
-  J[3] = -(c.ty * s1 + c1 * L);   J[4] = s1 * K;   J[5] = s1 * (L_CALF * s23);
-  J[6] = c.ty * c1 - s1 * L;      J[7] = -c1 * K;  J[8] = -c1 * (L_CALF * s23);
-}
-struct Body { bool on; double p[3], R[9]; };
-__device__ __forceinline__ void fk_any(const double q[3], const LegC& c, const Body& bd, double pos[3], double J[9]) {
-  if (!bd.on) { fk_hip(q, c, pos, J); return; }
-  double pl[3], Jl[9];
-  fk_hip(q, c, pl, Jl);
-#pragma unroll
-  for (int i = 0; i < 3; i++) {
-    pos[i] = bd.p[i] + (bd.R[3 * i] * pl[0] + bd.R[3 * i + 1] * pl[1] + bd.R[3 * i + 2] * pl[2]);
-#pragma unroll
-    for (int j = 0; j < 3; j++) J[3 * i + j] = bd.R[3 * i] * Jl[j] + bd.R[3 * i + 1] * Jl[3 + j] + bd.R[3 * i + 2] * Jl[6 + j];
-  }
-}
 __device__ __forceinline__ Body load_body(const double* bp, const double* br, size_t B, int b) {
   Body bd;
   bd.on = (bp != nullptr);
   if (bd.on) {
-    double sr, cr, sp, cp, sy, cy;
     for (int k = 0; k < 3; k++) bd.p[k] = bp[k * B + b];
-    sincos(br[b], &sr, &cr); sincos(br[B + b], &sp, &cp); sincos(br[2 * B + b], &sy, &cy);
-    bd.R[0] = cp * cy; bd.R[1] = cy * sp * sr - cr * sy; bd.R[2] = sr * sy + cr * cy * sp;
-    bd.R[3] = cp * sy; bd.R[4] = cr * cy + sp * sr * sy; bd.R[5] = cr * sp * sy - cy * sr;
-    bd.R[6] = -sp;     bd.R[7] = cp * sr;                bd.R[8] = cp * cr;
+    body_rotation(br[b], br[B + b], br[2 * B + b], bd.R);
   }
   return bd;
-}
-// dq = lamda J^-1 dp by cofactors
-__device__ __forceinline__ void newton_step(const double J[9], const double dp[3], double lamda, double dq[3]) {
-  const double c00 = J[4] * J[8] - J[5] * J[7], c01 = J[5] * J[6] - J[3] * J[8], c02 = J[3] * J[7] - J[4] * J[6];
-  const double det = J[0] * c00 + J[1] * c01 + J[2] * c02;
-  const double id = 1.0 / det;
-  const double i00 = c00 * id, i01 = (J[2] * J[7] - J[1] * J[8]) * id, i02 = (J[1] * J[5] - J[2] * J[4]) * id;
-  const double i10 = c01 * id, i11 = (J[0] * J[8] - J[2] * J[6]) * id, i12 = (J[2] * J[3] - J[0] * J[5]) * id;
-  const double i20 = c02 * id, i21 = (J[1] * J[6] - J[0] * J[7]) * id, i22 = (J[0] * J[4] - J[1] * J[3]) * id;
-  dq[0] = (lamda * i00) * dp[0] + (lamda * i01) * dp[1] + (lamda * i02) * dp[2];
-  dq[1] = (lamda * i10) * dp[0] + (lamda * i11) * dp[1] + (lamda * i12) * dp[2];
-  dq[2] = (lamda * i20) * dp[0] + (lamda * i21) * dp[1] + (lamda * i22) * dp[2];
 }
 }  // namespace
 
@@ -133,36 +83,20 @@ __global__ void __launch_bounds__(256) servo_kin_kernel(ServoKParams P) {
   if (idx >= 4 * P.B) return;
   const int b = idx >> 2, leg = idx & 3;
   const size_t B = (size_t)P.B;
-  // which virtual foot this leg follows: bit `leg` of the mask set = right foot
-  const unsigned right_mask = (P.gait_mode == 101) ? 0x5u : ((P.gait_mode == 102) ? 0x9u : 0x3u);   // FR=0, FL=1, RR=2, RL=3
-  const bool right = (right_mask >> leg) & 1u;
+  const bool right = servo_follows_right(P.gait_mode, leg);
   const double* vf = right ? P.rfoot : P.lfoot;
+  const double hom[3] = {P.homing[(size_t)(3 * leg) * B + b], P.homing[(size_t)(3 * leg + 1) * B + b], P.homing[(size_t)(3 * leg + 2) * B + b]};
+  const double v[3] = {vf[b], vf[B + b], vf[2 * B + b]};
   double pdes[3];
-  for (int k = 0; k < 3; k++) pdes[k] = P.homing[(size_t)(3 * leg + k) * B + b] + vf[(size_t)k * B + b];
-  pdes[1] = P.homing[(size_t)(3 * leg + 1) * B + b] + vf[B + b] + (right ? P.half_hip_width : -P.half_hip_width);
+  servo_leg_target(hom, v, right, P.half_hip_width, pdes);
   const LegC c = leg_consts(leg);
   Body bd;
   bd.on = true;
-  {
-    double sr, cr, sp, cp, sy, cy;
-    bd.p[0] = P.com[b]; bd.p[1] = P.com[B + b] * P.y_offset; bd.p[2] = P.com[2 * B + b];
-    sincos(P.theta[b], &sr, &cr); sincos(P.theta[B + b], &sp, &cp); sincos(P.theta[2 * B + b], &sy, &cy);
-    bd.R[0] = cp * cy; bd.R[1] = cy * sp * sr - cr * sy; bd.R[2] = sr * sy + cr * cy * sp;
-    bd.R[3] = cp * sy; bd.R[4] = cr * cy + sp * sr * sy; bd.R[5] = cr * sp * sy - cy * sr;
-    bd.R[6] = -sp;     bd.R[7] = cp * sr;                bd.R[8] = cp * cr;
-  }
+  bd.p[0] = P.com[b]; bd.p[1] = P.com[B + b] * P.y_offset; bd.p[2] = P.com[2 * B + b];
+  body_rotation(P.theta[b], P.theta[B + b], P.theta[2 * B + b], bd.R);
   double q[3] = {P.q[(size_t)(3 * leg) * B + b], P.q[(size_t)(3 * leg + 1) * B + b], P.q[(size_t)(3 * leg + 2) * B + b]};
-  double pc[3], J[9], dp[3], dq[3];
-  fk_any(q, c, bd, pc, J);
-  int it = 0;
-  for (int j = 0; j < 15; j++) {
-    for (int k = 0; k < 3; k++) dp[k] = pdes[k] - pc[k];
-    newton_step(J, dp, 0.5, dq);
-    if (fabs(dp[0] * dp[0] + dp[1] * dp[1] + dp[2] * dp[2]) <= 0.000001) break;
-    q[0] += dq[0]; q[1] += dq[1]; q[2] += dq[2];
-    fk_any(q, c, bd, pc, J);
-    it++;
-  }
+  double J[9];
+  const int it = servo_leg_ik(c, bd, pdes, q, J);
   for (int k = 0; k < 3; k++) P.q[(size_t)(3 * leg + k) * B + b] = q[k];
   if (P.jac) for (int k = 0; k < 9; k++) P.jac[(size_t)(9 * leg + k) * B + b] = J[k];
   if (P.foot_des) for (int k = 0; k < 3; k++) P.foot_des[(size_t)(3 * leg + k) * B + b] = pdes[k];
