@@ -680,6 +680,59 @@ int go1mpc_gait_stack_default_state(go1mpc_t *h, int nh, double *column);
 int go1mpc_gait_stack_tick_host_async(go1mpc_t *h, int B, const Go1GaitStackTick *t, void *stream);
 
 /* ---------------------------------------------------------------------------
+ * Gait stack with per-robot clocks and on-device resets: one batch holds robots at arbitrary points of their episodes (Monte-Carlo /
+ * RL farms), and each robot's run is bit-identical to a fresh run of that robot started at its reset.
+ *
+ * go1mpc_gait_stack_tick_clocked_async: go1mpc_gait_stack_tick_host_async with the planner flag taken per robot from
+ *   clock_d  device [B] ints, in/out, caller-owned: 10 ms periods since the robot's reset (zero-initialise a fresh batch).
+ *   Robot b with clock c plans in this call when c == 0 or (10c)/25 > (10(c-1))/25 (c = 0, 3, 5, 8, 10, ...: the reference's
+ *   schedule, run on the robot's own time); its clock is c + 1 after the call.  walkdtime += 1 only for the robots that plan.  A robot
+ *   that does not plan leaves the planner node's rows, /MPC/Gait and walkdtime untouched; the 100 Hz node, the pack and the copy to
+ *   `rows` run for every robot.  cmd / start are uploaded whenever given and read only for the robots that plan.  The planner node's
+ *   kernels are enqueued on every call (robots that do not plan exit at once), so every call enqueues the same work and one captured
+ *   period graph replays for all periods.  Errors: those of go1mpc_gait_stack_tick_host_async, and GO1MPC_E_INVALID for a NULL
+ *   clock_d; nothing is enqueued on an error.  B = 0 is a no-op.
+ *
+ * go1mpc_gait_stack_reset_async: for every robot b with reset[b] != 0 (reset: host [B] ints, pinned so the call can sit in a graph,
+ *   uploaded by the call):
+ *     the column b of state_d = go1mpc_gait_stack_default_state(nh);  body_out_d record b = 0;  clock_d[b] = 0;
+ *     when servo_state_d is given: rows GO1MPC_SERVO_ROW_Q..+12 = servo_q0, the 45 filter rows = 0 (the homing rows are the
+ *     caller's input and stay).
+ *   Other robots are not touched.  Two kernel launches of a fixed shape; the flagged robots are listed on the device, so the
+ *   flags never change what is enqueued, and the work grows with the number of robots flagged.  The default column is built once
+ *   per (handle, nh), with a synchronous upload, and kept on the device: the first reset call with each nh must come before any
+ *   graph capture.  Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL reset / clock_d / state_d / body_out_d or
+ *   body_out_d not 16-byte aligned, GO1MPC_E_UNSUPPORTED for nh outside 3..40.
+ *
+ * Both entries allocate only on their first call with a given (stream, B) (and, for the reset, nh), so a warmed-up period
+ *   reset -> clocked tick -> go1mpc_servo_stack_tick_async can be captured once with go1mpc_graph_capture_* and replayed every period,
+ *   the caller rewriting the pinned sensor and reset buffers between replays.
+ * ------------------------------------------------------------------------ */
+typedef struct {
+  int nh;                    /* body-MPC horizon, 3..40 */
+  const double *sensor;      /* host [11][B] SoA, as Go1GaitStackTick */
+  const int *cmd, *start;    /* host [B] or NULL; read only for the robots that plan in this call */
+  double *state_d;           /* device [go1mpc_gait_stack_state_doubles(nh)][B] SoA, in/out */
+  double *body_out_d;        /* device [B][go1mpc_body_out_stride(nh)], in/out, zero-initialised, 16-byte aligned */
+  int n_slots;
+  int slots[GO1MPC_STACK_SLOTS_MAX];   /* as Go1GaitStackTick */
+  double *rows_d;            /* device [B][n_slots] */
+  double *rows;              /* host [B][n_slots] or NULL */
+  int *clock_d;              /* device [B] ints, in/out: periods since each robot's reset */
+} Go1GaitStackClockedTick;
+int go1mpc_gait_stack_tick_clocked_async(go1mpc_t *h, int B, const Go1GaitStackClockedTick *t, void *stream);
+typedef struct {
+  int nh;
+  const int *reset;          /* host [B] ints (pinned): non-zero = reset this robot */
+  int *clock_d;              /* device [B], as Go1GaitStackClockedTick */
+  double *state_d;           /* device [go1mpc_gait_stack_state_doubles(nh)][B] */
+  double *body_out_d;        /* device [B][go1mpc_body_out_stride(nh)], 16-byte aligned */
+  double *servo_state_d;     /* device [GO1MPC_SERVO_STATE_ROWS][B] or NULL */
+  double servo_q0[12];       /* joint angles (FR, FL, RR, RL) a reset robot's servo starts from */
+} Go1GaitStackReset;
+int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r, void *stream);
+
+/* ---------------------------------------------------------------------------
  * Servo stack tick: K consecutive ticks of go1_servo's 1 kHz loop for B robots in ONE call, fed in place from the messages the
  * gait stack keeps resident -- the call a controller farm makes after each gait stack call (K = 10 per 10 ms period), joint
  * targets out.  Per robot b and tick k = 1..K:

@@ -34,7 +34,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_nlp_node_tick_batch", "go1mpc_foot_trajectory_stop_batch", "go1mpc_nlp_node_tick_batch_host", "go1mpc_rt_node_tick_batch_host", "go1mpc_foot_trajectory_stop_batch_host",
     "go1mpc_grf_force_opt_batch_host", "go1mpc_grf_force_distribution_batch_host", "go1mpc_grf_joint_torques_batch_host", "go1mpc_leg_fk_batch_host", "go1mpc_leg_ik_batch_host",
     "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
-    "go1mpc_servo_stack_tick_async",
+    "go1mpc_servo_stack_tick_async", "go1mpc_gait_stack_tick_clocked_async", "go1mpc_gait_stack_reset_async",
 ]
 
 
@@ -169,6 +169,8 @@ def load_library():
     lib.go1mpc_gait_stack_default_state.argtypes = [vp, ctypes.c_int, vp]
     lib.go1mpc_gait_stack_tick_host_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackTick), vp]
     lib.go1mpc_servo_stack_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoStackTick), vp]
+    lib.go1mpc_gait_stack_tick_clocked_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackClockedTick), vp]
+    lib.go1mpc_gait_stack_reset_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackReset), vp]
     _LIB = lib
     return lib
 
@@ -269,6 +271,20 @@ class GaitStackTick(ctypes.Structure):
                 ("start", ctypes.c_void_p), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p),
                 ("n_slots", ctypes.c_int), ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p),
                 ("rows", ctypes.c_void_p)]
+
+
+class GaitStackClockedTick(ctypes.Structure):
+    """Go1GaitStackClockedTick of include/go1mpc.h."""
+    _fields_ = [("nh", ctypes.c_int), ("sensor", ctypes.c_void_p), ("cmd", ctypes.c_void_p), ("start", ctypes.c_void_p),
+                ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p), ("n_slots", ctypes.c_int),
+                ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p), ("rows", ctypes.c_void_p),
+                ("clock_d", ctypes.c_void_p)]
+
+
+class GaitStackReset(ctypes.Structure):
+    """Go1GaitStackReset of include/go1mpc.h."""
+    _fields_ = [("nh", ctypes.c_int), ("reset", ctypes.c_void_p), ("clock_d", ctypes.c_void_p), ("state_d", ctypes.c_void_p),
+                ("body_out_d", ctypes.c_void_p), ("servo_state_d", ctypes.c_void_p), ("servo_q0", ctypes.c_double * 12)]
 
 
 SERVO_TICKS_MAX = 10      # GO1MPC_SERVO_TICKS_MAX
@@ -597,6 +613,34 @@ class Go1Mpc:
         """go1mpc_gait_stack_tick_host_async with a GaitStackTick (gait_stack_tick_struct); returns after enqueueing on `stream`
         (None = the handle's)."""
         self._check(self.lib.go1mpc_gait_stack_tick_host_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_host_async")
+
+    def gait_stack_tick_clocked_struct(self, nh, sensor, clock_d, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None):
+        """Go1GaitStackClockedTick for the given buffers (device clock_d [B] int32: periods since each robot's reset)."""
+        t = GaitStackClockedTick(nh, _ptr(sensor), _ptr(cmd), _ptr(start), _ptr(state_d), _ptr(body_out_d), len(slots))
+        for k, v in enumerate(slots[:STACK_SLOTS_MAX]):
+            t.slots[k] = int(v)
+        t.rows_d = _ptr(rows_d)
+        t.rows = _ptr(rows)
+        t.clock_d = _ptr(clock_d)
+        return t
+
+    def gait_stack_tick_clocked_async(self, B, t, stream=None):
+        """go1mpc_gait_stack_tick_clocked_async with a GaitStackClockedTick: each robot plans on its own clock; returns after
+        enqueueing on `stream` (None = the handle's)."""
+        self._check(self.lib.go1mpc_gait_stack_tick_clocked_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_clocked_async")
+
+    def gait_stack_reset_struct(self, nh, reset, clock_d, state_d, body_out_d, servo_state_d=None, servo_q0=None):
+        """Go1GaitStackReset for the given buffers (host reset [B] int32, pinned for graph capture; servo_q0: 12 joint angles)."""
+        r = GaitStackReset(nh, _ptr(reset), _ptr(clock_d), _ptr(state_d), _ptr(body_out_d), _ptr(servo_state_d))
+        if servo_q0 is not None:
+            q0 = np.asarray(servo_q0, dtype=np.float64).reshape(12)
+            for k in range(12):
+                r.servo_q0[k] = float(q0[k])
+        return r
+
+    def gait_stack_reset_async(self, B, r, stream=None):
+        """go1mpc_gait_stack_reset_async with a GaitStackReset: the flagged robots restart from the default state on the device."""
+        self._check(self.lib.go1mpc_gait_stack_reset_async(self.h, B, ctypes.byref(r), stream), "gait_stack_reset_async")
 
     # --- servo stack tick: K 1 kHz servo ticks from the gait stack's resident messages ---
     def servo_stack_tick_struct(self, K, gait_mode, y_offset, stack_state_d, servo_state_d, q_d, q=None, jac_d=None, foot_des_d=None,

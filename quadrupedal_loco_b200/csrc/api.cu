@@ -71,10 +71,11 @@ struct go1mpc {
   double* squat_d = nullptr;       // X_CoM_position_squat table of the planner node (host libm), built on first use
   struct NlpWs { DevBuf b[7]; };   // workspace of go1mpc_nlp_node_tick_batch, one per caller stream
   std::map<cudaStream_t, NlpWs> nlp_ws;
-  // workspace of go1mpc_gait_stack_tick_host_async, one per caller stream (grown on demand): sensor | /control2rtmpc/state |
-  // walkdtime ints | cmd | start | body-MPC input records
-  struct StackWs { DevBuf b[6]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
+  // workspace of the gait stack entries, one per caller stream (grown on demand): sensor | /control2rtmpc/state |
+  // walkdtime ints | cmd | start | body-MPC input records | planner mask of the clocked tick | reset count, flags and robot list
+  struct StackWs { DevBuf b[8]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
   std::map<cudaStream_t, StackWs> stack_ws;
+  std::map<int, double*> stack_col_d;   // go1mpc_gait_stack_default_state(nh) on the device, per nh, built on first use
   double* trtab_d = nullptr;       // remaining-time bound table of the planner tick (host libm), built on first use
   std::vector<cudaEvent_t> ev_pool;   // go1mpc_stream_wait: events, reused round-robin
   unsigned ev_next = 0;
@@ -335,6 +336,7 @@ void go1mpc_destroy(go1mpc_t* h) {
   for (cudaEvent_t e : h->phase_ev) if (e) cudaEventDestroy(e);
   for (auto& kv : h->nlp_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
   for (auto& kv : h->stack_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
+  for (auto& kv : h->stack_col_d) cudaFree(kv.second);
   for (auto& L : h->lanes) {
     for (DevBuf& b : L.stage) if (b.p) cudaFree(b.p);
     if (L.stream) cudaStreamDestroy(L.stream);
@@ -1204,8 +1206,18 @@ int go1mpc_nlp_node_default_state(go1mpc_t* h, double* s) {
   return GO1MPC_OK;
 }
 
+namespace {
+int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
+                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, void* stream);
+}
 int go1mpc_nlp_node_tick_batch(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
                                const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, void* stream) {
+  return nlp_node_enqueue(h, B, state_d, walkdtime_d, start_d, cmd_d, rfoot_fb_d, lfoot_fb_d, msg_d, nullptr, stream);
+}
+namespace {
+// active_d: [B] ints or null (= all); robots with 0 leave the node untouched (per-robot clocks of the gait stack)
+int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
+                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, void* stream) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B < 0 || !state_d || !walkdtime_d || !msg_d) return fail(h, GO1MPC_E_INVALID, "nlp_node_tick_batch: bad argument");
@@ -1246,6 +1258,7 @@ int go1mpc_nlp_node_tick_batch(go1mpc_t* h, int B, double* state_d, const int* w
   P.node = state_d; P.walkdtime = walkdtime_d; P.start = start_d; P.cmd = cmd_d; P.rfoot_fb = rfoot_fb_d; P.lfoot_fb = lfoot_fb_d;
   P.tick = (int*)W.b[0].p; P.in = (double*)W.b[1].p; P.out38 = (double*)W.b[2].p; P.out18 = (double*)W.b[3].p;
   P.right_support = (int*)W.b[4].p; P.hz_co = (double*)W.b[5].p; P.lipm = (double*)W.b[6].p; P.msg = msg_d;
+  P.active = active_d;
   CU(h, nlp_pre_launch(P, st));
   h->launches++;
   // the planner state is rows [0, 202) of the node, the swing-foot window rows [202, 234): same SoA stride B
@@ -1258,6 +1271,7 @@ int go1mpc_nlp_node_tick_batch(go1mpc_t* h, int B, double* state_d, const int* w
   h->launches++;
   return GO1MPC_OK;
 }
+}  // namespace
 
 // host form: SoA host buffers of the same shapes; state and msg are copied up, the tick runs, state and msg come down
 int go1mpc_nlp_node_tick_batch_host(go1mpc_t* h, int B, double* state, const int* walkdtime, const int* start, const int* cmd,
@@ -1421,36 +1435,40 @@ int go1mpc_gait_stack_default_state(go1mpc_t* h, int nh, double* s) {
   return go1mpc_rt_node_default_state(h, nh, s + GO1MPC_STACK_ROW_RT);
 }
 
-int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick* t, void* stream) {
-  if (!h) return GO1MPC_E_INVALID;
-  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+namespace {
+// The node sequence of both gait stack ticks.  clock_d == null: every robot gets t.planner (go1mpc_gait_stack_tick_host_async);
+// otherwise each robot's planner flag comes from its clock (go1mpc_gait_stack_tick_clocked_async), and the planner node is always
+// enqueued, with the robots that do not plan masked out -- the same launches every period, so one captured graph fits all.
+int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock_d, void* stream, const char* name) {
+  const std::string nm(name);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
-  if (!t || !t->sensor || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: bad argument");
+  if (!t || !t->sensor || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, nm + ": bad argument");
   const int nh = t->nh, n = t->n_slots;
-  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_tick_host_async: 3 <= nh <= 40");
+  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, nm + ": 3 <= nh <= 40");
   if (h->cfg.step.ext_height)
-    return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_tick_host_async: cfg.step.ext_height must be 0 (the planner node owns CoM_height_solve)");
-  if (n < 1 || n > GO1MPC_STACK_SLOTS_MAX) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: 1 <= n_slots <= 64");
+    return fail(h, GO1MPC_E_UNSUPPORTED, nm + ": cfg.step.ext_height must be 0 (the planner node owns CoM_height_solve)");
+  if (n < 1 || n > GO1MPC_STACK_SLOTS_MAX) return fail(h, GO1MPC_E_INVALID, nm + ": 1 <= n_slots <= 64");
   GaitStackSlots S;
   S.n = n;
   for (int k = 0; k < GO1MPC_STACK_SLOTS_MAX; k++) {
     S.slot[k] = k < n ? t->slots[k] : 0;
-    if (S.slot[k] < 0 || S.slot[k] >= 200) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: slots must lie in 0..199");
+    if (S.slot[k] < 0 || S.slot[k] >= 200) return fail(h, GO1MPC_E_INVALID, nm + ": slots must lie in 0..199");
   }
   // the body kernels read and write body_out_d with 16-byte loads / TMA; the pack kernel stores doubles into rows_d
   if (((uintptr_t)t->body_out_d & 15) || ((uintptr_t)t->rows_d & 7))
-    return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_host_async: body_out_d must be 16-byte and rows_d 8-byte aligned");
+    return fail(h, GO1MPC_E_INVALID, nm + ": body_out_d must be 16-byte and rows_d 8-byte aligned");
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
     return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
   go1mpc::StackWs& W = h->stack_ws[st];
   const size_t b = (size_t)B;
-  const size_t bytes[6] = {b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), b * 25 * sizeof(double), b * sizeof(int), b * sizeof(int),
-                           b * sizeof(int), b * go1mpc_body_in_stride(nh) * sizeof(double)};
-  void* d[6];
+  const int nbuf = clock_d ? 7 : 6;
+  const size_t bytes[7] = {b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), b * 25 * sizeof(double), b * sizeof(int), b * sizeof(int),
+                           b * sizeof(int), b * go1mpc_body_in_stride(nh) * sizeof(double), b * sizeof(int)};
+  void* d[7] = {};
   int rc;
-  for (int k = 0; k < 6; k++) {
+  for (int k = 0; k < nbuf; k++) {
     const bool grow = bytes[k] > W.b[k].cap;
     if (grow) CU(h, cudaStreamSynchronize(st));     // growing: earlier work on this stream may still use the old buffer
     if ((rc = stage_buf2(h, W.b[k], bytes[k], &d[k]))) return rc;
@@ -1464,18 +1482,26 @@ int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick
   }
   double* state = t->state_d;
   CU(h, cudaMemcpyAsync(d[0], t->sensor, bytes[0], cudaMemcpyHostToDevice, st));
+  // with per-robot clocks some robot may plan in any call, so cmd / start go up whenever they are given
+  const bool planner = clock_d || t->planner;
   const int* cmd_d = nullptr;
   const int* start_d = nullptr;
-  if (t->planner && t->cmd) { CU(h, cudaMemcpyAsync(d[3], t->cmd, bytes[3], cudaMemcpyHostToDevice, st)); cmd_d = (const int*)d[3]; }
-  if (t->planner && t->start) { CU(h, cudaMemcpyAsync(d[4], t->start, bytes[4], cudaMemcpyHostToDevice, st)); start_d = (const int*)d[4]; }
-  CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl, h->sms, st));
+  if (planner && t->cmd) { CU(h, cudaMemcpyAsync(d[3], t->cmd, bytes[3], cudaMemcpyHostToDevice, st)); cmd_d = (const int*)d[3]; }
+  if (planner && t->start) { CU(h, cudaMemcpyAsync(d[4], t->start, bytes[4], cudaMemcpyHostToDevice, st)); start_d = (const int*)d[4]; }
+  int* plan_d = (int*)d[6];
+  if (clock_d)
+    CU(h, gait_stack_clocked_pre_launch(B, clock_d, plan_d, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl,
+                                        h->sms, st));
+  else
+    CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl,
+                                h->sms, st));
   h->launches++;
   double* gait = state + GO1MPC_STACK_ROW_GAIT * b;
   double* rt2nrt = state + GO1MPC_STACK_ROW_RT2NRT * b;
   double* traj = state + GO1MPC_STACK_ROW_TRAJ * b;
-  if (t->planner &&
-      (rc = go1mpc_nlp_node_tick_batch(h, B, state + GO1MPC_STACK_ROW_NLP * b, (const int*)d[2], start_d, cmd_d, rt2nrt + 22 * b,
-                                       rt2nrt + 19 * b, gait, st)))
+  if (planner &&
+      (rc = nlp_node_enqueue(h, B, state + GO1MPC_STACK_ROW_NLP * b, (const int*)d[2], start_d, cmd_d, rt2nrt + 22 * b, rt2nrt + 19 * b,
+                             gait, clock_d ? plan_d : nullptr, st)))
     return rc;
   if ((rc = rt_node_enqueue(h, nh, B, state + GO1MPC_STACK_ROW_RT * b, gait, nullptr, nullptr, ctl, (double*)d[5], t->body_out_d, nullptr,
                             traj, rt2nrt, nullptr, st)))
@@ -1483,6 +1509,68 @@ int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick
   CU(h, gait_stack_pack_launch(S, B, gait, traj, t->rows_d, h->sms, st));
   h->launches++;
   if (t->rows) CU(h, cudaMemcpyAsync(t->rows, t->rows_d, b * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+  return GO1MPC_OK;
+}
+}  // namespace
+
+int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick* t, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  return gait_stack_enqueue(h, B, t, nullptr, stream, "gait_stack_tick_host_async");
+}
+
+int go1mpc_gait_stack_tick_clocked_async(go1mpc_t* h, int B, const Go1GaitStackClockedTick* t, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
+  if (!t || !t->clock_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_clocked_async: bad argument");
+  Go1GaitStackTick u;
+  u.nh = t->nh; u.planner = 0; u.sensor = t->sensor; u.cmd = t->cmd; u.start = t->start; u.state_d = t->state_d;
+  u.body_out_d = t->body_out_d; u.n_slots = t->n_slots; u.rows_d = t->rows_d; u.rows = t->rows;
+  memcpy(u.slots, t->slots, sizeof u.slots);
+  return gait_stack_enqueue(h, B, &u, t->clock_d, stream, "gait_stack_tick_clocked_async");
+}
+
+int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
+  if (!r || !r->reset || !r->clock_d || !r->state_d || !r->body_out_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: bad argument");
+  const int nh = r->nh;
+  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_reset_async: 3 <= nh <= 40");
+  if ((uintptr_t)r->body_out_d & 15) return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: body_out_d must be 16-byte aligned");
+  CU(h, cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  const int rows = go1mpc_gait_stack_state_doubles(nh);
+  auto it = h->stack_col_d.find(nh);
+  if (it == h->stack_col_d.end()) {
+    std::vector<double> col(rows);
+    int rc = go1mpc_gait_stack_default_state(h, nh, col.data());
+    if (rc) return rc;
+    double* p = nullptr;
+    CU(h, cudaMalloc((void**)&p, sizeof(double) * rows));
+    cudaError_t e = cudaMemcpy(p, col.data(), sizeof(double) * rows, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { cudaFree(p); return cuda_fail(h, e, "cudaMemcpy(default gait stack column)"); }
+    it = h->stack_col_d.emplace(nh, p).first;
+  }
+  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
+    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
+  go1mpc::StackWs& W = h->stack_ws[st];
+  // {count, 3 pad, flags[B], list[B]}
+  const size_t b = (size_t)B, bytes = (4 + 2 * b) * sizeof(int);
+  if (bytes > W.b[7].cap) CU(h, cudaStreamSynchronize(st));
+  void* ws;
+  int rc;
+  if ((rc = stage_buf2(h, W.b[7], bytes, &ws))) return rc;
+  StackResetParams P;
+  P.B = B; P.rows = rows; P.out_stride = go1mpc_body_out_stride(nh);
+  P.count = (int*)ws; P.reset = P.count + 4; P.list = P.count + 4 + B;
+  P.clock = r->clock_d; P.state = r->state_d; P.column = it->second; P.body_out = r->body_out_d; P.servo = r->servo_state_d;
+  memcpy(P.q0, r->servo_q0, sizeof P.q0);
+  CU(h, cudaMemcpyAsync((void*)P.reset, r->reset, b * sizeof(int), cudaMemcpyHostToDevice, st));
+  CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
+  CU(h, gait_stack_reset_launch(P, h->sms, st));
+  h->launches += 2;
   return GO1MPC_OK;
 }
 

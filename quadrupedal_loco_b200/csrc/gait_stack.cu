@@ -1,9 +1,13 @@
-// gait_stack.cu -- the two copy kernels of the gait stack tick (go1mpc_gait_stack_tick_host_async): both MPC nodes of the
-// reference behind one host call, everything the nodes keep as members resident in one SoA state [row][B].
+// gait_stack.cu -- the copy kernels of the gait stack ticks (go1mpc_gait_stack_tick_host_async, go1mpc_gait_stack_tick_clocked_async)
+// and the robot reset (go1mpc_gait_stack_reset_async): both MPC nodes of the reference behind one host call, everything the nodes
+// keep as members resident in one SoA state [row][B].
 //
 //   gait_stack_pre_kernel  : when the planner ticks, walkdtime += 1 in the state (kept as an exact integer double) and as the
 //                            int the planner node reads; the 11 uploaded sensor rows -> their slots of /control2rtmpc/state
 //   gait_stack_pack_kernel : the selected slots of /MPC/Gait and /rtMPC/traj -> one row of n_slots doubles per robot
+//   gait_stack_clocked_pre_kernel : per-robot clocks (periods since the robot's reset): whether each robot's planner ticks this
+//                            call, into a mask the planner node reads; walkdtime += 1 for those robots; clock += 1; the sensor scatter
+//   gait_stack_reset_mark_kernel / gait_stack_reset_column_kernel : robot resets, see below
 // Thread per robot (pre) / per output double (pack): every warp access is coalesced over B.
 #include "kernels.h"
 
@@ -13,6 +17,16 @@ namespace {
 // /control2rtmpc/state slot of uploaded sensor row k: 0 | 10 11 13 14 | 19 20 21 | 22 23 24 (flag | body angles / rates |
 // left foot xyz | right foot xyz)
 __device__ __forceinline__ constexpr int sensor_slot(int k) { return k == 0 ? 0 : (k < 3 ? 9 + k : (k < 5 ? 10 + k : 14 + k)); }
+
+__device__ __forceinline__ void scatter_sensors(size_t b, size_t Bs, const double* __restrict__ sensor, double* __restrict__ ctl) {
+#pragma unroll
+  for (int k = 0; k < GAIT_STACK_SENSOR_ROWS; k++) ctl[(size_t)sensor_slot(k) * Bs + b] = sensor[(size_t)k * Bs + b];
+}
+__device__ __forceinline__ void bump_walkdtime(size_t b, double* __restrict__ walkdtime_row, int* __restrict__ walkdtime_i) {
+  const double w = walkdtime_row[b] + 1.0;
+  walkdtime_row[b] = w;
+  walkdtime_i[b] = (int)w;
+}
 }  // namespace
 
 __global__ void __launch_bounds__(256) gait_stack_pre_kernel(int B, int planner, double* __restrict__ walkdtime_row,
@@ -20,13 +34,24 @@ __global__ void __launch_bounds__(256) gait_stack_pre_kernel(int B, int planner,
                                                              double* __restrict__ ctl) {
   const size_t Bs = (size_t)B;
   for (size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x; b < Bs; b += (size_t)gridDim.x * blockDim.x) {
-    if (planner) {
-      const double w = walkdtime_row[b] + 1.0;
-      walkdtime_row[b] = w;
-      walkdtime_i[b] = (int)w;
-    }
-#pragma unroll
-    for (int k = 0; k < GAIT_STACK_SENSOR_ROWS; k++) ctl[(size_t)sensor_slot(k) * Bs + b] = sensor[(size_t)k * Bs + b];
+    if (planner) bump_walkdtime(b, walkdtime_row, walkdtime_i);
+    scatter_sensors(b, Bs, sensor, ctl);
+  }
+}
+
+// The reference's clock, per robot: the fast tick at 10c ms after the robot's reset runs the planner first when a multiple of 25
+// lies in (10(c-1), 10c], i.e. c = 0, 3, 5, 8, 10, ... (c mod 5 in {0, 3}).  64-bit products: no overflow at any int clock.
+__global__ void __launch_bounds__(256) gait_stack_clocked_pre_kernel(int B, int* __restrict__ clock, int* __restrict__ plan,
+                                                                     double* __restrict__ walkdtime_row, int* __restrict__ walkdtime_i,
+                                                                     const double* __restrict__ sensor, double* __restrict__ ctl) {
+  const size_t Bs = (size_t)B;
+  for (size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x; b < Bs; b += (size_t)gridDim.x * blockDim.x) {
+    const long long c = clock[b];
+    const int p = (c == 0 || (10 * c) / 25 > (10 * (c - 1)) / 25) ? 1 : 0;
+    plan[b] = p;
+    if (p) bump_walkdtime(b, walkdtime_row, walkdtime_i);
+    clock[b] = (int)(c + 1);
+    scatter_sensors(b, Bs, sensor, ctl);
   }
 }
 
@@ -40,6 +65,45 @@ __global__ void __launch_bounds__(256) gait_stack_pack_kernel(GaitStackSlots S, 
   }
 }
 
+// ---- robot resets.  Thread per robot: the flagged robots are appended to a list with one atomic per warp, and get their small
+// writes here -- clock 0, the body-MPC record zeroed with 16-byte stores (records are 16-byte aligned, an even number of doubles),
+// the servo joint angles q0 and zero filter rows (the homing rows are the caller's input and stay).  Every lane reaches the ballot:
+// the grid covers B exactly, lanes past B vote 0.
+__global__ void __launch_bounds__(256) gait_stack_reset_mark_kernel(StackResetParams P) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool flag = b < P.B && P.reset[b] != 0;
+  const unsigned m = __ballot_sync(0xffffffffu, flag);
+  if (!m) return;
+  const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+  int base = 0;
+  if (lane == leader) base = atomicAdd(P.count, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  if (!flag) return;
+  P.list[base + __popc(m & ((1u << lane) - 1))] = b;
+  P.clock[b] = 0;
+  double2* rec = reinterpret_cast<double2*>(P.body_out + (size_t)b * P.out_stride);
+  const double2 z = make_double2(0.0, 0.0);
+  for (int k = 0; k < P.out_stride / 2; k++) rec[k] = z;
+  if (P.servo) {
+    const size_t Bs = (size_t)P.B;
+    double* S = P.servo + b;
+#pragma unroll
+    for (int k = 0; k < 12; k++) S[(size_t)(SERVO_ROW_Q + k) * Bs] = P.q0[k];
+#pragma unroll 5
+    for (int k = SERVO_ROW_LPF; k < SERVO_STATE_ROWS; k++) S[(size_t)k * Bs] = 0.0;
+  }
+}
+
+// Grid-stride over (row, listed robot), robot-minor: the count is read on the device, so the launch does not depend on how many
+// robots reset, and a call with no reset costs one read of the count per thread.
+__global__ void __launch_bounds__(256) gait_stack_reset_column_kernel(StackResetParams P) {
+  const size_t n = (size_t)*P.count, total = n * (size_t)P.rows, Bs = (size_t)P.B;
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const size_t r = idx / n;
+    P.state[r * Bs + P.list[idx - r * n]] = P.column[r];
+  }
+}
+
 static int stack_grid(size_t total, int sms) {
   size_t g = (total + 255) / 256;
   const size_t cap = (size_t)sms * 8;
@@ -49,6 +113,18 @@ static int stack_grid(size_t total, int sms) {
 cudaError_t gait_stack_pre_launch(int B, int planner, double* walkdtime_row, int* walkdtime_i, const double* sensor, double* ctl,
                                   int sms, cudaStream_t st) {
   gait_stack_pre_kernel<<<stack_grid((size_t)B, sms), 256, 0, st>>>(B, planner, walkdtime_row, walkdtime_i, sensor, ctl);
+  return cudaGetLastError();
+}
+cudaError_t gait_stack_clocked_pre_launch(int B, int* clock, int* plan, double* walkdtime_row, int* walkdtime_i, const double* sensor,
+                                          double* ctl, int sms, cudaStream_t st) {
+  gait_stack_clocked_pre_kernel<<<stack_grid((size_t)B, sms), 256, 0, st>>>(B, clock, plan, walkdtime_row, walkdtime_i, sensor, ctl);
+  return cudaGetLastError();
+}
+cudaError_t gait_stack_reset_launch(const StackResetParams& P, int sms, cudaStream_t st) {
+  gait_stack_reset_mark_kernel<<<(P.B + 255) / 256, 256, 0, st>>>(P);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  gait_stack_reset_column_kernel<<<stack_grid((size_t)P.B * P.rows, sms), 256, 0, st>>>(P);
   return cudaGetLastError();
 }
 cudaError_t gait_stack_pack_launch(const GaitStackSlots& S, int B, const double* gait, const double* traj, double* rows, int sms,

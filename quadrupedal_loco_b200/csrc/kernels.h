@@ -219,6 +219,8 @@ struct NlpKParams {
   double* hz_co;              // [8][B] workspace
   double* lipm;               // [6][B] workspace
   double* msg;                // [100][B] /MPC/Gait
+  const int* active;          // [B] or null (= every robot): robots with 0 skip the node -- no node row, tick input or message
+                              //   slot is read or written, and their tick index is 0 so the planner kernels skip them too
 };
 cudaError_t nlp_pre_launch(NlpKParams P, cudaStream_t st);
 cudaError_t nlp_post_launch(NlpKParams P, cudaStream_t st);
@@ -254,6 +256,25 @@ cudaError_t gait_stack_pre_launch(int B, int planner, double* walkdtime_row, int
                                   int sms, cudaStream_t st);
 cudaError_t gait_stack_pack_launch(const GaitStackSlots& S, int B, const double* gait, const double* traj, double* rows, int sms,
                                    cudaStream_t st);
+// per-robot clocks: plan[b] = whether robot b's planner ticks in this call (from clock[b], which is then incremented); walkdtime
+// += 1 for those robots; the sensor scatter as gait_stack_pre_launch
+cudaError_t gait_stack_clocked_pre_launch(int B, int* clock, int* plan, double* walkdtime_row, int* walkdtime_i, const double* sensor,
+                                          double* ctl, int sms, cudaStream_t st);
+// robot resets: ws = {count, 3 pad, flags[B], list[B]} ints, count zero on entry.  The mark kernel lists the flagged robots and does their
+// small writes (clock 0, body record 0, servo rows); the column kernel writes the default column into the listed robots' state
+struct StackResetParams {
+  int B, rows, out_stride;
+  const int* reset;           // [B]
+  int* clock;                 // [B]
+  double* state;              // [rows][B]
+  const double* column;       // [rows] the default column
+  double* body_out;           // [B][out_stride], 16-byte aligned
+  double* servo;              // [SERVO_STATE_ROWS][B] or null
+  double q0[12];              // servo joint angles after a reset
+  int* count;
+  int* list;                  // [B]
+};
+cudaError_t gait_stack_reset_launch(const StackResetParams& P, int sms, cudaStream_t st);
 
 // ---- the servo stack tick: K consecutive 1 kHz servo ticks from the gait stack's messages (servo_stack.cu) ----
 constexpr int SERVO_TICKS_MAX = 10, SERVO_LPF_CHANNELS = 9;

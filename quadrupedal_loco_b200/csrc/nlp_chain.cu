@@ -13,6 +13,8 @@
 //   step_sqp / step_height / step_finish / foot_traj   (skip robots whose tick index is 0)
 //   nlp_post_kernel   thread per robot: ZMP samples i+3 .. i+_nTdx-1 of the LIPM roll-out (:938-955, only Zmp_distributor
 //                     reads them) into the robot's ZMP ring, force / moment distribution, the outgoing message
+// With an active mask (per-robot clocks of the gait stack) a robot whose entry is 0 leaves the node untouched: nlp_pre_kernel gives it
+// tick index 0, which the four planner kernels skip, and both node kernels return before touching its rows or its message.
 // Node state: ONE SoA buffer [NLP_NODE_DOUBLES][B] -- rows [0,202) planner state, [202,234) swing-foot window, then the ZMP
 // ring (the reference's whole-walk _zmpx_real / _zmpy_real as 2 x 64 entries, index & 63, with the highest index written)
 // and the members of NLPRTControlClass that persist (layout of oracle/nlp_node.c).  Checkpoint = memcpy.
@@ -43,6 +45,7 @@ constexpr int MODE_NONE = 0, MODE_SQUAT = 1, MODE_GAIT = 2, MODE_OVER = 3, MODE_
 __global__ void __launch_bounds__(128) nlp_pre_kernel(NlpKParams P) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= P.B) return;
+  if (P.active && !P.active[b]) { P.tick[b] = 0; return; }     // robot skips the node this call: its rows stay as they are
   const size_t B = (size_t)P.B;
   double* Nn = P.node + b;
 #define N(f) Nn[(size_t)(f) * B]
@@ -114,6 +117,7 @@ __device__ __forceinline__ void dsp_weights(double* co_a, double* co_b, const do
 __global__ void __launch_bounds__(128) nlp_post_kernel(NlpKParams P) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= P.B) return;
+  if (P.active && !P.active[b]) return;
   const size_t B = (size_t)P.B;
   double* Nn = P.node + b;
 #define N(f) Nn[(size_t)(f) * B]
