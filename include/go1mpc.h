@@ -752,7 +752,7 @@ int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r
  * A robot is reset by rewriting its column, a batch is checkpointed by a memcpy.
  * Not included: the servo's other filter objects (/MPC/Gait 39-41 and 73-75 at 10 Hz, ...) -- their outputs feed nothing here
  * and go1mpc_lpf_batch runs them on the resident message --, FK of the measured joints (servo.cpp:734-741), the GRF QP and
- * the torque map: how the servo assembles their inputs from the messages and the state estimator is not documented here.
+ * the torque map: go1mpc_servo_torque_tick_async below adds those three with its documented wiring.
  * One kernel launch, plus the D2H copy of q_d when q is given; nothing is allocated, so a warmed-up gait stack + servo period
  * can be captured with go1mpc_graph_capture_*.  B = 0 is a no-op.
  * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer, K outside 1..GO1MPC_SERVO_TICKS_MAX, q_d not
@@ -776,6 +776,69 @@ typedef struct {
   int *iters_d;                 /* last tick's Newton updates [4][B], or NULL */
 } Go1ServoStackTick;
 int go1mpc_servo_stack_tick_async(go1mpc_t *h, int B, const Go1ServoStackTick *t, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * Servo torque tick: go1mpc_servo_stack_tick_async's K ticks, each followed by the rest of go1_servo's 1 kHz tick
+ * (servo.cpp: force_distribution / force_opt -> 4 x compute_joint_torques) -- joint targets AND feed-forward joint torques for
+ * a Go1 in torque mode, with every member of Dynamiccclass resident on the device.  Per robot b and tick k = 1..K, after the
+ * tick's filters and IK (identical to go1mpc_servo_stack_tick_async: q_d, the servo state, jac_d / foot_des_d / iters_d are
+ * bit-identical to that call's):
+ *   argument of the reference             source
+ *   com_des, base_p                       the IK's body position of tick k (filtered slots 0, 1 * y_offset, 2)
+ *   leg_des, leg_p, p_des                 the four IK foot targets of tick k (go1mpc_servo_stack_tick_async's foot_des_d)
+ *   rfoot_des / lfoot_des                 the filtered virtual feet (filter channels 6-8 / 3-5)
+ *   F_force_des                           /MPC/Gait 15-20 (F_L xyz, F_R xyz, force_distribution's order)
+ *   FT_total_des                          (F_L + F_R, M_L + M_R) from /MPC/Gait 15-26
+ *   right_support                         /MPC/Gait 99
+ *   swing flag of leg l                   bit l of the QP's zero-force rule (mode 102: right_support 0 -> FL RR, 1 -> FR RL;
+ *                                         mode 101: 0 -> FL RL, 1 -> FR RR; otherwise none)
+ *   Jaco                                  the IK Jacobian at the tick's joint angles (the fused tick's wiring)
+ *   p_est, pv_est                         FK of the measured joints with tick k's body pose (the planned pose: there is no
+ *                                         estimator) = go1mpc_leg_fk_batch with body_r (roll, pitch, 0); pv_est_i =
+ *                                         (J_i0 dq_0 + J_i1 dq_1) + J_i2 dq_2 with the measured-joint Jacobian J, no FMA
+ *   pv_des                                /MPC/Gait 46-48 (right foot) / 49-51 (left foot), picked by the leg's virtual foot
+ *   stance force in the torque map        the QP's grf_opt, or F_leg_guess when the QP returns NaN (the fused tick's wiring)
+ * force_distribution runs for gait modes 101 / 102; mode 103 holds F_leg_ref (Dynamiccclass leaves it as it is).  The QP
+ * (go1mpc_grf_force_opt_batch's constants) starts from the previous tick's grf_opt, so the K ticks chain.  Each tick equals
+ * go1mpc_grf_force_distribution_batch -> go1mpc_grf_force_opt_batch -> go1mpc_grf_joint_torques_batch on records built as
+ * above, bit for bit.
+ * Buffers (device unless noted):
+ *   force_state_d  [GO1MPC_SERVO_FORCE_ROWS][B] in/out, caller-owned, zero-initialise: rows [0,12) the previous tick's
+ *                  grf_opt, rows [12,24) F_leg_ref (FR, FL, RR, RL xyz)
+ *   meas_d         [24][B] measured joint angles (FR, FL, RR, RL) then joint velocities; sampled once per call and held over
+ *                  its K ticks, as the messages are (K = 1 gives feedback every tick).  A host caller uploads it itself.
+ *   reset          host [B] ints (pinned) or NULL: robots with a non-zero flag start from a zero force state -- the buffer
+ *                  go1mpc_gait_stack_reset_async takes, so reset -> clocked tick -> torque tick replays with one set of flags
+ *   tau_d          [B][12*K] joint torques, tick-major per robot like q_d;  tau: host [B][12*K] or NULL (D2H copy)
+ *   grf_d, grf_diag_d  [B][16] / [B][32] or NULL: the last tick's out / diag records in go1mpc_grf_force_opt_batch's layout
+ * Two kernel launches (the servo stack, then one warp per robot for the K force stages), plus the reset upload and the D2H
+ * copies when given.  A workspace of 720 B per robot is allocated on the first call with a given (stream, B); later calls
+ * allocate nothing and can be captured with go1mpc_graph_capture_*.  B = 0 is a no-op.
+ * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer (stack_state_d, servo_state_d, q_d,
+ * force_state_d, meas_d, tau_d), K outside 1..GO1MPC_SERVO_TICKS_MAX, q_d or tau_d not 8-byte aligned;
+ * GO1MPC_E_UNSUPPORTED for gait_mode outside 101..103.
+ * ------------------------------------------------------------------------ */
+#define GO1MPC_SERVO_FORCE_ROWS 24
+typedef struct {
+  int K;                        /* as Go1ServoStackTick */
+  int gait_mode;
+  double y_offset;
+  const double *stack_state_d;
+  double *servo_state_d;
+  double *q_d;
+  double *q;
+  double *jac_d, *foot_des_d;
+  int *iters_d;
+  double y_coefficient;         /* force_distribution's y_coefficient */
+  double *force_state_d;        /* [GO1MPC_SERVO_FORCE_ROWS][B] in/out */
+  const double *meas_d;         /* [24][B] */
+  const int *reset;             /* host [B] (pinned) or NULL */
+  double *tau_d;                /* [B][12*K] */
+  double *tau;                  /* host [B][12*K] or NULL */
+  double *grf_d;                /* [B][16] or NULL */
+  int *grf_diag_d;              /* [B][32] or NULL */
+} Go1ServoTorqueTick;
+int go1mpc_servo_torque_tick_async(go1mpc_t *h, int B, const Go1ServoTorqueTick *t, void *stream);
 
 /* Per-kernel timing of the three-launch body tick (measurement aid for bench.py's roofline): while enabled, each
  * go1mpc_body_mpc_step_batch call on that path records CUDA events around its setup / solve / merge launches;

@@ -6,15 +6,15 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgo1mpc.so")
-SOURCES = ["api.cu", "body_mpc.cu", "body_fast.cu", "body_tri.cu", "body_duo.cu", "body_resident.cu", "qp_dense.cu", "step_timing.cu", "step_sqp.cu", "foot_traj.cu", "leg_kin.cu", "grf_qp.cu", "ref_interp.cu", "rt_chain.cu", "nlp_chain.cu", "filters.cu", "peer_gather.cu", "gait_stack.cu", "servo_stack.cu"]
+SOURCES = ["api.cu", "body_mpc.cu", "body_fast.cu", "body_tri.cu", "body_duo.cu", "body_resident.cu", "qp_dense.cu", "step_timing.cu", "step_sqp.cu", "foot_traj.cu", "leg_kin.cu", "grf_qp.cu", "ref_interp.cu", "rt_chain.cu", "nlp_chain.cu", "filters.cu", "peer_gather.cu", "gait_stack.cu", "servo_stack.cu", "servo_torque.cu"]
 # A/B variants that `auto` never chooses (body_split.cu: roll / pitch halves side by side in one warp) are only compiled
 # into the library with GO1MPC_BUILD_AB=1 (then GO1MPC_BODY_MODE=split selects it)
 AB_SOURCES = ["body_split.cu"]
 # per-source extra flags: the thread-per-instance kernels keep the oracle's operation order and
 # must not contract a*b+c into FMA
 EXTRA = {"step_timing.cu": ["-fmad=false"], "step_sqp.cu": ["-fmad=false"], "foot_traj.cu": ["-fmad=false"], "leg_kin.cu": ["-fmad=false"], "ref_interp.cu": ["-fmad=false"], "rt_chain.cu": ["-fmad=false"], "nlp_chain.cu": ["-fmad=false"], "filters.cu": ["-fmad=false"],
-         "servo_stack.cu": ["-fmad=false"]}
-HEADERS = ["gi_warp.cuh", "tma.cuh", "powi.cuh", "servo_math.cuh", "kernels.h", os.path.join("..", "..", "include", "go1mpc.h")]
+         "servo_stack.cu": ["-fmad=false"], "servo_torque.cu": ["-fmad=false"]}
+HEADERS = ["gi_warp.cuh", "grf_math.cuh", "tma.cuh", "powi.cuh", "servo_math.cuh", "kernels.h", os.path.join("..", "..", "include", "go1mpc.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC",

@@ -35,6 +35,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_grf_force_opt_batch_host", "go1mpc_grf_force_distribution_batch_host", "go1mpc_grf_joint_torques_batch_host", "go1mpc_leg_fk_batch_host", "go1mpc_leg_ik_batch_host",
     "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
     "go1mpc_servo_stack_tick_async", "go1mpc_gait_stack_tick_clocked_async", "go1mpc_gait_stack_reset_async",
+    "go1mpc_servo_torque_tick_async",
 ]
 
 
@@ -171,6 +172,7 @@ def load_library():
     lib.go1mpc_servo_stack_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoStackTick), vp]
     lib.go1mpc_gait_stack_tick_clocked_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackClockedTick), vp]
     lib.go1mpc_gait_stack_reset_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackReset), vp]
+    lib.go1mpc_servo_torque_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoTorqueTick), vp]
     _LIB = lib
     return lib
 
@@ -299,6 +301,17 @@ class ServoStackTick(ctypes.Structure):
     _fields_ = [("K", ctypes.c_int), ("gait_mode", ctypes.c_int), ("y_offset", ctypes.c_double),
                 ("stack_state_d", ctypes.c_void_p), ("servo_state_d", ctypes.c_void_p), ("q_d", ctypes.c_void_p),
                 ("q", ctypes.c_void_p), ("jac_d", ctypes.c_void_p), ("foot_des_d", ctypes.c_void_p), ("iters_d", ctypes.c_void_p)]
+
+
+SERVO_FORCE_ROWS = 24     # GO1MPC_SERVO_FORCE_ROWS: previous grf_opt [0,12) | F_leg_ref [12,24)
+
+
+class ServoTorqueTick(ctypes.Structure):
+    """Go1ServoTorqueTick of include/go1mpc.h."""
+    _fields_ = ServoStackTick._fields_ + [
+        ("y_coefficient", ctypes.c_double), ("force_state_d", ctypes.c_void_p), ("meas_d", ctypes.c_void_p),
+        ("reset", ctypes.c_void_p), ("tau_d", ctypes.c_void_p), ("tau", ctypes.c_void_p), ("grf_d", ctypes.c_void_p),
+        ("grf_diag_d", ctypes.c_void_p)]
 
 
 def _ptr(a):
@@ -655,6 +668,25 @@ class Go1Mpc:
         targets into q_d [B][12 K] (and the host q when given).  Returns after enqueueing on `stream` (None = the handle's)."""
         t = self.servo_stack_tick_struct(K, gait_mode, y_offset, stack_state_d, servo_state_d, q_d, q, jac_d, foot_des_d, iters_d)
         self._check(self.lib.go1mpc_servo_stack_tick_async(self.h, B, ctypes.byref(t), stream), "servo_stack_tick_async")
+
+    # --- servo torque tick: the servo stack, then force distribution, force QP and torque map per tick ---
+    def servo_torque_tick_struct(self, K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
+                                 q_d, tau_d, q=None, tau=None, reset=None, grf_d=None, grf_diag_d=None, jac_d=None, foot_des_d=None,
+                                 iters_d=None):
+        """Go1ServoTorqueTick for the given buffers (device: stack state, servo state [69][B], force state [24][B], meas [24][B],
+        q_d / tau_d [B][12 K]; host q / tau / reset (pinned) or None)."""
+        return ServoTorqueTick(int(K), int(gait_mode), float(y_offset), _ptr(stack_state_d), _ptr(servo_state_d), _ptr(q_d), _ptr(q),
+                               _ptr(jac_d), _ptr(foot_des_d), _ptr(iters_d), float(y_coefficient), _ptr(force_state_d), _ptr(meas_d),
+                               _ptr(reset), _ptr(tau_d), _ptr(tau), _ptr(grf_d), _ptr(grf_diag_d))
+
+    def servo_torque_tick(self, B, K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d, q_d,
+                          tau_d, stream=None, **kw):
+        """go1mpc_servo_torque_tick_async: K 1 kHz servo ticks (filters, leg IK, force distribution, force QP, joint torques) on
+        the gait stack state; joint targets into q_d and torques into tau_d, both [B][12 K].  Keyword arguments: q, tau, reset,
+        grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.  Returns after enqueueing on `stream` (None = the handle's)."""
+        t = self.servo_torque_tick_struct(K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
+                                          q_d, tau_d, **kw)
+        self._check(self.lib.go1mpc_servo_torque_tick_async(self.h, B, ctypes.byref(t), stream), "servo_torque_tick_async")
 
     def measure_dfma_peak(self, ms=200):
         g = ctypes.c_double(0.0)

@@ -75,6 +75,8 @@ struct go1mpc {
   // walkdtime ints | cmd | start | body-MPC input records | planner mask of the clocked tick | reset count, flags and robot list
   struct StackWs { DevBuf b[8]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
   std::map<cudaStream_t, StackWs> stack_ws;
+  struct ServoWs { DevBuf ch, reset; };   // servo torque tick: filtered channels [SERVO_TICKS_MAX][9][B], reset flags [B]
+  std::map<cudaStream_t, ServoWs> servo_ws;
   std::map<int, double*> stack_col_d;   // go1mpc_gait_stack_default_state(nh) on the device, per nh, built on first use
   double* trtab_d = nullptr;       // remaining-time bound table of the planner tick (host libm), built on first use
   std::vector<cudaEvent_t> ev_pool;   // go1mpc_stream_wait: events, reused round-robin
@@ -336,6 +338,7 @@ void go1mpc_destroy(go1mpc_t* h) {
   for (cudaEvent_t e : h->phase_ev) if (e) cudaEventDestroy(e);
   for (auto& kv : h->nlp_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
   for (auto& kv : h->stack_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
+  for (auto& kv : h->servo_ws) for (DevBuf* b : {&kv.second.ch, &kv.second.reset}) if (b->p) cudaFree(b->p);
   for (auto& kv : h->stack_col_d) cudaFree(kv.second);
   for (auto& L : h->lanes) {
     for (DevBuf& b : L.stage) if (b.p) cudaFree(b.p);
@@ -1598,10 +1601,67 @@ int go1mpc_servo_stack_tick_async(go1mpc_t* h, int B, const Go1ServoStackTick* t
   P.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
   P.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
   P.state = t->servo_state_d; P.q_out = t->q_d;
-  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d;
+  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d; P.ch = nullptr;
   CU(h, servo_stack_launch(P, st));
   h->launches++;
   if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, b * 12 * t->K * sizeof(double), cudaMemcpyDeviceToHost, st));
+  return GO1MPC_OK;
+}
+
+// ------------------------------------------------------------------ servo torque tick: the servo stack + force QP + torque map
+static_assert(GO1MPC_SERVO_FORCE_ROWS == SERVO_FORCE_ROWS, "servo force state layout");
+int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick* t, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
+  if (!t || !t->stack_state_d || !t->servo_state_d || !t->q_d || !t->force_state_d || !t->meas_d || !t->tau_d)
+    return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: bad argument");
+  if (t->K < 1 || t->K > GO1MPC_SERVO_TICKS_MAX) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: 1 <= K <= 10");
+  if (((uintptr_t)t->q_d | (uintptr_t)t->tau_d) & 7)
+    return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: q_d and tau_d must be 8-byte aligned");
+  if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, "servo_torque_tick_async: gait_mode 101, 102 or 103");
+  CU(h, cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  if (h->servo_ws.size() >= 256 && h->servo_ws.find(st) == h->servo_ws.end())
+    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
+  go1mpc::ServoWs& W = h->servo_ws[st];
+  const size_t b = (size_t)B;
+  // sized for K = GO1MPC_SERVO_TICKS_MAX, so that K changes do not reallocate; a growing buffer may still be read by the
+  // stream's previous call
+  const size_t chb = b * SERVO_TICKS_MAX * SERVO_LPF_CHANNELS * sizeof(double), rb = b * sizeof(int);
+  if (chb > W.ch.cap || (t->reset && rb > W.reset.cap)) CU(h, cudaStreamSynchronize(st));
+  void *ch, *rst = nullptr;
+  int rc;
+  if ((rc = stage_buf2(h, W.ch, chb, &ch))) return rc;
+  if (t->reset && (rc = stage_buf2(h, W.reset, rb, &rst))) return rc;
+  ServoStackKParams S;
+  S.B = B; S.K = t->K; S.gait_mode = t->gait_mode;
+  S.half_hip_width = h->cfg.step.half_hip_width; S.y_offset = t->y_offset;
+  double k6[6];
+  go1mpc_lpf_coefficients(1000.0, 3.0, k6);
+  S.coef = LpfCoef{k6[0], k6[1], k6[2], k6[3], k6[4], k6[5]};
+  S.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
+  S.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
+  S.state = t->servo_state_d; S.q_out = t->q_d;
+  S.jac = t->jac_d; S.foot_des = t->foot_des_d; S.iters = t->iters_d; S.ch = (double*)ch;
+  ServoTorqueKParams P;
+  P.g.B = B; P.g.cap = h->cfg.qp_iter_cap_scale * (12 + 12 + 24) + 50; P.g.warp_doubles = 0;
+  P.g.qp_alpha = 10000; P.g.qp_beta = 1000; P.g.qp_gama = 10; P.g.fz_max = 160; P.g.mu = 0.25;   // as go1mpc_grf_force_opt_batch
+  P.g.in = nullptr; P.g.out = nullptr; P.g.diag = nullptr;
+  P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
+  P.half_hip_width = S.half_hip_width; P.y_offset = t->y_offset; P.y_coefficient = t->y_coefficient;
+  P.swing_kp = 1; P.swing_kd = 0.01;                                                               // as go1mpc_grf_joint_torques_batch
+  P.gait = S.gait; P.traj = S.traj; P.homing = t->servo_state_d + SERVO_ROW_HOMING * b; P.ch = S.ch; P.q = t->q_d;
+  P.meas = t->meas_d; P.reset = (const int*)rst; P.force = t->force_state_d; P.tau = t->tau_d;
+  P.grf = t->grf_d; P.grf_diag = t->grf_diag_d;
+  if (rst) CU(h, cudaMemcpyAsync(rst, t->reset, rb, cudaMemcpyHostToDevice, st));
+  CU(h, servo_stack_launch(S, st));
+  h->launches++;
+  CU(h, servo_torque_launch(P, h->sms, st));
+  h->launches++;
+  const size_t kb = b * 12 * t->K * sizeof(double);
+  if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, kb, cudaMemcpyDeviceToHost, st));
+  if (t->tau) CU(h, cudaMemcpyAsync(t->tau, t->tau_d, kb, cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
 }
 

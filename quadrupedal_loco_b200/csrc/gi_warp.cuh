@@ -31,6 +31,16 @@
 
 namespace go1 {
 
+// The three multiply-adds below that the code writes as a*b+c follow the including file's -fmad setting: contracted in the
+// default build (qp_dense.cu, body_*.cu, grf_qp.cu), rounded twice in the -fmad=false build of step_timing.cu.  A file built
+// with -fmad=false that must reproduce the contracting build's bits (servo_torque.cu: grf_qp.cu's force QP) defines
+// GO1_GI_FMA before the first include, which writes them as fma().
+#ifdef GO1_GI_FMA
+#define GI_MAD(a, b, c) fma((a), (b), (c))
+#else
+#define GI_MAD(a, b, c) ((a) * (b) + (c))
+#endif
+
 constexpr unsigned FULL_MASK = 0xffffffffu;
 constexpr double EPS_D = 2.220446049250313e-16;
 
@@ -72,8 +82,8 @@ __device__ __forceinline__ void warp_argmin_redux(double& v, int& idx) {
 // EiQuadProg.hpp:100-118
 __device__ __forceinline__ double gi_hypot(double a, double b) {
   double a1 = fabs(a), b1 = fabs(b), t;
-  if (a1 > b1) { t = b1 / a1; return a1 * sqrt(1.0 + t * t); }
-  if (b1 > a1) { t = a1 / b1; return b1 * sqrt(1.0 + t * t); }
+  if (a1 > b1) { t = b1 / a1; return a1 * sqrt(GI_MAD(t, t, 1.0)); }
+  if (b1 > a1) { t = a1 / b1; return b1 * sqrt(GI_MAD(t, t, 1.0)); }
   return a1 * sqrt(2.0);
 }
 
@@ -322,7 +332,7 @@ __device__ inline void gi_loop(const GiWs& w, Pol& pol, double c1, double c2, in
     for (int k = lane; k < n; k += 32) w.x[k] = fma(t2, w.z[k], w.x[k]);
     for (int k = lane; k < iq; k += 32) w.u[k] = fma(-t2, w.r[k], w.u[k]);
     if (lane == 0) { w.u[iq] = t2; w.A[i] = -i - 1; }
-    f_value += 0.5 * (t2 * t2) * zn;
+    f_value = GI_MAD(0.5 * (t2 * t2), zn, f_value);
     __syncwarp();
     if (!gi_add_constraint(w, iq, R_norm, lane)) { status = ST_EQ_DEP; goto done; }
   }
@@ -399,7 +409,7 @@ __device__ inline void gi_loop(const GiWs& w, Pol& pol, double c1, double c2, in
       double uiq = w.u[iq];
       __syncwarp();
       for (int k = lane; k < n; k += 32) w.x[k] = fma(t, w.z[k], w.x[k]);
-      f_value += t * zn * (0.5 * t + uiq);
+      f_value = GI_MAD(t * zn, GI_MAD(0.5, t, uiq), f_value);
       for (int k = lane; k < iq; k += 32) w.u[k] = fma(-t, w.r[k], w.u[k]);
       if (lane == 0) w.u[iq] = uiq + t;
       __syncwarp();

@@ -9,47 +9,13 @@
 //                                      inequalities: unilateral + friction pyramid per leg)
 //   skew_hat               :375-385   (frozen bug: vec_w[2,0] is the comma operator -> every entry is vec_w[0])
 //   compute_joint_torques  :109-138   (thread per leg)
-// Records are instance-major (a warp reads its robot's 48-double record with coalesced loads).
+// Records are instance-major (a warp reads its robot's 48-double record with coalesced loads).  The per-robot arithmetic is
+// grf_math.cuh's, which servo_torque_kernel also runs.
 #include <cuda_runtime.h>
-#include "gi_warp.cuh"
+#include "grf_math.cuh"
 #include "kernels.h"
 
 namespace go1 {
-
-namespace {
-struct SmemPolicy {    // dense policy over shared-memory matrices (column-major, one constraint per column)
-  const double *CI, *ci0, *CE, *ce0v;
-  int n, m;
-  __device__ __forceinline__ void eval_s(const GiWs& w, int lane, double& psi) const {
-    for (int c = lane; c < m; c += 32) {
-      const double* col = CI + c * n;
-      double acc = 0.0;
-      for (int j = 0; j < n; j++) acc = fma(col[j], w.x[j], acc);
-      const double sv = acc + ci0[c];
-      w.s[c] = sv;
-      psi += fmin(0.0, sv);
-    }
-  }
-  __device__ __forceinline__ void load_np(const GiWs& w, int ip, int lane, int& klo, int& khi) const {
-    for (int j = lane; j < n; j += 32) w.np[j] = CI[ip * n + j];
-    klo = 0; khi = n;
-    __syncwarp();
-  }
-  __device__ __forceinline__ double eval_one(const GiWs& w, int ip, int lane) const {
-    double acc = 0.0;
-    for (int j = lane; j < n; j += 32) acc = fma(CI[ip * n + j], w.x[j], acc);
-    return warp_sum(acc) + ci0[ip];
-  }
-  __device__ __forceinline__ void load_eq(const GiWs& w, int i, int lane, bool& allzero) const {
-    bool z = true;
-    for (int j = lane; j < n; j += 32) { const double v = CE[i * n + j]; w.np[j] = v; z = z && (fabs(v) <= 1e-12); }
-    allzero = __all_sync(FULL_MASK, z);
-    __syncwarp();
-  }
-  __device__ __forceinline__ double ce0(int i) const { return ce0v[i]; }
-};
-constexpr int GN = 12, GP = 12, GM = 24;
-}  // namespace
 
 int grf_warp_doubles() { return gi_ws_doubles(GN, GM) + 72 + GN + GN * GP + GP + GRF_IN_DOUBLES; }   // ws | A(6x12) | g0 | CE | ce0 | record
 
@@ -58,21 +24,8 @@ __global__ void __launch_bounds__(WPC * 32) grf_force_opt_kernel(GrfKParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* smem = reinterpret_cast<double*>(smem_raw);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // CTA-shared inequality data: CI = -qp_H' (12 x 24), ci0 = qp_h
-  double* CI = smem;
-  double* ci0 = CI + GN * GM;
-  for (int t = threadIdx.x; t < GN * GM + GM; t += blockDim.x) smem[t] = 0.0;
-  __syncthreads();
-  if (threadIdx.x < 4) {
-    const int i = threadIdx.x;
-    // rows 2i, 2i+1: -fz <= 0, fz <= fz_max; rows 8+2i(+1): -+fx - mu fz <= 0; rows 16+2i(+1): -+fy - mu fz <= 0
-    CI[(2 * i) * GN + 3 * i + 2] = 1.0;           CI[(2 * i + 1) * GN + 3 * i + 2] = -1.0;  ci0[2 * i + 1] = P.fz_max;
-    CI[(8 + 2 * i) * GN + 3 * i] = 1.0;           CI[(8 + 2 * i) * GN + 3 * i + 2] = P.mu;
-    CI[(8 + 2 * i + 1) * GN + 3 * i] = -1.0;      CI[(8 + 2 * i + 1) * GN + 3 * i + 2] = P.mu;
-    CI[(16 + 2 * i) * GN + 3 * i + 1] = 1.0;      CI[(16 + 2 * i) * GN + 3 * i + 2] = P.mu;
-    CI[(16 + 2 * i + 1) * GN + 3 * i + 1] = -1.0; CI[(16 + 2 * i + 1) * GN + 3 * i + 2] = P.mu;
-  }
-  __syncthreads();
+  double* CI = smem;                             // CTA-shared inequality data: CI = -qp_H' (12 x 24), ci0 = qp_h
+  grf_ci_build(CI, P.fz_max, P.mu);
   double* wbase = smem + GN * GM + GM + (size_t)warp * P.warp_doubles;
   GiWs w;
   gi_ws_carve(w, wbase, GN, GP, GM);
@@ -88,83 +41,8 @@ __global__ void __launch_bounds__(WPC * 32) grf_force_opt_kernel(GrfKParams P) {
     recs[lane] = rec[lane];
     if (lane < GRF_IN_DOUBLES - 32) recs[32 + lane] = rec[32 + lane];
     __syncwarp();
-    auto field = [&](int k) -> double { return recs[k]; };
-    const double base_x = field(0);
-    const int mode = (int)field(45), right_support = (int)field(46);
-    // A = [I I I I; W_FR W_FL W_RR W_RL], W from skew_hat with its comma-operator reading of vec_w[0]
-    for (int t = lane; t < 72; t += 32) {
-      const int col = t / 6, r = t - 6 * col, l = col / 3, k = col - 3 * l;
-      double v;
-      if (r < 3) v = (r == k) ? 1.0 : 0.0;
-      else {
-        const double w0 = base_x - field(3 + 3 * l);
-        const int rr = r - 3;
-        v = (rr == k) ? 0.0 : (((k - rr + 3) % 3 == 1) ? -w0 : w0);    // [0 -w w; w 0 -w; -w w 0]
-      }
-      A[t] = v;
-    }
-    for (int t = lane; t < GN * GP; t += 32) CE[t] = 0.0;
-    if (lane < GP) ce0[lane] = 0.0;
-    __syncwarp();
-    // which legs carry no force (:315-350)
-    unsigned zero_legs = 0u;   // bit l: FR, FL, RR, RL
-    if (mode == 102) zero_legs = (right_support == 0) ? 0x6u : ((right_support == 1) ? 0x9u : 0u);
-    else if (mode == 101) zero_legs = (right_support == 0) ? 0x5u : ((right_support == 1) ? 0xAu : 0u);
-    if (lane < GN && ((zero_legs >> (lane / 3)) & 1u)) CE[lane * GN + lane] = 1.0;
-    // G = sym(2 (alpha A'A + (beta + gama) I)) into w.R (lower triangle is what the factorisation reads)
-    double tr = 0.0;
-    for (int t = lane; t < GN * GN; t += 32) {
-      const int j = t / GN, i = t - GN * j;
-      double a1 = 0.0, a2 = 0.0;
-      for (int r = 0; r < 6; r++) { a1 += (P.qp_alpha * A[i * 6 + r]) * A[j * 6 + r]; a2 += (P.qp_alpha * A[j * 6 + r]) * A[i * 6 + r]; }
-      const double unit = (i == j) ? 1.0 : 0.0;
-      const double qij = 2 * (a1 + (P.qp_beta + P.qp_gama) * unit), qji = 2 * (a2 + (P.qp_beta + P.qp_gama) * unit);
-      const double g = (qji + qij) / 2.0;
-      w.R[j * w.ld + i] = g;
-      if (i == j) tr += g;
-    }
-    const double c1 = warp_sum(tr);
-    if (lane < GN) {
-      double acc = 0.0;
-      for (int r = 0; r < 6; r++) acc += (P.qp_alpha * A[lane * 6 + r]) * field(15 + r);
-      g0[lane] = -2 * ((acc + P.qp_beta * field(21 + lane)) + P.qp_gama * field(33 + lane));
-    }
-    for (int t = lane; t < GN * w.ld; t += 32) w.J[t] = 0.0;
-    if (lane < GN) w.x[lane] = field(33 + lane);
-    __syncwarp();
-    GiResult res; res.f = 0.0; res.iq = 0; res.status = ST_OK;
-    res.it_outer = res.it_add = res.it_drop = res.it_degen = res.it_l2a = 0; res.flops = gi_flops_setup(GN, GP);
-    const bool pd = gi_llt(w, GN, lane);
-    if (!pd) { res.status = ST_NOT_PD; res.f = CUDART_INF; }
-    else {
-      gi_inv_lt(w, GN, 0, lane);
-      double c2 = (lane < GN) ? w.J[lane * w.ld + lane] : 0.0;
-      c2 = warp_sum(c2);
-      for (int t = lane; t < GN * w.ld; t += 32) w.R[t] = 0.0;
-      if (lane < GN) w.np[lane] = g0[lane];
-      __syncwarp();
-      gi_compute_d(w, 0, GN, lane);
-      gi_update_z(w, 0, lane);
-      double f = 0.0;
-      if (lane < GN) { const double xv = -w.z[lane]; w.x[lane] = xv; f = g0[lane] * xv; }
-      res.f = 0.5 * warp_sum(f);
-      __syncwarp();
-      SmemPolicy pol{CI, ci0, CE, ce0, GN, GM};
-      gi_loop(w, pol, c1, c2, P.cap, res, lane);
-    }
-    // qp_solution = "no NaN in X"; on failure the reference falls back to the closed-form guess (:364-367)
-    bool nan = (lane < GN) && (w.x[lane] != w.x[lane]);
-    nan = __any_sync(FULL_MASK, nan);
-    if (nan && (res.status == ST_OK || res.status == ST_EQ_DEP)) res.status = ST_NAN;
-    double* out = P.out + (size_t)b * GRF_OUT_DOUBLES;
-    const double guess = field(21 + (lane % GN));
-    if (lane < GN) out[lane] = nan ? guess : w.x[lane];
-    if (lane == 0) { out[12] = res.f; out[13] = nan ? 0.0 : 1.0; out[14] = 0.0; out[15] = 0.0; }
-    if (P.diag) {
-      int* dg = P.diag + (size_t)b * GRF_DIAG_INTS;
-      if (lane == 0) { dg[0] = res.status; dg[1] = pd ? res.iq : 0; dg[2] = res.it_outer; dg[3] = res.it_add; dg[4] = res.it_drop; dg[5] = res.it_degen; dg[6] = nan ? 0 : 1; dg[7] = 0; }
-      if (lane < 24) dg[8 + lane] = (pd && lane < res.iq) ? w.A[lane] : -99;
-    }
+    grf_force_opt_warp(P, CI, w, A, g0, CE, ce0, recs, P.out + (size_t)b * GRF_OUT_DOUBLES,
+                       P.diag ? P.diag + (size_t)b * GRF_DIAG_INTS : nullptr, lane);
     __syncwarp();
   }
 }
@@ -178,40 +56,7 @@ __global__ void __launch_bounds__(256) grf_force_distribution_kernel(GrfDistPara
   for (int k = 0; k < 3; k++) { com[k] = P.com[k * B + b]; rf[k] = P.rfoot[k * B + b]; lf[k] = P.lfoot[k * B + b]; }
   for (int k = 0; k < 12; k++) { leg[k] = P.leg[k * B + b]; out[k] = 0.0; }
   for (int k = 0; k < 6; k++) F[k] = P.F[k * B + b];
-  const double yc = P.y_coefficient;
-#define FR_(r, c) out[(c) * 3 + (r)]
-  if (P.mode == 101) {
-    double dis[4];
-    for (int l = 0; l < 4; l++) {
-      const double a = com[0] - leg[3 * l], bb = com[1] - leg[3 * l + 1], cc = com[2] - leg[3 * l + 2];
-      dis[l] = sqrt(a * a + bb * bb + cc * cc);
-    }
-    const double FRd = dis[0], FLd = dis[1], RRd = dis[2], RLd = dis[3];
-    double f;
-    f = F[0] * FLd / (FLd + RLd);       FR_(0, 3) = f; FR_(0, 1) = F[0] - f;
-    f = F[1] * FLd / (FLd + RLd) * yc;  FR_(1, 3) = f; FR_(1, 1) = F[1] * yc - f;
-    f = F[2] * FLd / (FLd + RLd);       FR_(2, 3) = f; FR_(2, 1) = F[2] - f;
-    f = F[3] * FRd / (FRd + RRd);       FR_(0, 2) = f; FR_(0, 0) = F[3] - f;
-    f = F[4] * FRd / (FRd + RRd) * yc;  FR_(1, 2) = f; FR_(1, 0) = F[4] * yc - f;
-    f = F[5] * FRd / (FRd + RRd);       FR_(2, 2) = f; FR_(2, 0) = F[5] - f;
-  } else if (P.mode == 102) {
-    double v[3], w[3], f;
-    for (int k = 0; k < 3; k++) { v[k] = leg[9 + k] - leg[k]; w[k] = lf[k] - leg[k]; }
-    double len = sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
-    double prj = v[0] * w[0] + v[1] * w[1] + v[2] * w[2];
-    double r = fmax(fmin(prj / len, 1.0), 0.0);
-    f = F[0] * r;       FR_(0, 3) = f; FR_(0, 0) = F[0] - f;
-    f = F[1] * r * yc;  FR_(1, 3) = f; FR_(1, 0) = F[1] * yc - f;
-    f = F[2] * r;       FR_(2, 3) = f; FR_(2, 0) = F[2] - f;
-    for (int k = 0; k < 3; k++) { v[k] = leg[6 + k] - leg[3 + k]; w[k] = rf[k] - leg[3 + k]; }
-    len = sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
-    prj = v[0] * w[0] + v[1] * w[1] + v[2] * w[2];
-    r = fmax(fmin(prj / len, 1.0), 0.0);
-    f = F[3] * r;       FR_(0, 2) = f; FR_(0, 1) = F[3] - f;
-    f = F[4] * r * yc;  FR_(1, 2) = f; FR_(1, 1) = F[4] * yc - f;
-    f = F[5] * r;       FR_(2, 2) = f; FR_(2, 1) = F[5] - f;
-  }
-#undef FR_
+  grf_distribute(P.mode, P.y_coefficient, com, leg, F, rf, lf, out);
   for (int k = 0; k < 12; k++) P.F_leg_ref[k * B + b] = out[k];
 }
 
@@ -228,16 +73,15 @@ __global__ void __launch_bounds__(256) grf_joint_torques_kernel(GrfTauParams P) 
   if (P.swing[leg * B + b]) {
     for (int k = 0; k < 3; k++) {
       const size_t i = (size_t)(3 * leg + k) * B + b;
-      w[k] = __dadd_rn(__dmul_rn(P.swing_kp, __dsub_rn(P.p_des[i], P.p_est[i])), __dmul_rn(P.swing_kd, __dsub_rn(P.pv_des[i], P.pv_est[i])));
+      w[k] = grf_swing_w(P.swing_kp, P.swing_kd, P.p_des[i], P.p_est[i], P.pv_des[i], P.pv_est[i]);
     }
   } else {
     for (int k = 0; k < 3; k++) w[k] = P.F_leg_ref[(long long)(3 * leg + k) * P.f_ks + (long long)b * P.f_bs];
   }
   for (int i = 0; i < 3; i++) {
-    double acc = 0.0;
-    for (int r = 0; r < 3; r++) acc = __dadd_rn(acc, __dmul_rn(-P.jac[(size_t)(9 * leg + 3 * r + i) * B + b], w[r]));
-    const double grav = (i == 0) ? ((leg & 1) ? 0.80 : -0.80) : 0.0;    // gravity_compensate, dynmics_compute.cpp:39-41
-    P.tau[(size_t)(3 * leg + i) * B + b] = __dadd_rn(acc, grav);
+    double j[3];
+    for (int r = 0; r < 3; r++) j[r] = P.jac[(size_t)(9 * leg + 3 * r + i) * B + b];
+    P.tau[(size_t)(3 * leg + i) * B + b] = grf_tau(leg, i, j, w);
   }
 }
 

@@ -158,6 +158,7 @@ struct GrfDistParams {
   double* F_leg_ref;                             // SoA [12][B] (FR, FL, RR, RL xyz)
 };
 cudaError_t grf_force_opt_launch(GrfKParams P, int sms, cudaStream_t st);
+int grf_warp_doubles();                          // shared-memory doubles of one force-QP warp: workspace | A | g0 | CE | ce0 | record
 cudaError_t grf_force_distribution_launch(GrfDistParams P, cudaStream_t st);
 struct GrfTauParams {
   int B;
@@ -290,8 +291,29 @@ struct ServoStackKParams {
   double* jac;                  // [36][B] or null (last tick)
   double* foot_des;             // [12][B] or null (last tick)
   int* iters;                   // [4][B] or null (last tick)
+  double* ch;                   // [K][9][B] or null: each tick's filtered channels
 };
 cudaError_t servo_stack_launch(const ServoStackKParams& P, cudaStream_t st);
+
+// ---- the servo torque tick: force distribution, force QP and torque map after the servo stack (servo_torque.cu) ----
+constexpr int SERVO_FORCE_ROWS = 24, SERVO_MEAS_ROWS = 24;
+struct ServoTorqueKParams {
+  GrfKParams g;                 // QP constants, cap and warp_doubles (in / out / diag unused)
+  int B, K, gait_mode;
+  double half_hip_width, y_offset, y_coefficient, swing_kp, swing_kd;
+  const double* gait;           // [100][B] /MPC/Gait
+  const double* traj;           // [100][B] /rtMPC/traj: slots 72, 73 = roll, pitch
+  const double* homing;         // [12][B] the servo state's homing rows
+  const double* ch;             // [K][9][B] filtered channels of each tick (servo_stack_kernel<true>)
+  const double* q;              // [B][12 K] the IK's joint angles of each tick
+  const double* meas;           // [24][B] measured q (12) and dq (12), FR FL RR RL
+  const int* reset;             // [B] or null
+  double* force;                // [SERVO_FORCE_ROWS][B] in/out: grf_opt 12 | F_leg_ref 12
+  double* tau;                  // [B][12 K]
+  double* grf;                  // [B][16] or null (last tick)
+  int* grf_diag;                // [B][32] or null (last tick)
+};
+cudaError_t servo_torque_launch(ServoTorqueKParams P, int sms, cudaStream_t st);
 
 // register-resident DFMA loop: flops executed are returned through *flops
 cudaError_t dfma_peak_launch(int grid, int block, int iters, double* sink, cudaStream_t st);

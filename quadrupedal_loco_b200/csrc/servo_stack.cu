@@ -19,6 +19,8 @@ namespace {
 __device__ __forceinline__ constexpr int lpf_slot(int c) { return c < 3 ? c : c + 3; }
 }  // namespace
 
+// CH: also store each tick's nine filtered channels to P.ch [K][9][B] (the servo torque tick's second kernel reads them)
+template <bool CH>
 __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const size_t B = (size_t)P.B;
@@ -63,6 +65,11 @@ __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
     double f[3];
 #pragma unroll
     for (int j = 0; j < 3; j++) f[j] = (j < nch) ? lpf_step(P.coef, fs[j], y[j]) : 0.0;
+    if constexpr (CH) {
+#pragma unroll
+      for (int j = 0; j < 3; j++)
+        if (j < nch) P.ch[((size_t)k * SERVO_LPF_CHANNELS + leg + 4 * j) * B + b] = f[j];
+    }
     double ch[SERVO_LPF_CHANNELS];                // channel c: lane c % 4 of the group, its f[c / 4]
 #pragma unroll
     for (int c = 0; c < SERVO_LPF_CHANNELS; c++) ch[c] = __shfl_sync(live, f[c >> 2], c & 3, 4);
@@ -90,7 +97,8 @@ __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
 
 cudaError_t servo_stack_launch(const ServoStackKParams& P, cudaStream_t st) {
   const size_t threads = 4 * (size_t)P.B;
-  servo_stack_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
+  if (P.ch) servo_stack_kernel<true><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
+  else servo_stack_kernel<false><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
   return cudaGetLastError();
 }
 
