@@ -733,6 +733,53 @@ typedef struct {
 int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r, void *stream);
 
 /* ---------------------------------------------------------------------------
+ * Farm column copy: whole robots copied between two farm-shaped buffer sets, the source column picked per destination column by
+ * a device index array -- to snapshot robots into a bank, restore them, fork one stored mid-walk state into many robots, or
+ * restart robots chosen by a device kernel (a simulator's episode end) with no host round trip.
+ *
+ * A robot's whole state is its gait stack column state_d[:, b], its body-MPC record body_out_d[b], its clock clock_d[b], its
+ * servo column servo_state_d[:, b] and its force column force_state_d[:, b]: a run that starts from copied values is
+ * bit-identical to the run of the robot they were copied from.  For every destination column i with 0 <= index_d[i] < src.B,
+ * every given block of column i becomes the same block of source column index_d[i].  The servo column is copied whole, homing
+ * rows included (go1mpc_gait_stack_reset_async keeps them).  index_d[i] = -1 keeps column i; any other entry outside
+ * -1..src.B-1 also keeps column i and, when bad_d is given, adds 1 to *bad_d.  Each destination has one source, so there are no
+ * write conflicts; many destinations may share one source.  The same call serves
+ *   snapshot  farm -> bank    (dst = a bank of any B, index_d[j] = the farm column to store in bank column j)
+ *   restore   bank -> farm    (index_d[i] = the bank column robot i restarts from, -1 for robots that keep walking)
+ *   fork      bank -> farm with a repeated index (one stored state into many robots), or farm A -> farm B
+ * A fork inside one farm is two calls through a bank: snapshot robot 7 into bank column 0 (bank index {7}), then restore with
+ * index_d[i] = 0 for the robots that fork and -1 elsewhere.  A bank column holding a freshly reset robot (snapshot right after
+ * go1mpc_gait_stack_reset_async, force column zero) restarts robots as that reset plus the torque tick's reset flag do, except
+ * that the homing rows come from the bank column.
+ * clock_d, servo_state_d and force_state_d are each given on both sides or on neither; both sides share nh.
+ * Two kernel launches of a fixed shape after a memset of a device counter: the first lists the copied destinations (one
+ * atomic per warp) and copies their clocks, the second copies the listed columns, reading the count on the device.  The index
+ * never changes what is enqueued, and the work grows with the number of columns copied.  A workspace of 8 B per destination
+ * column is allocated on the first call with a given (stream, dst.B); later calls allocate nothing, so a warmed-up period
+ * restore -> go1mpc_gait_stack_tick_clocked_async -> go1mpc_servo_torque_tick_async can be captured once with
+ * go1mpc_graph_capture_* and replayed, the caller (or a device kernel) rewriting index_d between replays.  dst.B = 0 is a no-op.
+ * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL c, state_d, body_out_d or index_d, an optional block given on one
+ * side only, body_out_d not 16-byte aligned on either side, a negative B, src.B < 1 while dst.B > 0, or any destination block
+ * whose address range overlaps any source block; GO1MPC_E_UNSUPPORTED for nh outside 3..40.  index_d is device memory and is
+ * not checked on the host: an out-of-range entry never causes an out-of-bounds access.
+ * ------------------------------------------------------------------------ */
+typedef struct {
+  int B;                    /* columns (robots) of this buffer set */
+  double *state_d;          /* [go1mpc_gait_stack_state_doubles(nh)][B] SoA */
+  double *body_out_d;       /* [B][go1mpc_body_out_stride(nh)], 16-byte aligned */
+  int *clock_d;             /* [B] or NULL */
+  double *servo_state_d;    /* [GO1MPC_SERVO_STATE_ROWS][B] or NULL */
+  double *force_state_d;    /* [GO1MPC_SERVO_FORCE_ROWS][B] or NULL */
+} Go1FarmColumns;
+typedef struct {
+  int nh;                   /* 3..40, shared by both sides */
+  Go1FarmColumns dst, src;
+  const int *index_d;       /* device [dst.B]: -1 = keep column i; 0..src.B-1 = column i <- source column index_d[i] */
+  int *bad_d;               /* device int or NULL: += number of entries outside -1..src.B-1 (those columns are kept) */
+} Go1FarmCopy;
+int go1mpc_farm_copy_async(go1mpc_t *h, const Go1FarmCopy *c, void *stream);
+
+/* ---------------------------------------------------------------------------
  * Servo stack tick: K consecutive ticks of go1_servo's 1 kHz loop for B robots in ONE call, fed in place from the messages the
  * gait stack keeps resident -- the call a controller farm makes after each gait stack call (K = 10 per 10 ms period), joint
  * targets out.  Per robot b and tick k = 1..K:

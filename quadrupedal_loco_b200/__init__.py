@@ -12,7 +12,7 @@ from .binding import (  # noqa: F401
     ControlTick, COMPACT_DOUBLES, lpf_coefficients, GaitStackTick, STACK_SENSOR_ROWS, STACK_SLOTS_MAX, STACK_ROW_NLP,
     STACK_ROW_GAIT, STACK_ROW_RT2NRT, STACK_ROW_WALKDTIME, STACK_ROW_TRAJ, STACK_ROW_RT,
     ServoStackTick, SERVO_TICKS_MAX, SERVO_STATE_ROWS, SERVO_ROW_Q, SERVO_ROW_HOMING, SERVO_ROW_LPF, SERVO_LPF_SLOTS,
-    GaitStackClockedTick, GaitStackReset, ServoTorqueTick, SERVO_FORCE_ROWS,
+    GaitStackClockedTick, GaitStackReset, ServoTorqueTick, SERVO_FORCE_ROWS, FarmColumns, FarmCopy,
 )
 from ._build import build  # noqa: F401
 
@@ -24,5 +24,5 @@ __all__ = [
     "GaitStackTick", "STACK_SENSOR_ROWS", "STACK_SLOTS_MAX", "STACK_ROW_NLP", "STACK_ROW_GAIT", "STACK_ROW_RT2NRT",
     "STACK_ROW_WALKDTIME", "STACK_ROW_TRAJ", "STACK_ROW_RT",
     "ServoStackTick", "SERVO_TICKS_MAX", "SERVO_STATE_ROWS", "SERVO_ROW_Q", "SERVO_ROW_HOMING", "SERVO_ROW_LPF", "SERVO_LPF_SLOTS",
-    "GaitStackClockedTick", "GaitStackReset", "ServoTorqueTick", "SERVO_FORCE_ROWS",
+    "GaitStackClockedTick", "GaitStackReset", "ServoTorqueTick", "SERVO_FORCE_ROWS", "FarmColumns", "FarmCopy",
 ]

@@ -35,7 +35,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_grf_force_opt_batch_host", "go1mpc_grf_force_distribution_batch_host", "go1mpc_grf_joint_torques_batch_host", "go1mpc_leg_fk_batch_host", "go1mpc_leg_ik_batch_host",
     "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
     "go1mpc_servo_stack_tick_async", "go1mpc_gait_stack_tick_clocked_async", "go1mpc_gait_stack_reset_async",
-    "go1mpc_servo_torque_tick_async",
+    "go1mpc_servo_torque_tick_async", "go1mpc_farm_copy_async",
 ]
 
 
@@ -173,6 +173,7 @@ def load_library():
     lib.go1mpc_gait_stack_tick_clocked_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackClockedTick), vp]
     lib.go1mpc_gait_stack_reset_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackReset), vp]
     lib.go1mpc_servo_torque_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoTorqueTick), vp]
+    lib.go1mpc_farm_copy_async.argtypes = [vp, ctypes.POINTER(FarmCopy), vp]
     _LIB = lib
     return lib
 
@@ -312,6 +313,18 @@ class ServoTorqueTick(ctypes.Structure):
         ("y_coefficient", ctypes.c_double), ("force_state_d", ctypes.c_void_p), ("meas_d", ctypes.c_void_p),
         ("reset", ctypes.c_void_p), ("tau_d", ctypes.c_void_p), ("tau", ctypes.c_void_p), ("grf_d", ctypes.c_void_p),
         ("grf_diag_d", ctypes.c_void_p)]
+
+
+class FarmColumns(ctypes.Structure):
+    """Go1FarmColumns of include/go1mpc.h: one farm-shaped buffer set (device)."""
+    _fields_ = [("B", ctypes.c_int), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p), ("clock_d", ctypes.c_void_p),
+                ("servo_state_d", ctypes.c_void_p), ("force_state_d", ctypes.c_void_p)]
+
+
+class FarmCopy(ctypes.Structure):
+    """Go1FarmCopy of include/go1mpc.h."""
+    _fields_ = [("nh", ctypes.c_int), ("dst", FarmColumns), ("src", FarmColumns), ("index_d", ctypes.c_void_p),
+                ("bad_d", ctypes.c_void_p)]
 
 
 def _ptr(a):
@@ -687,6 +700,21 @@ class Go1Mpc:
         t = self.servo_torque_tick_struct(K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
                                           q_d, tau_d, **kw)
         self._check(self.lib.go1mpc_servo_torque_tick_async(self.h, B, ctypes.byref(t), stream), "servo_torque_tick_async")
+
+    # --- farm column copy: whole robots between two farm-shaped buffer sets, picked by a device index ---
+    @staticmethod
+    def farm_columns(B, state_d, body_out_d, clock_d=None, servo_state_d=None, force_state_d=None):
+        """FarmColumns for one buffer set (torch CUDA tensors or raw addresses)."""
+        return FarmColumns(int(B), _ptr(state_d), _ptr(body_out_d), _ptr(clock_d), _ptr(servo_state_d), _ptr(force_state_d))
+
+    def farm_copy(self, nh, dst, src, index_d, bad_d=None, stream=None):
+        """go1mpc_farm_copy_async: destination column i of every given block <- source column index_d[i] (device int32 [dst.B];
+        -1 keeps column i).  dst / src are FarmColumns (farm_columns) or dicts of its fields.  bad_d (device int32) counts the
+        entries outside -1..src.B-1, whose columns are kept.  Returns after enqueueing on `stream` (None = the handle's)."""
+        d = dst if isinstance(dst, FarmColumns) else self.farm_columns(**dst)
+        s = src if isinstance(src, FarmColumns) else self.farm_columns(**src)
+        c = FarmCopy(int(nh), d, s, _ptr(index_d), _ptr(bad_d))
+        self._check(self.lib.go1mpc_farm_copy_async(self.h, ctypes.byref(c), stream), "farm_copy_async")
 
     def measure_dfma_peak(self, ms=200):
         g = ctypes.c_double(0.0)

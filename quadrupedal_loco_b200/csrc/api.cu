@@ -72,8 +72,9 @@ struct go1mpc {
   struct NlpWs { DevBuf b[7]; };   // workspace of go1mpc_nlp_node_tick_batch, one per caller stream
   std::map<cudaStream_t, NlpWs> nlp_ws;
   // workspace of the gait stack entries, one per caller stream (grown on demand): sensor | /control2rtmpc/state |
-  // walkdtime ints | cmd | start | body-MPC input records | planner mask of the clocked tick | reset count, flags and robot list
-  struct StackWs { DevBuf b[8]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
+  // walkdtime ints | cmd | start | body-MPC input records | planner mask of the clocked tick | reset count, flags and robot list |
+  // farm copy count and lists
+  struct StackWs { DevBuf b[9]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
   std::map<cudaStream_t, StackWs> stack_ws;
   struct ServoWs { DevBuf ch, reset; };   // servo torque tick: filtered channels [SERVO_TICKS_MAX][9][B], reset flags [B]
   std::map<cudaStream_t, ServoWs> servo_ws;
@@ -1573,6 +1574,67 @@ int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r
   CU(h, cudaMemcpyAsync((void*)P.reset, r->reset, b * sizeof(int), cudaMemcpyHostToDevice, st));
   CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
   CU(h, gait_stack_reset_launch(P, h->sms, st));
+  h->launches += 2;
+  return GO1MPC_OK;
+}
+
+int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (!c) return fail(h, GO1MPC_E_INVALID, "farm_copy_async: bad argument");
+  const Go1FarmColumns &D = c->dst, &S = c->src;
+  if (D.B < 0 || S.B < 0) return fail(h, GO1MPC_E_INVALID, "farm_copy_async: negative B");
+  if (D.B == 0) return GO1MPC_OK;
+  if (S.B < 1) return fail(h, GO1MPC_E_INVALID, "farm_copy_async: src.B must be at least 1");
+  if (!D.state_d || !D.body_out_d || !S.state_d || !S.body_out_d || !c->index_d)
+    return fail(h, GO1MPC_E_INVALID, "farm_copy_async: bad argument");
+  if (!D.clock_d != !S.clock_d || !D.servo_state_d != !S.servo_state_d || !D.force_state_d != !S.force_state_d)
+    return fail(h, GO1MPC_E_INVALID, "farm_copy_async: clock_d, servo_state_d and force_state_d must be given on both sides or neither");
+  if (((uintptr_t)D.body_out_d | (uintptr_t)S.body_out_d) & 15)
+    return fail(h, GO1MPC_E_INVALID, "farm_copy_async: body_out_d must be 16-byte aligned");
+  const int nh = c->nh;
+  if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "farm_copy_async: 3 <= nh <= 40");
+  const int rows = go1mpc_gait_stack_state_doubles(nh), out_stride = go1mpc_body_out_stride(nh);
+  // the kernels read the source while they write the destination: no destination block may share a byte with a source block
+  auto blocks = [&](const Go1FarmColumns& F, uintptr_t* lo, uintptr_t* hi) {
+    const size_t b = (size_t)F.B;
+    const void* p[5] = {F.state_d, F.body_out_d, F.clock_d, F.servo_state_d, F.force_state_d};
+    const size_t n[5] = {b * rows * sizeof(double), b * out_stride * sizeof(double), b * sizeof(int), b * SERVO_STATE_ROWS * sizeof(double),
+                         b * SERVO_FORCE_ROWS * sizeof(double)};
+    for (int k = 0; k < 5; k++) { lo[k] = (uintptr_t)p[k]; hi[k] = p[k] ? lo[k] + n[k] : lo[k]; }
+  };
+  uintptr_t dlo[5], dhi[5], slo[5], shi[5];
+  blocks(D, dlo, dhi);
+  blocks(S, slo, shi);
+  for (int i = 0; i < 5; i++)
+    for (int k = 0; k < 5; k++)
+      if (dlo[i] < shi[k] && slo[k] < dhi[i])
+        return fail(h, GO1MPC_E_INVALID, "farm_copy_async: a destination block overlaps a source block");
+  CU(h, cudaSetDevice(h->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
+    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
+  go1mpc::StackWs& W = h->stack_ws[st];
+  // {count, 3 pad, destination list[dst.B], source list[dst.B]}
+  const size_t bytes = (4 + 2 * (size_t)D.B) * sizeof(int);
+  if (bytes > W.b[8].cap) CU(h, cudaStreamSynchronize(st));
+  void* ws;
+  int rc;
+  if ((rc = stage_buf2(h, W.b[8], bytes, &ws))) return rc;
+  FarmCopyParams P;
+  P.dst_B = D.B; P.src_B = S.B;
+  P.rows = rows;
+  P.servo_end = rows + (D.servo_state_d ? SERVO_STATE_ROWS : 0);
+  P.soa_rows = P.servo_end + (D.force_state_d ? SERVO_FORCE_ROWS : 0);
+  P.rec2 = out_stride / 2;
+  P.index = c->index_d; P.bad = c->bad_d;
+  P.dst_state = D.state_d; P.dst_servo = D.servo_state_d; P.dst_force = D.force_state_d;
+  P.src_state = S.state_d; P.src_servo = S.servo_state_d; P.src_force = S.force_state_d;
+  P.dst_body = reinterpret_cast<double2*>(D.body_out_d); P.src_body = reinterpret_cast<const double2*>(S.body_out_d);
+  P.dst_clock = D.clock_d; P.src_clock = S.clock_d;
+  P.count = (int*)ws; P.dlist = P.count + 4; P.slist = P.count + 4 + D.B;
+  CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
+  CU(h, farm_copy_launch(P, h->sms, st));
   h->launches += 2;
   return GO1MPC_OK;
 }

@@ -276,6 +276,25 @@ struct StackResetParams {
   int* list;                  // [B]
 };
 cudaError_t gait_stack_reset_launch(const StackResetParams& P, int sms, cudaStream_t st);
+// farm column copy: ws = {count, 3 pad, dst list[dst_B], src list[dst_B]} ints, count zero on entry.  The list kernel lists the
+// destinations with a valid index and copies their clocks; the column kernel copies the listed columns' SoA rows (state | servo |
+// force as one row range) and body records
+struct FarmCopyParams {
+  int dst_B, src_B;
+  int rows, servo_end, soa_rows;    // state rows; + servo rows (0 or SERVO_STATE_ROWS); + force rows (0 or SERVO_FORCE_ROWS)
+  int rec2;                         // double2 per body record
+  const int* index;                 // [dst_B]
+  int* bad;                         // or null
+  double *dst_state, *dst_servo, *dst_force;
+  const double *src_state, *src_servo, *src_force;
+  double2* dst_body;
+  const double2* src_body;
+  int* dst_clock;                   // or null (then src_clock too)
+  const int* src_clock;
+  int* count;
+  int *dlist, *slist;               // [dst_B]
+};
+cudaError_t farm_copy_launch(const FarmCopyParams& P, int sms, cudaStream_t st);
 
 // ---- the servo stack tick: K consecutive 1 kHz servo ticks from the gait stack's messages (servo_stack.cu) ----
 constexpr int SERVO_TICKS_MAX = 10, SERVO_LPF_CHANNELS = 9;
