@@ -641,7 +641,8 @@ int go1mpc_rt_node_tick_batch_host(go1mpc_t *h, int nh, int B, double *state, co
  *   [GO1MPC_STACK_ROW_TRAJ, +100)      /rtMPC/traj                [GO1MPC_STACK_ROW_RT, +go1mpc_rt_node_state_doubles(nh))  the 100 Hz node
  * go1mpc_gait_stack_default_state gives one robot's initial column; a robot is reset by rewriting its column, a batch is
  * checkpointed by a memcpy.  One call enqueues on `stream`:
- *   1. H2D of sensor (and, when planner = 1, of cmd / start if given)
+ *   1. H2D of sensor (and, when planner = 1, of cmd / start if given); an input given as a device buffer (sensor_d, cmd_d,
+ *      start_d) is read in place instead, with no copy
  *   2. planner = 1: walkdtime += 1, then go1mpc_nlp_node_tick_batch on the state with rfoot_fb / lfoot_fb = rows 22..24 / 19..21
  *      of the resident /rt2nrt/state (the foot feedback the previous fast tick forwarded, as the reference's ROS graph wires it)
  *   3. the sensor rows into their slots of a /control2rtmpc/state buffer (its other 14 slots 0), then
@@ -652,8 +653,15 @@ int go1mpc_rt_node_tick_batch_host(go1mpc_t *h, int nh, int B, double *state, co
  * 8, 10, ...  The body-MPC input records and all staging are per-stream workspace owned by the handle, allocated on the
  * first call with a given (stream, B): later calls with that pair allocate nothing, so a warmed-up schedule can be captured
  * with go1mpc_graph_capture_*.  Host buffers should be pinned and stay untouched until the stream has passed the call.
- * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer, n_slots outside 1..64, a slot outside 0..199,
- * body_out_d not 16-byte or rows_d not 8-byte aligned; GO1MPC_E_UNSUPPORTED for nh outside 3..40 or cfg.step.ext_height set.
+ * Device inputs: sensor_d [11][B] (in place of sensor), cmd_d / start_d [B] (in place of cmd / start) give bit-identical
+ * results to host inputs holding the same values.  They are read by the call's own kernels in stream order: a kernel enqueued
+ * earlier on `stream` may write them and one enqueued after the call may overwrite them (a writer on another stream needs the
+ * caller's events).  Device values are not checked: as for the host inputs, a cmd other than 1 or 2 is no command.
+ * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer, both or neither of sensor / sensor_d, both of
+ * cmd / cmd_d or of start / start_d, n_slots outside 1..64, a slot outside 0..199, body_out_d not 16-byte, rows_d or sensor_d
+ * not 8-byte, cmd_d or start_d not 4-byte aligned, a device input whose address range overlaps state_d, body_out_d, rows_d
+ * (or the clocked tick's clock_d) -- the call's kernels take them as non-aliasing; GO1MPC_E_UNSUPPORTED for nh outside 3..40
+ * or cfg.step.ext_height set.
  * ------------------------------------------------------------------------ */
 #define GO1MPC_STACK_SENSOR_ROWS 11   /* /control2rtmpc/state slots 0 | 10 11 13 14 | 19 20 21 | 22 23 24 */
 #define GO1MPC_STACK_SLOTS_MAX 64
@@ -674,6 +682,8 @@ typedef struct {
   int slots[GO1MPC_STACK_SLOTS_MAX];   /* 0..99 = /MPC/Gait slot, 100..199 = /rtMPC/traj slot - 100 */
   double *rows_d;            /* device [B][n_slots], caller-owned (e.g. go1mpc_gather_dest with row_doubles = n_slots) */
   double *rows;              /* host [B][n_slots] or NULL: copy of rows_d */
+  const double *sensor_d;    /* device [11][B] SoA, same rows as `sensor`; exactly one of sensor / sensor_d */
+  const int *cmd_d, *start_d;  /* device [B] or NULL; at most one of cmd / cmd_d and one of start / start_d */
 } Go1GaitStackTick;
 int go1mpc_gait_stack_state_doubles(int nh);
 int go1mpc_gait_stack_default_state(go1mpc_t *h, int nh, double *column);
@@ -688,25 +698,31 @@ int go1mpc_gait_stack_tick_host_async(go1mpc_t *h, int B, const Go1GaitStackTick
  *   Robot b with clock c plans in this call when c == 0 or (10c)/25 > (10(c-1))/25 (c = 0, 3, 5, 8, 10, ...: the reference's
  *   schedule, run on the robot's own time); its clock is c + 1 after the call.  walkdtime += 1 only for the robots that plan.  A robot
  *   that does not plan leaves the planner node's rows, /MPC/Gait and walkdtime untouched; the 100 Hz node, the pack and the copy to
- *   `rows` run for every robot.  cmd / start are uploaded whenever given and read only for the robots that plan.  The planner node's
+ *   `rows` run for every robot.  cmd / start are uploaded whenever given (cmd_d / start_d are read in place) and read only for
+ *   the robots that plan; sensor_d / cmd_d / start_d as go1mpc_gait_stack_tick_host_async.  The planner node's
  *   kernels are enqueued on every call (robots that do not plan exit at once), so every call enqueues the same work and one captured
  *   period graph replays for all periods.  Errors: those of go1mpc_gait_stack_tick_host_async, and GO1MPC_E_INVALID for a NULL
  *   clock_d; nothing is enqueued on an error.  B = 0 is a no-op.
  *
  * go1mpc_gait_stack_reset_async: for every robot b with reset[b] != 0 (reset: host [B] ints, pinned so the call can sit in a graph,
- *   uploaded by the call):
+ *   uploaded by the call; or reset_d: device [B] ints read in place in stream order, as the ticks' device inputs):
  *     the column b of state_d = go1mpc_gait_stack_default_state(nh);  body_out_d record b = 0;  clock_d[b] = 0;
  *     when servo_state_d is given: rows GO1MPC_SERVO_ROW_Q..+12 = servo_q0, the 45 filter rows = 0 (the homing rows are the
  *     caller's input and stay).
  *   Other robots are not touched.  Two kernel launches of a fixed shape; the flagged robots are listed on the device, so the
  *   flags never change what is enqueued, and the work grows with the number of robots flagged.  The default column is built once
  *   per (handle, nh), with a synchronous upload, and kept on the device: the first reset call with each nh must come before any
- *   graph capture.  Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL reset / clock_d / state_d / body_out_d or
- *   body_out_d not 16-byte aligned, GO1MPC_E_UNSUPPORTED for nh outside 3..40.
+ *   graph capture.  Any non-zero flag resets the robot.  Errors (nothing is enqueued): GO1MPC_E_INVALID for both or neither of
+ *   reset / reset_d, a NULL clock_d / state_d / body_out_d, body_out_d not 16-byte or reset_d not 4-byte aligned, reset_d
+ *   overlapping state_d, body_out_d, clock_d or servo_state_d; GO1MPC_E_UNSUPPORTED for nh outside 3..40.
  *
  * Both entries allocate only on their first call with a given (stream, B) (and, for the reset, nh), so a warmed-up period
- *   reset -> clocked tick -> go1mpc_servo_stack_tick_async can be captured once with go1mpc_graph_capture_* and replayed every period,
- *   the caller rewriting the pinned sensor and reset buffers between replays.
+ *   reset -> clocked tick -> go1mpc_servo_stack_tick_async can be captured once with go1mpc_graph_capture_* and replayed every period.
+ *   Fed from host buffers, the caller rewrites the pinned sensor and reset buffers between replays, after the previous replay has
+ *   finished.  Fed from device buffers -- sensor_d, cmd_d / start_d, reset_d (or a restart by go1mpc_farm_copy_async), with the
+ *   optional host copies (rows, and the servo entries' q / tau) left NULL -- a period enqueues no host<->device copy: a simulator
+ *   kernel on the same stream writes the next period's inputs, and periods are enqueued or replayed back to back with no host
+ *   synchronisation.
  * ------------------------------------------------------------------------ */
 typedef struct {
   int nh;                    /* body-MPC horizon, 3..40 */
@@ -719,16 +735,19 @@ typedef struct {
   double *rows_d;            /* device [B][n_slots] */
   double *rows;              /* host [B][n_slots] or NULL */
   int *clock_d;              /* device [B] ints, in/out: periods since each robot's reset */
+  const double *sensor_d;    /* as Go1GaitStackTick */
+  const int *cmd_d, *start_d;  /* as Go1GaitStackTick */
 } Go1GaitStackClockedTick;
 int go1mpc_gait_stack_tick_clocked_async(go1mpc_t *h, int B, const Go1GaitStackClockedTick *t, void *stream);
 typedef struct {
   int nh;
-  const int *reset;          /* host [B] ints (pinned): non-zero = reset this robot */
+  const int *reset;          /* host [B] ints (pinned) or NULL: non-zero = reset this robot */
   int *clock_d;              /* device [B], as Go1GaitStackClockedTick */
   double *state_d;           /* device [go1mpc_gait_stack_state_doubles(nh)][B] */
   double *body_out_d;        /* device [B][go1mpc_body_out_stride(nh)], 16-byte aligned */
   double *servo_state_d;     /* device [GO1MPC_SERVO_STATE_ROWS][B] or NULL */
   double servo_q0[12];       /* joint angles (FR, FL, RR, RL) a reset robot's servo starts from */
+  const int *reset_d;        /* device [B] ints, same flags as `reset`; exactly one of reset / reset_d */
 } Go1GaitStackReset;
 int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r, void *stream);
 
@@ -856,14 +875,18 @@ int go1mpc_servo_stack_tick_async(go1mpc_t *h, int B, const Go1ServoStackTick *t
  *                  its K ticks, as the messages are (K = 1 gives feedback every tick).  A host caller uploads it itself.
  *   reset          host [B] ints (pinned) or NULL: robots with a non-zero flag start from a zero force state -- the buffer
  *                  go1mpc_gait_stack_reset_async takes, so reset -> clocked tick -> torque tick replays with one set of flags
+ *   reset_d        device [B] ints or NULL: the same flags read in place in stream order (at most one of reset / reset_d);
+ *                  with reset_d, q = tau = NULL and the gait stack fed from device buffers, a period enqueues no
+ *                  host<->device copy and runs back to back with a simulator kernel on the same stream
  *   tau_d          [B][12*K] joint torques, tick-major per robot like q_d;  tau: host [B][12*K] or NULL (D2H copy)
  *   grf_d, grf_diag_d  [B][16] / [B][32] or NULL: the last tick's out / diag records in go1mpc_grf_force_opt_batch's layout
  * Two kernel launches (the servo stack, then one warp per robot for the K force stages), plus the reset upload and the D2H
  * copies when given.  A workspace of 720 B per robot is allocated on the first call with a given (stream, B); later calls
  * allocate nothing and can be captured with go1mpc_graph_capture_*.  B = 0 is a no-op.
  * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL required pointer (stack_state_d, servo_state_d, q_d,
- * force_state_d, meas_d, tau_d), K outside 1..GO1MPC_SERVO_TICKS_MAX, q_d or tau_d not 8-byte aligned;
- * GO1MPC_E_UNSUPPORTED for gait_mode outside 101..103.
+ * force_state_d, meas_d, tau_d), K outside 1..GO1MPC_SERVO_TICKS_MAX, q_d or tau_d not 8-byte aligned, both reset and reset_d,
+ * reset_d not 4-byte aligned or overlapping force_state_d, servo_state_d, q_d or tau_d; GO1MPC_E_UNSUPPORTED for gait_mode
+ * outside 101..103.
  * ------------------------------------------------------------------------ */
 #define GO1MPC_SERVO_FORCE_ROWS 24
 typedef struct {
@@ -884,6 +907,7 @@ typedef struct {
   double *tau;                  /* host [B][12*K] or NULL */
   double *grf_d;                /* [B][16] or NULL */
   int *grf_diag_d;              /* [B][32] or NULL */
+  const int *reset_d;           /* device [B] or NULL, same flags as `reset`; at most one of reset / reset_d */
 } Go1ServoTorqueTick;
 int go1mpc_servo_torque_tick_async(go1mpc_t *h, int B, const Go1ServoTorqueTick *t, void *stream);
 

@@ -273,7 +273,7 @@ class GaitStackTick(ctypes.Structure):
     _fields_ = [("nh", ctypes.c_int), ("planner", ctypes.c_int), ("sensor", ctypes.c_void_p), ("cmd", ctypes.c_void_p),
                 ("start", ctypes.c_void_p), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p),
                 ("n_slots", ctypes.c_int), ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p),
-                ("rows", ctypes.c_void_p)]
+                ("rows", ctypes.c_void_p), ("sensor_d", ctypes.c_void_p), ("cmd_d", ctypes.c_void_p), ("start_d", ctypes.c_void_p)]
 
 
 class GaitStackClockedTick(ctypes.Structure):
@@ -281,13 +281,14 @@ class GaitStackClockedTick(ctypes.Structure):
     _fields_ = [("nh", ctypes.c_int), ("sensor", ctypes.c_void_p), ("cmd", ctypes.c_void_p), ("start", ctypes.c_void_p),
                 ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p), ("n_slots", ctypes.c_int),
                 ("slots", ctypes.c_int * STACK_SLOTS_MAX), ("rows_d", ctypes.c_void_p), ("rows", ctypes.c_void_p),
-                ("clock_d", ctypes.c_void_p)]
+                ("clock_d", ctypes.c_void_p), ("sensor_d", ctypes.c_void_p), ("cmd_d", ctypes.c_void_p), ("start_d", ctypes.c_void_p)]
 
 
 class GaitStackReset(ctypes.Structure):
     """Go1GaitStackReset of include/go1mpc.h."""
     _fields_ = [("nh", ctypes.c_int), ("reset", ctypes.c_void_p), ("clock_d", ctypes.c_void_p), ("state_d", ctypes.c_void_p),
-                ("body_out_d", ctypes.c_void_p), ("servo_state_d", ctypes.c_void_p), ("servo_q0", ctypes.c_double * 12)]
+                ("body_out_d", ctypes.c_void_p), ("servo_state_d", ctypes.c_void_p), ("servo_q0", ctypes.c_double * 12),
+                ("reset_d", ctypes.c_void_p)]
 
 
 SERVO_TICKS_MAX = 10      # GO1MPC_SERVO_TICKS_MAX
@@ -312,7 +313,7 @@ class ServoTorqueTick(ctypes.Structure):
     _fields_ = ServoStackTick._fields_ + [
         ("y_coefficient", ctypes.c_double), ("force_state_d", ctypes.c_void_p), ("meas_d", ctypes.c_void_p),
         ("reset", ctypes.c_void_p), ("tau_d", ctypes.c_void_p), ("tau", ctypes.c_void_p), ("grf_d", ctypes.c_void_p),
-        ("grf_diag_d", ctypes.c_void_p)]
+        ("grf_diag_d", ctypes.c_void_p), ("reset_d", ctypes.c_void_p)]
 
 
 class FarmColumns(ctypes.Structure):
@@ -626,13 +627,16 @@ class Go1Mpc:
         self._check(self.lib.go1mpc_gait_stack_default_state(self.h, nh, _ptr(s)), "gait_stack_default_state")
         return s
 
-    def gait_stack_tick_struct(self, nh, planner, sensor, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None):
-        """Go1GaitStackTick for the given buffers (host: sensor [11][B], cmd / start [B] int32, rows [B][len(slots)])."""
+    def gait_stack_tick_struct(self, nh, planner, sensor, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None,
+                               sensor_d=None, cmd_d=None, start_d=None):
+        """Go1GaitStackTick for the given buffers (host: sensor [11][B], cmd / start [B] int32, rows [B][len(slots)]).  sensor_d /
+        cmd_d / start_d: the same inputs as device buffers, read in place (sensor = None with sensor_d)."""
         t = GaitStackTick(nh, 1 if planner else 0, _ptr(sensor), _ptr(cmd), _ptr(start), _ptr(state_d), _ptr(body_out_d), len(slots))
         for k, v in enumerate(slots[:STACK_SLOTS_MAX]):
             t.slots[k] = int(v)
         t.rows_d = _ptr(rows_d)
         t.rows = _ptr(rows)
+        t.sensor_d, t.cmd_d, t.start_d = _ptr(sensor_d), _ptr(cmd_d), _ptr(start_d)
         return t
 
     def gait_stack_tick_host_async(self, B, t, stream=None):
@@ -640,14 +644,17 @@ class Go1Mpc:
         (None = the handle's)."""
         self._check(self.lib.go1mpc_gait_stack_tick_host_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_host_async")
 
-    def gait_stack_tick_clocked_struct(self, nh, sensor, clock_d, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None):
-        """Go1GaitStackClockedTick for the given buffers (device clock_d [B] int32: periods since each robot's reset)."""
+    def gait_stack_tick_clocked_struct(self, nh, sensor, clock_d, state_d, body_out_d, slots, rows_d, rows=None, cmd=None, start=None,
+                                       sensor_d=None, cmd_d=None, start_d=None):
+        """Go1GaitStackClockedTick for the given buffers (device clock_d [B] int32: periods since each robot's reset); sensor_d /
+        cmd_d / start_d as gait_stack_tick_struct."""
         t = GaitStackClockedTick(nh, _ptr(sensor), _ptr(cmd), _ptr(start), _ptr(state_d), _ptr(body_out_d), len(slots))
         for k, v in enumerate(slots[:STACK_SLOTS_MAX]):
             t.slots[k] = int(v)
         t.rows_d = _ptr(rows_d)
         t.rows = _ptr(rows)
         t.clock_d = _ptr(clock_d)
+        t.sensor_d, t.cmd_d, t.start_d = _ptr(sensor_d), _ptr(cmd_d), _ptr(start_d)
         return t
 
     def gait_stack_tick_clocked_async(self, B, t, stream=None):
@@ -655,9 +662,11 @@ class Go1Mpc:
         enqueueing on `stream` (None = the handle's)."""
         self._check(self.lib.go1mpc_gait_stack_tick_clocked_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_clocked_async")
 
-    def gait_stack_reset_struct(self, nh, reset, clock_d, state_d, body_out_d, servo_state_d=None, servo_q0=None):
-        """Go1GaitStackReset for the given buffers (host reset [B] int32, pinned for graph capture; servo_q0: 12 joint angles)."""
+    def gait_stack_reset_struct(self, nh, reset, clock_d, state_d, body_out_d, servo_state_d=None, servo_q0=None, reset_d=None):
+        """Go1GaitStackReset for the given buffers (host reset [B] int32, pinned for graph capture, or reset = None and device
+        reset_d [B] int32; servo_q0: 12 joint angles)."""
         r = GaitStackReset(nh, _ptr(reset), _ptr(clock_d), _ptr(state_d), _ptr(body_out_d), _ptr(servo_state_d))
+        r.reset_d = _ptr(reset_d)
         if servo_q0 is not None:
             q0 = np.asarray(servo_q0, dtype=np.float64).reshape(12)
             for k in range(12):
@@ -685,18 +694,18 @@ class Go1Mpc:
     # --- servo torque tick: the servo stack, then force distribution, force QP and torque map per tick ---
     def servo_torque_tick_struct(self, K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
                                  q_d, tau_d, q=None, tau=None, reset=None, grf_d=None, grf_diag_d=None, jac_d=None, foot_des_d=None,
-                                 iters_d=None):
+                                 iters_d=None, reset_d=None):
         """Go1ServoTorqueTick for the given buffers (device: stack state, servo state [69][B], force state [24][B], meas [24][B],
-        q_d / tau_d [B][12 K]; host q / tau / reset (pinned) or None)."""
+        q_d / tau_d [B][12 K], reset_d [B] int32 or None; host q / tau / reset (pinned) or None)."""
         return ServoTorqueTick(int(K), int(gait_mode), float(y_offset), _ptr(stack_state_d), _ptr(servo_state_d), _ptr(q_d), _ptr(q),
                                _ptr(jac_d), _ptr(foot_des_d), _ptr(iters_d), float(y_coefficient), _ptr(force_state_d), _ptr(meas_d),
-                               _ptr(reset), _ptr(tau_d), _ptr(tau), _ptr(grf_d), _ptr(grf_diag_d))
+                               _ptr(reset), _ptr(tau_d), _ptr(tau), _ptr(grf_d), _ptr(grf_diag_d), _ptr(reset_d))
 
     def servo_torque_tick(self, B, K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d, q_d,
                           tau_d, stream=None, **kw):
         """go1mpc_servo_torque_tick_async: K 1 kHz servo ticks (filters, leg IK, force distribution, force QP, joint torques) on
         the gait stack state; joint targets into q_d and torques into tau_d, both [B][12 K].  Keyword arguments: q, tau, reset,
-        grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.  Returns after enqueueing on `stream` (None = the handle's)."""
+        reset_d, grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.  Returns after enqueueing on `stream` (None = the handle's)."""
         t = self.servo_torque_tick_struct(K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
                                           q_d, tau_d, **kw)
         self._check(self.lib.go1mpc_servo_torque_tick_async(self.h, B, ctypes.byref(t), stream), "servo_torque_tick_async")

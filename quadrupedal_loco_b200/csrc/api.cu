@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
@@ -1440,13 +1441,26 @@ int go1mpc_gait_stack_default_state(go1mpc_t* h, int nh, double* s) {
 }
 
 namespace {
+struct Block { const void* p; size_t bytes; };
+// Whether the device input [in, in + bytes) shares a byte with one of the blocks a call writes (null blocks are skipped).  The
+// kernels that read the inputs declare their pointers __restrict__, so a caller's input must not alias what the call writes.
+bool overlaps_written(const void* in, size_t bytes, std::initializer_list<Block> written) {
+  if (!in) return false;
+  const uintptr_t lo = (uintptr_t)in, hi = lo + bytes;
+  for (const Block& w : written)
+    if (w.p && (uintptr_t)w.p < hi && lo < (uintptr_t)w.p + w.bytes) return true;
+  return false;
+}
+
 // The node sequence of both gait stack ticks.  clock_d == null: every robot gets t.planner (go1mpc_gait_stack_tick_host_async);
 // otherwise each robot's planner flag comes from its clock (go1mpc_gait_stack_tick_clocked_async), and the planner node is always
 // enqueued, with the robots that do not plan masked out -- the same launches every period, so one captured graph fits all.
 int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock_d, void* stream, const char* name) {
   const std::string nm(name);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
-  if (!t || !t->sensor || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, nm + ": bad argument");
+  if (!t || !t->sensor == !t->sensor_d || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, nm + ": bad argument");
+  if ((t->cmd && t->cmd_d) || (t->start && t->start_d))
+    return fail(h, GO1MPC_E_INVALID, nm + ": at most one of cmd / cmd_d and one of start / start_d");
   const int nh = t->nh, n = t->n_slots;
   if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, nm + ": 3 <= nh <= 40");
   if (h->cfg.step.ext_height)
@@ -1461,6 +1475,17 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
   // the body kernels read and write body_out_d with 16-byte loads / TMA; the pack kernel stores doubles into rows_d
   if (((uintptr_t)t->body_out_d & 15) || ((uintptr_t)t->rows_d & 7))
     return fail(h, GO1MPC_E_INVALID, nm + ": body_out_d must be 16-byte and rows_d 8-byte aligned");
+  if (((uintptr_t)t->sensor_d & 7) || (((uintptr_t)t->cmd_d | (uintptr_t)t->start_d) & 3))
+    return fail(h, GO1MPC_E_INVALID, nm + ": sensor_d must be 8-byte and cmd_d / start_d 4-byte aligned");
+  {
+    const size_t b = (size_t)B;
+    const std::initializer_list<Block> written = {{t->state_d, b * go1mpc_gait_stack_state_doubles(nh) * sizeof(double)},
+                                                  {t->body_out_d, b * go1mpc_body_out_stride(nh) * sizeof(double)},
+                                                  {t->rows_d, b * n * sizeof(double)}, {clock_d, b * sizeof(int)}};
+    if (overlaps_written(t->sensor_d, b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), written) ||
+        overlaps_written(t->cmd_d, b * sizeof(int), written) || overlaps_written(t->start_d, b * sizeof(int), written))
+      return fail(h, GO1MPC_E_INVALID, nm + ": sensor_d / cmd_d / start_d overlap state_d, body_out_d, rows_d or clock_d");
+  }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
@@ -1485,20 +1510,20 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
     W.zero_B = B;
   }
   double* state = t->state_d;
-  CU(h, cudaMemcpyAsync(d[0], t->sensor, bytes[0], cudaMemcpyHostToDevice, st));
+  // device inputs are read in place; host inputs go up into the stream's staging buffers
+  const double* sensor = t->sensor_d;
+  if (!sensor) { CU(h, cudaMemcpyAsync(d[0], t->sensor, bytes[0], cudaMemcpyHostToDevice, st)); sensor = (const double*)d[0]; }
   // with per-robot clocks some robot may plan in any call, so cmd / start go up whenever they are given
   const bool planner = clock_d || t->planner;
-  const int* cmd_d = nullptr;
-  const int* start_d = nullptr;
+  const int* cmd_d = t->cmd_d;
+  const int* start_d = t->start_d;
   if (planner && t->cmd) { CU(h, cudaMemcpyAsync(d[3], t->cmd, bytes[3], cudaMemcpyHostToDevice, st)); cmd_d = (const int*)d[3]; }
   if (planner && t->start) { CU(h, cudaMemcpyAsync(d[4], t->start, bytes[4], cudaMemcpyHostToDevice, st)); start_d = (const int*)d[4]; }
   int* plan_d = (int*)d[6];
   if (clock_d)
-    CU(h, gait_stack_clocked_pre_launch(B, clock_d, plan_d, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl,
-                                        h->sms, st));
+    CU(h, gait_stack_clocked_pre_launch(B, clock_d, plan_d, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], sensor, ctl, h->sms, st));
   else
-    CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], (const double*)d[0], ctl,
-                                h->sms, st));
+    CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], sensor, ctl, h->sms, st));
   h->launches++;
   double* gait = state + GO1MPC_STACK_ROW_GAIT * b;
   double* rt2nrt = state + GO1MPC_STACK_ROW_RT2NRT * b;
@@ -1531,6 +1556,7 @@ int go1mpc_gait_stack_tick_clocked_async(go1mpc_t* h, int B, const Go1GaitStackC
   Go1GaitStackTick u;
   u.nh = t->nh; u.planner = 0; u.sensor = t->sensor; u.cmd = t->cmd; u.start = t->start; u.state_d = t->state_d;
   u.body_out_d = t->body_out_d; u.n_slots = t->n_slots; u.rows_d = t->rows_d; u.rows = t->rows;
+  u.sensor_d = t->sensor_d; u.cmd_d = t->cmd_d; u.start_d = t->start_d;
   memcpy(u.slots, t->slots, sizeof u.slots);
   return gait_stack_enqueue(h, B, &u, t->clock_d, stream, "gait_stack_tick_clocked_async");
 }
@@ -1539,10 +1565,17 @@ int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
-  if (!r || !r->reset || !r->clock_d || !r->state_d || !r->body_out_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: bad argument");
+  if (!r || !r->reset == !r->reset_d || !r->clock_d || !r->state_d || !r->body_out_d)
+    return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: bad argument");
   const int nh = r->nh;
   if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "gait_stack_reset_async: 3 <= nh <= 40");
   if ((uintptr_t)r->body_out_d & 15) return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: body_out_d must be 16-byte aligned");
+  if ((uintptr_t)r->reset_d & 3) return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: reset_d must be 4-byte aligned");
+  if (overlaps_written(r->reset_d, (size_t)B * sizeof(int),
+                       {{r->state_d, (size_t)B * go1mpc_gait_stack_state_doubles(nh) * sizeof(double)},
+                        {r->body_out_d, (size_t)B * go1mpc_body_out_stride(nh) * sizeof(double)},
+                        {r->clock_d, (size_t)B * sizeof(int)}, {r->servo_state_d, (size_t)B * SERVO_STATE_ROWS * sizeof(double)}}))
+    return fail(h, GO1MPC_E_INVALID, "gait_stack_reset_async: reset_d overlaps state_d, body_out_d, clock_d or servo_state_d");
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   const int rows = go1mpc_gait_stack_state_doubles(nh);
@@ -1568,10 +1601,10 @@ int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r
   if ((rc = stage_buf2(h, W.b[7], bytes, &ws))) return rc;
   StackResetParams P;
   P.B = B; P.rows = rows; P.out_stride = go1mpc_body_out_stride(nh);
-  P.count = (int*)ws; P.reset = P.count + 4; P.list = P.count + 4 + B;
+  P.count = (int*)ws; P.reset = r->reset_d ? r->reset_d : P.count + 4; P.list = P.count + 4 + B;
   P.clock = r->clock_d; P.state = r->state_d; P.column = it->second; P.body_out = r->body_out_d; P.servo = r->servo_state_d;
   memcpy(P.q0, r->servo_q0, sizeof P.q0);
-  CU(h, cudaMemcpyAsync((void*)P.reset, r->reset, b * sizeof(int), cudaMemcpyHostToDevice, st));
+  if (r->reset) CU(h, cudaMemcpyAsync((void*)P.reset, r->reset, b * sizeof(int), cudaMemcpyHostToDevice, st));
   CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
   CU(h, gait_stack_reset_launch(P, h->sms, st));
   h->launches += 2;
@@ -1682,6 +1715,15 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
   if (((uintptr_t)t->q_d | (uintptr_t)t->tau_d) & 7)
     return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: q_d and tau_d must be 8-byte aligned");
   if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, "servo_torque_tick_async: gait_mode 101, 102 or 103");
+  if (t->reset && t->reset_d) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: at most one of reset / reset_d");
+  if ((uintptr_t)t->reset_d & 3) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: reset_d must be 4-byte aligned");
+  {
+    const size_t b = (size_t)B, kb = b * 12 * t->K * sizeof(double);
+    if (overlaps_written(t->reset_d, b * sizeof(int),
+                         {{t->force_state_d, b * SERVO_FORCE_ROWS * sizeof(double)}, {t->servo_state_d, b * SERVO_STATE_ROWS * sizeof(double)},
+                          {t->q_d, kb}, {t->tau_d, kb}}))
+      return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: reset_d overlaps force_state_d, servo_state_d, q_d or tau_d");
+  }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   if (h->servo_ws.size() >= 256 && h->servo_ws.find(st) == h->servo_ws.end())
@@ -1714,7 +1756,7 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
   P.half_hip_width = S.half_hip_width; P.y_offset = t->y_offset; P.y_coefficient = t->y_coefficient;
   P.swing_kp = 1; P.swing_kd = 0.01;                                                               // as go1mpc_grf_joint_torques_batch
   P.gait = S.gait; P.traj = S.traj; P.homing = t->servo_state_d + SERVO_ROW_HOMING * b; P.ch = S.ch; P.q = t->q_d;
-  P.meas = t->meas_d; P.reset = (const int*)rst; P.force = t->force_state_d; P.tau = t->tau_d;
+  P.meas = t->meas_d; P.reset = t->reset_d ? t->reset_d : (const int*)rst; P.force = t->force_state_d; P.tau = t->tau_d;
   P.grf = t->grf_d; P.grf_diag = t->grf_diag_d;
   if (rst) CU(h, cudaMemcpyAsync(rst, t->reset, rb, cudaMemcpyHostToDevice, st));
   CU(h, servo_stack_launch(S, st));
