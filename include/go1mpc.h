@@ -543,6 +543,8 @@ int go1mpc_gather_status(go1mpc_gather_t *g, int *status);
  *   go1mpc_graph_capture_begin(h, s0); go1mpc_stream_wait(h, s1, s0); ...ticks on s0, s1...;
  *   go1mpc_stream_wait(h, s0, s1); go1mpc_graph_capture_end(h, s0, &g); go1mpc_graph_launch(h, g, s0);
  * go1mpc_stream_wait makes `waiter` wait for the work enqueued so far on `signaller` (NULL = the handle's stream).
+ * A handle keeps a workspace for at most 256 distinct streams; a call that would bring in a 257th returns
+ * GO1MPC_E_UNSUPPORTED and enqueues nothing.
  * ------------------------------------------------------------------------ */
 int go1mpc_stream_wait(go1mpc_t *h, void *waiter, void *signaller);
 int go1mpc_graph_capture_begin(go1mpc_t *h, void *stream);

@@ -3,6 +3,7 @@
 // Host side of the boundary.  No CPU compute path exists here: every entry point
 // either launches the sm_100a kernels or fails with an error code.
 #include <cuda_runtime.h>
+#include <assert.h>
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -29,9 +30,35 @@ struct BodyModel {
   double tx0[GO1MPC_FOOTSTEPS];
 };
 
+// device buffer grown on demand by grow(); freed with its owner
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { reset(); }
+  void reset() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// Workspace of one caller stream.  Keyed by stream because launches on one stream are ordered: a buffer is free again when
+// the next call on that stream starts, and calls on different streams never share one.
+struct StreamWs {
+  // {next, done} scheduler counters of the persistent body kernels and the hand-over list {count, total, ids[kFlistCap]}
+  DevBuf ctl;
+  // body_tri workspace, laid out for capB instances: J | half state | half result | queue | meta | hand-over at off[], then the
+  // 16-byte queue control block at qctl_off
+  struct { DevBuf buf; int capB = 0; size_t off[6] = {0, 0, 0, 0, 0, 0}; size_t qctl_off = 0; } tri;
+  // go1mpc_control_tick_host_async; zero_B: batch size for which rows 10..19 of the planner inputs are known zero
+  struct { DevBuf tick, step_in, body_tick_in, body_in, out38, step_diag, body_diag; int zero_B = -1; } control;
+  // go1mpc_nlp_node_tick_batch
+  struct { DevBuf tick, in, out38, out18, right_support, hz_co, lipm; } nlp;
+  // gait stack ticks: sensor | /control2rtmpc/state | walkdtime ints | cmd | start | body-MPC input records | planner mask of
+  // the clocked tick; zero_B: batch size for which the control message's other slots are zero
+  struct { DevBuf sensor, ctl_msg, walkdtime, cmd, start, body_in, plan; int zero_B = -1; } stack;
+  DevBuf reset_list;   // go1mpc_gait_stack_reset_async: {count, 3 pad, flags[B], robot list[B]}
+  DevBuf copy_list;    // go1mpc_farm_copy_async: {count, 3 pad, destination list[dst.B], source list[dst.B]}
+  DevBuf servo_ch, servo_reset;   // go1mpc_servo_torque_tick_async: filtered channels [SERVO_TICKS_MAX][9][B], reset flags [B]
 };
 
 }  // namespace
@@ -49,36 +76,19 @@ struct go1mpc {
   // lanes of the asynchronous *_host_async entry points (8: a lane is busy for H2D + kernel + D2H, a few
   // hundred microseconds at batch 4096, while the PCIe link needs a new batch every ~100 us): consecutive calls go to consecutive lanes
   // (own stream, own staging), so the H2D copy of one batch overlaps the kernel of the previous
-  // one and the D2H copy of the one before that
-  struct Lane { cudaStream_t stream = nullptr; DevBuf stage[12]; };
+  // one and the D2H copy of the one before that.  Each entry stages into its own slots.
+  struct Lane { cudaStream_t stream = nullptr; DevBuf body[3], resident[4], step[4]; };
   static const int kLanes = 8;
   Lane lanes[8];
   unsigned lane_next = 0;
   // device-resident buffers the pipelined calls read AND write (planner state): the last
   // enqueued writer per buffer, so that a later call on another lane is ordered after it
   std::map<const void*, cudaEvent_t> last_writer;
-  // per caller stream: {next, done} scheduler counters of the persistent body kernels and the hand-over list
-  // {count, total, ids[kFlistCap]}.  Keyed by stream because launches on one stream are ordered, so a block is idle
-  // again when the next launch on that stream starts; launches on different streams never share counters.
-  struct StreamCtl { int* p = nullptr; };
-  std::map<cudaStream_t, StreamCtl> ctl;
-  // staging of go1mpc_control_tick_host_async, one set per caller stream (grown on demand): tick | step_in | body tick
-  // records | expanded body records | out38 | planner diag | body diag
-  struct TickWs { DevBuf b[7]; int zero_B = -1; };   // zero_B: batch size for which rows 10..19 of the planner inputs are known zero
-  std::map<cudaStream_t, TickWs> tick_ws;
+  std::map<cudaStream_t, StreamWs> ws;   // per caller stream, at most 256 (stream_ws)
   cudaStream_t side = nullptr;     // side stream of the planner tick's out-of-place state copy
   bool phase_timing = false;       // go1mpc_body_phase_timing: events around the three launches of the body tick
   cudaEvent_t phase_ev[4] = {nullptr, nullptr, nullptr, nullptr};
   double* squat_d = nullptr;       // X_CoM_position_squat table of the planner node (host libm), built on first use
-  struct NlpWs { DevBuf b[7]; };   // workspace of go1mpc_nlp_node_tick_batch, one per caller stream
-  std::map<cudaStream_t, NlpWs> nlp_ws;
-  // workspace of the gait stack entries, one per caller stream (grown on demand): sensor | /control2rtmpc/state |
-  // walkdtime ints | cmd | start | body-MPC input records | planner mask of the clocked tick | reset count, flags and robot list |
-  // farm copy count and lists
-  struct StackWs { DevBuf b[9]; int zero_B = -1; };   // zero_B: batch size for which the control message's other slots are zero
-  std::map<cudaStream_t, StackWs> stack_ws;
-  struct ServoWs { DevBuf ch, reset; };   // servo torque tick: filtered channels [SERVO_TICKS_MAX][9][B], reset flags [B]
-  std::map<cudaStream_t, ServoWs> servo_ws;
   std::map<int, double*> stack_col_d;   // go1mpc_gait_stack_default_state(nh) on the device, per nh, built on first use
   double* trtab_d = nullptr;       // remaining-time bound table of the planner tick (host libm), built on first use
   std::vector<cudaEvent_t> ev_pool;   // go1mpc_stream_wait: events, reused round-robin
@@ -90,10 +100,6 @@ struct go1mpc {
                                    // 65536, 2.6x at 4096 with calls in flight on several streams), the combined kernel below
                                    // (latency of a lone small batch: 64 vs 95 us at 256)
   int body_tri_min = 2048;         // GO1MPC_BODY_TRI_MIN
-  // body_tri workspace, one per stream the entry point is called with (calls on one stream are ordered, so the
-  // buffers are free again when the next call's first kernel starts); grown on demand
-  struct TriWs { char* p = nullptr; int capB = 0; size_t off[6] = {0, 0, 0, 0, 0, 0}; size_t qctl_off = 0; };
-  std::map<cudaStream_t, TriWs> tri_ws;
   bool force_generic = false;      // GO1MPC_FORCE_GENERIC=1: always use the run-time-sized kernel
   int step_mode = 0;               // 0 auto, 1 thread per planner, 2 warp per planner (GO1MPC_STEP_MODE)
   int step_warp_below = 1024;      // auto: warp per planner below this batch size (measured: 82 vs 124 us at B = 256,
@@ -219,34 +225,153 @@ int get_body_model(go1mpc* h, int nh, BodyModel** out) {
   return GO1MPC_OK;
 }
 
-// scheduler counters + hand-over list of the stream `st` (allocated and zeroed on first use)
-int get_ctl(go1mpc* h, cudaStream_t st, int** out) {
-  auto it = h->ctl.find(st);
-  if (it == h->ctl.end()) {
-    if (h->ctl.size() >= 256) return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-    int* p = nullptr;
-    const size_t bytes = sizeof(int) * (size_t)(kFlistCap + 4);
-    CU(h, cudaMalloc((void**)&p, bytes));
-    cudaError_t e = cudaMemset(p, 0, bytes);
-    if (e != cudaSuccess) { cudaFree(p); return cuda_fail(h, e, "cudaMemset(stream control block)"); }
-    it = h->ctl.emplace(st, go1mpc::StreamCtl{p}).first;
+// The workspace record of stream `st`, created on first use.  One handle serves at most 256 distinct streams.
+int stream_ws(go1mpc* h, cudaStream_t st, StreamWs** out) {
+  auto it = h->ws.find(st);
+  if (it == h->ws.end()) {
+    if (h->ws.size() >= 256) return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
+    it = h->ws.try_emplace(st).first;
   }
-  *out = it->second.p;
+  *out = &it->second;
   return GO1MPC_OK;
 }
 
-int stage_buf2(go1mpc* h, DevBuf& b, size_t bytes, void** out);
-int stage_buf(go1mpc* h, int slot, size_t bytes, void** out) { return stage_buf2(h, h->stage[slot], bytes, out); }
-int stage_buf2(go1mpc* h, DevBuf& b, size_t bytes, void** out) {
-  if (bytes > b.cap) {
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr; b.cap = 0;
-    size_t cap = bytes + bytes / 4 + 256;
-    CU(h, cudaMalloc(&b.p, cap));
-    b.cap = cap;
+// Makes `b` hold at least `bytes`.  A buffer that is too small is replaced: `st`, the stream that used it, is synchronised
+// first (its earlier work may still read the old buffer), and the new one has headroom so that slowly rising sizes do not
+// reallocate on every call.  *grew (optional) tells the caller that the contents are gone.
+int grow(go1mpc* h, DevBuf& b, size_t bytes, cudaStream_t st, bool* grew = nullptr) {
+  if (grew) *grew = false;
+  if (bytes <= b.cap) return GO1MPC_OK;
+  if (b.p) {
+    CU(h, cudaStreamSynchronize(st));
+    b.reset();
   }
-  *out = b.p;
+  const size_t cap = bytes + bytes / 4 + 256;
+  CU(h, cudaMalloc(&b.p, cap));
+  b.cap = cap;
+  if (grew) *grew = true;
   return GO1MPC_OK;
+}
+
+// The workspace record of `st` with its scheduler counters and hand-over list (allocated and zeroed on first use)
+int stream_ctl(go1mpc* h, cudaStream_t st, StreamWs** out) {
+  int rc = stream_ws(h, st, out);
+  if (rc) return rc;
+  DevBuf& c = (*out)->ctl;
+  if (!c.p) {
+    const size_t bytes = sizeof(int) * (size_t)(kFlistCap + 4);
+    if ((rc = grow(h, c, bytes, st))) return rc;
+    cudaError_t e = cudaMemset(c.p, 0, bytes);
+    if (e != cudaSuccess) { c.reset(); return cuda_fail(h, e, "cudaMemset(stream control block)"); }
+  }
+  return GO1MPC_OK;
+}
+
+// Device staging of one host-buffer call in a set of slots, on one stream.  Each up / inout / out takes the next slot, also
+// for a null host pointer, so that a buffer keeps its slot from call to call.  H2D copies are enqueued at once, D2H copies by
+// finish() in staging order.  The first failure is kept in rc; later staging then does nothing.
+struct Staging {
+  go1mpc* h;
+  DevBuf* slot;
+  int nslots;
+  cudaStream_t st;
+  int rc = GO1MPC_OK, next = 0, ndown = 0;
+  struct Down { void* host; const void* dev; size_t bytes; } down[16];   // at most one per slot
+
+  template <int N>
+  Staging(go1mpc* h_, DevBuf (&s)[N], cudaStream_t st_) : h(h_), slot(s), nslots(N), st(st_) {
+    static_assert(N <= 16, "one D2H copy per slot at most");
+    cudaError_t e = cudaSetDevice(h->device);   // a host thread other than the creating one starts on device 0
+    if (e != cudaSuccess) rc = cuda_fail(h, e, "cudaSetDevice");
+  }
+
+  void* stage(size_t bytes) {
+    assert(next < nslots);
+    DevBuf& b = slot[next++];
+    if (!rc) rc = grow(h, b, bytes, st);
+    return rc ? nullptr : b.p;
+  }
+  // copied up; a null host pointer gives a null device pointer
+  template <class T> T* up(const T* host, size_t bytes) {
+    if (!host) { next++; return nullptr; }
+    void* d = stage(bytes);
+    cudaError_t e = rc ? cudaSuccess : cudaMemcpyAsync(d, host, bytes, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) rc = cuda_fail(h, e, "cudaMemcpyAsync(H2D staging)");
+    return (T*)d;
+  }
+  // copied up, and down again by finish(); null gives null
+  template <class T> T* inout(T* host, size_t bytes) {
+    T* d = (T*)up(host, bytes);
+    if (host) down[ndown++] = Down{host, d, bytes};
+    return d;
+  }
+  // copied down by finish(); null gives null
+  template <class T> T* out(T* host, size_t bytes) {
+    if (!host) { next++; return nullptr; }
+    return out_always(host, bytes, bytes);
+  }
+  // staged even for a null host pointer (the kernel writes it either way); down_bytes are copied down when host is given
+  template <class T> T* out_always(T* host, size_t bytes, size_t down_bytes) {
+    void* d = stage(bytes);
+    if (host) down[ndown++] = Down{host, d, down_bytes};
+    return (T*)d;
+  }
+  // enqueues the D2H copies; with sync, waits for them
+  int finish(bool sync) {
+    for (int k = 0; k < ndown; k++) CU(h, cudaMemcpyAsync(down[k].host, down[k].dev, down[k].bytes, cudaMemcpyDeviceToHost, st));
+    if (sync) CU(h, cudaStreamSynchronize(st));
+    return GO1MPC_OK;
+  }
+  // the device entry, when staging succeeded, then finish()
+  template <class F> int run(bool sync, F launch) {
+    if (rc) return rc;
+    if (int r = launch()) return r;
+    return finish(sync);
+  }
+};
+
+// Launch parameters of the body-MPC kernels common to every path; a path adds its scheduler, hand-over list and workspace
+BodyKParams body_params(const go1mpc* h, const BodyModel& M, int nh, int B, const double* in_d, double* out_d, int* diag_d) {
+  const Go1BodyMpcConfig& c = h->cfg.body;
+  BodyKParams P{};
+  P.nh = nh; P.B = B; P.in_stride = go1mpc_body_in_stride(nh); P.out_stride = go1mpc_body_out_stride(nh);
+  P.diag_stride = go1mpc_body_diag_stride(nh);
+  P.tab_doubles = M.tab_doubles; P.warp_doubles = 0;
+  P.cap_scale = h->cfg.qp_iter_cap_scale; P.gate = M.gate; P.nstepx = M.nstepx; P.nsum_mpc = M.nsum_mpc;
+  P.in = in_d; P.out = out_d; P.diag = diag_d; P.tab = M.tab_d; P.sched = nullptr;
+  P.flist = nullptr; P.flist_count = nullptr; P.flist_cap = 0;
+  P.dt_mpc = c.dt_mpc; P.j_ini = c.j_ini; P.mass = c.mass; P.g = c.g; P.gama = c.gama_zmp;
+  P.theta_lim = c.theta_lim; P.torque_lim = c.torque_lim;
+  for (int k = 0; k < 4; k++) P.lamda[k] = c.lamda[k];
+  return P;
+}
+
+// The 12-variable force QP of Dynamiccclass::force_opt: weights, friction and force bound of dynmics_compute.cpp:59-63
+GrfKParams grf_params(const go1mpc* h, int B, const double* in_d, double* out_d, int* diag_d) {
+  GrfKParams P;
+  P.B = B; P.cap = h->cfg.qp_iter_cap_scale * (12 + 12 + 24) + 50; P.warp_doubles = 0;
+  P.qp_alpha = 10000; P.qp_beta = 1000; P.qp_gama = 10; P.fz_max = 160; P.mu = 0.25;
+  P.in = in_d; P.out = out_d; P.diag = diag_d;
+  return P;
+}
+constexpr double kSwingKp = 1, kSwingKd = 0.01;   // swing-leg gains of compute_joint_torques (dynmics_compute.cpp:37-38)
+
+// The servo stack kernel's parameters from a Go1ServoStackTick or a Go1ServoTorqueTick (the same leading fields); ch: null or
+// where the kernel stores each tick's filtered channels
+template <class Tick>
+ServoStackKParams servo_stack_params(const go1mpc* h, int B, const Tick* t, double* ch) {
+  const size_t b = (size_t)B;
+  ServoStackKParams P;
+  P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
+  P.half_hip_width = h->cfg.step.half_hip_width; P.y_offset = t->y_offset;
+  double k6[6];
+  go1mpc_lpf_coefficients(1000.0, 3.0, k6);                     // the servo loop's 3 Hz filters at 1 kHz
+  P.coef = LpfCoef{k6[0], k6[1], k6[2], k6[3], k6[4], k6[5]};
+  P.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
+  P.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
+  P.state = t->servo_state_d; P.q_out = t->q_d;
+  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d; P.ch = ch;
+  return P;
 }
 
 }  // namespace
@@ -329,26 +454,16 @@ void go1mpc_destroy(go1mpc_t* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   for (auto& kv : h->body_models) if (kv.second.tab_d) cudaFree(kv.second.tab_d);
-  for (DevBuf& b : h->stage) if (b.p) cudaFree(b.p);
-  for (auto& kv : h->ctl) if (kv.second.p) cudaFree(kv.second.p);
-  for (auto& kv : h->tri_ws) if (kv.second.p) cudaFree(kv.second.p);
   for (auto& kv : h->last_writer) cudaEventDestroy(kv.second);
-  for (auto& kv : h->tick_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
   for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
   if (h->trtab_d) cudaFree(h->trtab_d);
   if (h->squat_d) cudaFree(h->squat_d);
   for (cudaEvent_t e : h->phase_ev) if (e) cudaEventDestroy(e);
-  for (auto& kv : h->nlp_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
-  for (auto& kv : h->stack_ws) for (DevBuf& b : kv.second.b) if (b.p) cudaFree(b.p);
-  for (auto& kv : h->servo_ws) for (DevBuf* b : {&kv.second.ch, &kv.second.reset}) if (b->p) cudaFree(b->p);
   for (auto& kv : h->stack_col_d) cudaFree(kv.second);
-  for (auto& L : h->lanes) {
-    for (DevBuf& b : L.stage) if (b.p) cudaFree(b.p);
-    if (L.stream) cudaStreamDestroy(L.stream);
-  }
+  for (auto& L : h->lanes) if (L.stream) cudaStreamDestroy(L.stream);
   if (h->side) cudaStreamDestroy(h->side);
   if (h->stream) cudaStreamDestroy(h->stream);
-  delete h;
+  delete h;   // frees the staging and every stream's workspace (DevBuf)
 }
 
 const char* go1mpc_last_error(const go1mpc_t* h) { return h ? h->err.c_str() : "null handle"; }
@@ -411,37 +526,23 @@ int go1mpc_qp_solve_batch_host(go1mpc_t* h, int n, int p, int m, int B, const do
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
-  CU(h, cudaSetDevice(h->device));
   const size_t szd = sizeof(double), szi = sizeof(int), b = (size_t)B;
-  void *dG, *dg0, *dCE = nullptr, *dce0 = nullptr, *dCI = nullptr, *dci0 = nullptr, *dx, *dcost, *dact, *dna, *dit, *dst;
-  int rc;
-  if ((rc = stage_buf(h, 0, b * n * n * szd, &dG))) return rc;
-  if ((rc = stage_buf(h, 1, b * n * szd, &dg0))) return rc;
-  if (p) { if ((rc = stage_buf(h, 2, b * n * p * szd, &dCE))) return rc; if ((rc = stage_buf(h, 3, b * p * szd, &dce0))) return rc; }
-  if (m) { if ((rc = stage_buf(h, 4, b * n * m * szd, &dCI))) return rc; if ((rc = stage_buf(h, 5, b * m * szd, &dci0))) return rc; }
-  if ((rc = stage_buf(h, 6, b * n * szd, &dx))) return rc;
-  if ((rc = stage_buf(h, 7, b * szd, &dcost))) return rc;
-  if ((rc = stage_buf(h, 8, b * (m + p + 1) * szi, &dact))) return rc;
-  if ((rc = stage_buf(h, 9, b * szi, &dna))) return rc;
-  if ((rc = stage_buf(h, 10, b * 6 * szi, &dit))) return rc;
-  if ((rc = stage_buf(h, 11, b * szi, &dst))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(dG, G, b * n * n * szd, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dg0, g0, b * n * szd, cudaMemcpyHostToDevice, st));
-  if (p) { CU(h, cudaMemcpyAsync(dCE, CE, b * n * p * szd, cudaMemcpyHostToDevice, st)); CU(h, cudaMemcpyAsync(dce0, ce0, b * p * szd, cudaMemcpyHostToDevice, st)); }
-  if (m) { CU(h, cudaMemcpyAsync(dCI, CI, b * n * m * szd, cudaMemcpyHostToDevice, st)); CU(h, cudaMemcpyAsync(dci0, ci0, b * m * szd, cudaMemcpyHostToDevice, st)); }
-  CU(h, cudaMemcpyAsync(dx, x, b * n * szd, cudaMemcpyHostToDevice, st));
-  rc = go1mpc_qp_solve_batch(h, n, p, m, B, (double*)dG, (double*)dg0, (double*)dCE, (double*)dce0, (double*)dCI,
-                             (double*)dci0, (double*)dx, (double*)dcost, (int*)dact, (int*)dna, (int*)dit, (int*)dst, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(x, dx, b * n * szd, cudaMemcpyDeviceToHost, st));
-  if (cost) CU(h, cudaMemcpyAsync(cost, dcost, b * szd, cudaMemcpyDeviceToHost, st));
-  if (active) CU(h, cudaMemcpyAsync(active, dact, b * (m + p) * szi, cudaMemcpyDeviceToHost, st));
-  if (nactive) CU(h, cudaMemcpyAsync(nactive, dna, b * szi, cudaMemcpyDeviceToHost, st));
-  if (iters) CU(h, cudaMemcpyAsync(iters, dit, b * 6 * szi, cudaMemcpyDeviceToHost, st));
-  if (status) CU(h, cudaMemcpyAsync(status, dst, b * szi, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  Staging S(h, h->stage, h->stream);
+  const double* dG = S.up(G, b * n * n * szd);
+  const double* dg0 = S.up(g0, b * n * szd);
+  const double* dCE = S.up(p ? CE : nullptr, b * n * p * szd);
+  const double* dce0 = S.up(p ? ce0 : nullptr, b * p * szd);
+  const double* dCI = S.up(m ? CI : nullptr, b * n * m * szd);
+  const double* dci0 = S.up(m ? ci0 : nullptr, b * m * szd);
+  double* dx = S.inout(x, b * n * szd);
+  double* dcost = S.out_always(cost, b * szd, b * szd);
+  int* dact = S.out_always(active, b * (m + p + 1) * szi, b * (m + p) * szi);
+  int* dna = S.out_always(nactive, b * szi, b * szi);
+  int* dit = S.out_always(iters, b * 6 * szi, b * 6 * szi);
+  int* dst = S.out_always(status, b * szi, b * szi);
+  return S.run(true, [&] {
+    return go1mpc_qp_solve_batch(h, n, p, m, B, dG, dg0, dCE, dce0, dCI, dci0, dx, dcost, dact, dna, dit, dst, S.st);
+  });
 }
 
 // ------------------------------------------------------------------ body MPC
@@ -461,39 +562,35 @@ int go1mpc_body_mpc_step_batch(go1mpc_t* h, int nh, int B, const double* in_d, d
   BodyModel* M;
   int rc = get_body_model(h, nh, &M);
   if (rc) return rc;
-  const int is = go1mpc_body_in_stride(nh), os = go1mpc_body_out_stride(nh);
+  BodyKParams P = body_params(h, *M, nh, B, in_d, out_d, diag_d);
   if (body_fast_supported(nh) && !h->force_generic && h->body_mode != 4) {
-    const Go1BodyMpcConfig& c = h->cfg.body;
-    BodyKParams P;
-    P.nh = nh; P.B = B; P.in_stride = is; P.out_stride = os; P.diag_stride = go1mpc_body_diag_stride(nh);
-    P.tab_doubles = M->tab_doubles; P.warp_doubles = 0;
-    P.cap_scale = h->cfg.qp_iter_cap_scale; P.gate = M->gate; P.nstepx = M->nstepx; P.nsum_mpc = M->nsum_mpc;
-    P.in = in_d; P.out = out_d; P.diag = diag_d; P.tab = M->tab_d;
-    int* ctl = nullptr;
-    if ((rc = get_ctl(h, st, &ctl))) return rc;
+    StreamWs* W;
+    if ((rc = stream_ctl(h, st, &W))) return rc;
+    int* ctl = (int*)W->ctl.p;
     P.sched = ctl;
-    P.flist = nullptr; P.flist_count = nullptr; P.flist_cap = 0;
-    P.dt_mpc = c.dt_mpc; P.j_ini = c.j_ini; P.mass = c.mass; P.g = c.g; P.gama = c.gama_zmp;
-    P.theta_lim = c.theta_lim; P.torque_lim = c.torque_lim;
-    for (int k = 0; k < 4; k++) P.lamda[k] = c.lamda[k];
     if (body_tri_supported(nh) && (h->body_mode == 2 || (h->body_mode == 3 && B >= h->body_tri_min))) {
-      if (h->tri_ws.size() >= 64 && h->tri_ws.find(st) == h->tri_ws.end()) {
-        // a caller that keeps creating streams: drop the workspaces of the old ones (their work is done after the sync)
-        CU(h, cudaDeviceSynchronize());
-        for (auto& kv : h->tri_ws) if (kv.second.p) cudaFree(kv.second.p);
-        h->tri_ws.clear();
+      if (!W->tri.buf.p) {
+        // a caller that keeps creating streams: past 64 streams with a workspace, drop them all (their work is done after
+        // the sync)
+        int held = 0;
+        for (auto& kv : h->ws) held += kv.second.tri.buf.p != nullptr;
+        if (held >= 64) {
+          CU(h, cudaDeviceSynchronize());
+          for (auto& kv : h->ws) { kv.second.tri.buf.reset(); kv.second.tri.capB = 0; }
+        }
       }
-      go1mpc::TriWs& W = h->tri_ws[st];
-      if (W.capB < B) {
-        if (W.p) { CU(h, cudaStreamSynchronize(st)); cudaFree(W.p); W.p = nullptr; W.capB = 0; }
-        const size_t bytes = body_tri_workspace_bytes(nh, B, W.off);
-        W.qctl_off = bytes;
-        CU(h, cudaMalloc((void**)&W.p, bytes + 16));
-        CU(h, cudaMemsetAsync(W.p + W.qctl_off, 0, 16, st));
-        W.capB = B;
+      auto& T = W->tri;
+      if (T.capB < B) {
+        // laid out anew for B instances, with the queue control block cleared
+        const size_t bytes = body_tri_workspace_bytes(nh, B, T.off);
+        T.qctl_off = bytes;
+        if ((rc = grow(h, T.buf, bytes + 16, st))) return rc;
+        CU(h, cudaMemsetAsync((char*)T.buf.p + T.qctl_off, 0, 16, st));
+        T.capB = B;
       }
-      P.tri_jb = (double*)(W.p + W.off[0]); P.tri_hs = (double*)(W.p + W.off[1]); P.tri_res = (double*)(W.p + W.off[2]);
-      P.tri_queue = (int*)(W.p + W.off[3]); P.tri_qctl = (int*)(W.p + W.qctl_off); P.tri_meta = (int*)(W.p + W.off[4]); P.tri_fr = (double*)(W.p + W.off[5]);
+      char* p = (char*)T.buf.p;
+      P.tri_jb = (double*)(p + T.off[0]); P.tri_hs = (double*)(p + T.off[1]); P.tri_res = (double*)(p + T.off[2]);
+      P.tri_queue = (int*)(p + T.off[3]); P.tri_qctl = (int*)(p + T.qctl_off); P.tri_meta = (int*)(p + T.off[4]); P.tri_fr = (double*)(p + T.off[5]);
       int* fl = ctl + 2;
       P.flist_count = fl; P.flist = fl + 2; P.flist_cap = kFlistCap;
       CU(h, body_tri_launch(P, M->tab_h.data(), h->sms, st, h->phase_timing ? h->phase_ev : nullptr));
@@ -521,31 +618,21 @@ int go1mpc_body_mpc_step_batch(go1mpc_t* h, int nh, int B, const double* in_d, d
   // the instances it hands over (normally none); GO1MPC_FORCE_GENERIC=1 keeps the dense kernel alone
   const bool duo = !h->force_generic;
   int wpc = 4, wd = 0;
-  size_t smem = body_smem_bytes(nh, wpc, is, os, M->tab_doubles, &wd);
-  while (wpc > 1 && smem > h->smem_optin / 2) { wpc >>= 1; smem = body_smem_bytes(nh, wpc, is, os, M->tab_doubles, &wd); }
+  size_t smem = body_smem_bytes(nh, wpc, P.in_stride, P.out_stride, M->tab_doubles, &wd);
+  while (wpc > 1 && smem > h->smem_optin / 2) { wpc >>= 1; smem = body_smem_bytes(nh, wpc, P.in_stride, P.out_stride, M->tab_doubles, &wd); }
   if (smem > h->smem_optin) return fail(h, GO1MPC_E_UNSUPPORTED, "body_mpc_step_batch: workspace exceeds shared memory");
   int occ = 0;
   CU(h, body_mpc_occupancy(wpc, smem, &occ));
   if (occ < 1) return fail(h, GO1MPC_E_UNSUPPORTED, "body_mpc_step_batch: kernel does not fit on an SM");
   int grid = (B + wpc - 1) / wpc;
   if (grid > h->sms * occ) grid = h->sms * occ;
-  const Go1BodyMpcConfig& c = h->cfg.body;
-  BodyKParams P;
-  P.nh = nh; P.B = B; P.in_stride = is; P.out_stride = os; P.diag_stride = go1mpc_body_diag_stride(nh);
-  P.tab_doubles = M->tab_doubles; P.warp_doubles = wd;
-  P.cap_scale = h->cfg.qp_iter_cap_scale; P.gate = M->gate; P.nstepx = M->nstepx; P.nsum_mpc = M->nsum_mpc;
-  P.in = in_d; P.out = out_d; P.diag = diag_d; P.tab = M->tab_d; P.sched = nullptr;
-  P.flist = nullptr; P.flist_count = nullptr; P.flist_cap = 0;
-  P.dt_mpc = c.dt_mpc; P.j_ini = c.j_ini; P.mass = c.mass; P.g = c.g; P.gama = c.gama_zmp;
-  P.theta_lim = c.theta_lim; P.torque_lim = c.torque_lim;
-  for (int k = 0; k < 4; k++) P.lamda[k] = c.lamda[k];
+  P.warp_doubles = wd;
   if (duo) {
-    int* ctl = nullptr;
-    if ((rc = get_ctl(h, st, &ctl))) return rc;
-    int* fl = ctl + 2;
+    StreamWs* W;
+    if ((rc = stream_ctl(h, st, &W))) return rc;
+    int* fl = (int*)W->ctl.p + 2;
     P.flist_count = fl; P.flist = fl + 2; P.flist_cap = kFlistCap;
     CU(h, body_duo_launch(P, h->sms, h->smem_optin, st));
-    P.warp_doubles = wd;
     CU(h, body_mpc_launch(P, wpc, grid, smem, st));           // list mode
     CU(h, cudaMemsetAsync(fl, 0, sizeof(int), st));
     h->launches += 2;
@@ -583,9 +670,10 @@ int go1mpc_body_handover_total(go1mpc_t* h, long long* total) {
   CU(h, cudaSetDevice(h->device));
   CU(h, cudaDeviceSynchronize());
   long long t = 0;
-  for (auto& kv : h->ctl) {
+  for (auto& kv : h->ws) {
+    if (!kv.second.ctl.p) continue;
     int v = 0;
-    CU(h, cudaMemcpy(&v, kv.second.p + 3, sizeof(int), cudaMemcpyDeviceToHost));
+    CU(h, cudaMemcpy(&v, (int*)kv.second.ctl.p + 3, sizeof(int), cudaMemcpyDeviceToHost));
     t += v;
   }
   *total = t;
@@ -600,10 +688,11 @@ int go1mpc_body_guard_trips(go1mpc_t* h, long long* total) {
   CU(h, cudaSetDevice(h->device));
   CU(h, cudaDeviceSynchronize());
   long long t = 0;
-  for (auto& kv : h->tri_ws) {
-    if (!kv.second.p) continue;
+  for (auto& kv : h->ws) {
+    const auto& T = kv.second.tri;
+    if (!T.buf.p) continue;
     int v = 0;
-    CU(h, cudaMemcpy(&v, kv.second.p + kv.second.qctl_off + 8, sizeof(int), cudaMemcpyDeviceToHost));
+    CU(h, cudaMemcpy(&v, (char*)T.buf.p + T.qctl_off + 8, sizeof(int), cudaMemcpyDeviceToHost));
     t += v;
   }
   *total = t;
@@ -615,24 +704,12 @@ int go1mpc_body_mpc_step_batch_host(go1mpc_t* h, int nh, int B, const double* in
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!in || !out) return fail(h, GO1MPC_E_INVALID, "body_mpc_step_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  const size_t ib = (size_t)B * go1mpc_body_in_stride(nh) * sizeof(double);
-  const size_t ob = (size_t)B * go1mpc_body_out_stride(nh) * sizeof(double);
-  const size_t db = (size_t)B * go1mpc_body_diag_stride(nh) * sizeof(int);
-  void *din, *dout, *ddiag = nullptr;
-  int rc;
-  if ((rc = stage_buf(h, 12, ib, &din))) return rc;
-  if ((rc = stage_buf(h, 13, ob, &dout))) return rc;
-  if (diag && (rc = stage_buf(h, 14, db, &ddiag))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(din, in, ib, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dout, out, ob, cudaMemcpyHostToDevice, st));   // out14 is in/out (gated ticks)
-  rc = go1mpc_body_mpc_step_batch(h, nh, B, (const double*)din, (double*)dout, (int*)ddiag, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(out, dout, ob, cudaMemcpyDeviceToHost, st));
-  if (diag) CU(h, cudaMemcpyAsync(diag, ddiag, db, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  const size_t b = (size_t)B;
+  Staging S(h, h->stage, h->stream);
+  const double* din = S.up(in, b * go1mpc_body_in_stride(nh) * sizeof(double));
+  double* dout = S.inout(out, b * go1mpc_body_out_stride(nh) * sizeof(double));   // out14 is in/out (gated ticks)
+  int* ddiag = S.out(diag, b * go1mpc_body_diag_stride(nh) * sizeof(int));
+  return S.run(true, [&] { return go1mpc_body_mpc_step_batch(h, nh, B, din, dout, ddiag, S.st); });
 }
 
 int go1mpc_body_model(go1mpc_t* h, int nh, double* pps, double* pvs, double* ppu, double* pvu, double* ppu_2, double* pvu_2) {
@@ -749,28 +826,14 @@ int go1mpc_step_timing_step_batch_host(go1mpc_t* h, int n_sqp, int B, const int*
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!tick || !state || !in || !out) return fail(h, GO1MPC_E_INVALID, "step_timing_step_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
   const size_t b = (size_t)B;
-  const size_t tb = b * sizeof(int), sb = b * STEP_STATE_DOUBLES * sizeof(double), ib = b * STEP_IN_DOUBLES * sizeof(double);
-  const size_t ob = b * STEP_OUT_DOUBLES * sizeof(double), db = b * STEP_DIAG_INTS * sizeof(int);
-  void *dt_, *ds, *di, *do_, *dd = nullptr;
-  int rc;
-  if ((rc = stage_buf(h, 0, tb, &dt_))) return rc;
-  if ((rc = stage_buf(h, 1, sb, &ds))) return rc;
-  if ((rc = stage_buf(h, 2, ib, &di))) return rc;
-  if ((rc = stage_buf(h, 3, ob, &do_))) return rc;
-  if (diag && (rc = stage_buf(h, 4, db, &dd))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(dt_, tick, tb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(ds, state, sb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(di, in, ib, cudaMemcpyHostToDevice, st));
-  rc = go1mpc_step_timing_step_batch(h, n_sqp, B, (const int*)dt_, (const double*)ds, (double*)ds, (const double*)di, (double*)do_, (int*)dd, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(state, ds, sb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaMemcpyAsync(out, do_, ob, cudaMemcpyDeviceToHost, st));
-  if (diag) CU(h, cudaMemcpyAsync(diag, dd, db, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  Staging S(h, h->stage, h->stream);
+  const int* dt_ = S.up(tick, b * sizeof(int));
+  double* ds = S.inout(state, b * STEP_STATE_DOUBLES * sizeof(double));
+  const double* di = S.up(in, b * STEP_IN_DOUBLES * sizeof(double));
+  double* do_ = S.out(out, b * STEP_OUT_DOUBLES * sizeof(double));
+  int* dd = S.out(diag, b * STEP_DIAG_INTS * sizeof(int));
+  return S.run(true, [&] { return go1mpc_step_timing_step_batch(h, n_sqp, B, dt_, ds, ds, di, do_, dd, S.st); });
 }
 
 // NLPClass::FootStepInputs (NLP/NLP/NLPClass_sqp.cpp:51-75) + Initialize (:131-206) step tables
@@ -841,37 +904,19 @@ int go1mpc_foot_trajectory_stop_batch_host(go1mpc_t* h, int B, const int* tick, 
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!tick || !state || !out38 || !foot || !out18) return fail(h, GO1MPC_E_INVALID, "foot_trajectory_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  const size_t b = (size_t)B, tb = b * sizeof(int), sb = b * STEP_STATE_DOUBLES * sizeof(double), ob = b * STEP_OUT_DOUBLES * sizeof(double);
-  const size_t fb = b * FOOT_STATE_DOUBLES * sizeof(double), o18 = b * FOOT_OUT_DOUBLES * sizeof(double);
-  void *dt_, *ds, *do_, *df, *d18, *drs = nullptr;
-  int rc;
-  if ((rc = stage_buf(h, 0, tb, &dt_))) return rc;
-  if ((rc = stage_buf(h, 1, sb, &ds))) return rc;
-  if ((rc = stage_buf(h, 3, ob, &do_))) return rc;
-  if ((rc = stage_buf(h, 5, fb, &df))) return rc;
-  if ((rc = stage_buf(h, 6, o18, &d18))) return rc;
-  if (right_support && (rc = stage_buf(h, 7, tb, &drs))) return rc;
-  void *dl0 = nullptr, *dstop = nullptr;
-  const size_t lb = b * sizeof(double);
-  if (lift0 && (rc = stage_buf(h, 8, lb, &dl0))) return rc;
-  if (lift0 && stop && (rc = stage_buf(h, 9, lb, &dstop))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(dt_, tick, tb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(ds, state, sb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(do_, out38, ob, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(df, foot, fb, cudaMemcpyHostToDevice, st));
-  if (lift0) CU(h, cudaMemcpyAsync(dl0, lift0, lb, cudaMemcpyHostToDevice, st));
-  if (dstop) CU(h, cudaMemcpyAsync(dstop, stop, lb, cudaMemcpyHostToDevice, st));
-  rc = foot_enqueue(h, B, (const int*)dt_, (const double*)ds, (const double*)do_, (double*)df, (double*)d18, (int*)drs, st,
-                    (double*)dl0, (const double*)dstop, lift0 ? go1mpc_nlp_t_end_footstep(h) : 0);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(foot, df, fb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaMemcpyAsync(out18, d18, o18, cudaMemcpyDeviceToHost, st));
-  if (right_support) CU(h, cudaMemcpyAsync(right_support, drs, tb, cudaMemcpyDeviceToHost, st));
-  if (lift0) CU(h, cudaMemcpyAsync(lift0, dl0, lb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  const size_t b = (size_t)B;
+  Staging S(h, h->stage, h->stream);
+  const int* dt_ = S.up(tick, b * sizeof(int));
+  const double* ds = S.up(state, b * STEP_STATE_DOUBLES * sizeof(double));
+  const double* do_ = S.up(out38, b * STEP_OUT_DOUBLES * sizeof(double));
+  double* df = S.inout(foot, b * FOOT_STATE_DOUBLES * sizeof(double));
+  double* d18 = S.out(out18, b * FOOT_OUT_DOUBLES * sizeof(double));
+  int* drs = S.out(right_support, b * sizeof(int));
+  double* dl0 = S.inout(lift0, b * sizeof(double));
+  const double* dstop = S.up(lift0 ? stop : nullptr, b * sizeof(double));
+  return S.run(true, [&] {
+    return foot_enqueue(h, B, dt_, ds, do_, df, d18, drs, S.st, dl0, dstop, lift0 ? go1mpc_nlp_t_end_footstep(h) : 0);
+  });
 }
 // initial foot window: _Rfooty = -stepwidth(0), _Lfooty = +stepwidth(0), rest 0 (NLPClass_sqp.cpp:496-500)
 int go1mpc_foot_default_state(go1mpc_t* h, double* fs) {
@@ -890,11 +935,7 @@ int go1mpc_grf_force_opt_batch(go1mpc_t* h, int B, const double* in_d, double* o
   if (B < 0 || !in_d || !out_d) return fail(h, GO1MPC_E_INVALID, "grf_force_opt_batch: bad argument");
   if (B == 0) return GO1MPC_OK;
   CU(h, cudaSetDevice(h->device));
-  GrfKParams P;
-  P.B = B; P.cap = h->cfg.qp_iter_cap_scale * (12 + 12 + 24) + 50; P.warp_doubles = 0;
-  P.qp_alpha = 10000; P.qp_beta = 1000; P.qp_gama = 10; P.fz_max = 160; P.mu = 0.25;   // dynmics_compute.cpp:59-63
-  P.in = in_d; P.out = out_d; P.diag = diag_d;
-  CU(h, grf_force_opt_launch(P, h->sms, stream ? (cudaStream_t)stream : h->stream));
+  CU(h, grf_force_opt_launch(grf_params(h, B, in_d, out_d, diag_d), h->sms, stream ? (cudaStream_t)stream : h->stream));
   h->launches++;
   return GO1MPC_OK;
 }
@@ -926,7 +967,7 @@ int go1mpc_grf_joint_torques_batch(go1mpc_t* h, int B, const double* jac_d, cons
   if (B == 0) return GO1MPC_OK;
   CU(h, cudaSetDevice(h->device));
   GrfTauParams P;
-  P.B = B; P.swing_kp = 1; P.swing_kd = 0.01;   // dynmics_compute.cpp:37-38
+  P.B = B; P.swing_kp = kSwingKp; P.swing_kd = kSwingKd;
   P.jac = jac_d; P.swing = swing_d; P.p_des = p_des_d; P.p_est = p_est_d; P.pv_des = pv_des_d; P.pv_est = pv_est_d;
   P.F_leg_ref = F_leg_ref_d; P.f_ks = F_elem_stride; P.f_bs = F_robot_stride; P.tau = tau_d;
   CU(h, grf_joint_torques_launch(P, stream ? (cudaStream_t)stream : h->stream));
@@ -940,22 +981,12 @@ int go1mpc_grf_force_opt_batch_host(go1mpc_t* h, int B, const double* in, double
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!in || !out) return fail(h, GO1MPC_E_INVALID, "grf_force_opt_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  const size_t ib = (size_t)B * GRF_IN_DOUBLES * sizeof(double), ob = (size_t)B * GRF_OUT_DOUBLES * sizeof(double);
-  const size_t db = (size_t)B * GRF_DIAG_INTS * sizeof(int);
-  void *di, *do_, *dd = nullptr;
-  int rc;
-  if ((rc = stage_buf(h, 0, ib, &di))) return rc;
-  if ((rc = stage_buf(h, 1, ob, &do_))) return rc;
-  if (diag && (rc = stage_buf(h, 2, db, &dd))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(di, in, ib, cudaMemcpyHostToDevice, st));
-  rc = go1mpc_grf_force_opt_batch(h, B, (const double*)di, (double*)do_, (int*)dd, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(out, do_, ob, cudaMemcpyDeviceToHost, st));
-  if (diag) CU(h, cudaMemcpyAsync(diag, dd, db, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  const size_t b = (size_t)B;
+  Staging S(h, h->stage, h->stream);
+  const double* di = S.up(in, b * GRF_IN_DOUBLES * sizeof(double));
+  double* do_ = S.out(out, b * GRF_OUT_DOUBLES * sizeof(double));
+  int* dd = S.out(diag, b * GRF_DIAG_INTS * sizeof(int));
+  return S.run(true, [&] { return go1mpc_grf_force_opt_batch(h, B, di, do_, dd, S.st); });
 }
 int go1mpc_grf_force_distribution_batch_host(go1mpc_t* h, int B, int gait_mode, double y_coefficient, const double* com_des,
                                              const double* leg_des, const double* F_force_des, const double* rfoot_des,
@@ -965,24 +996,17 @@ int go1mpc_grf_force_distribution_batch_host(go1mpc_t* h, int B, int gait_mode, 
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!com_des || !leg_des || !F_force_des || !rfoot_des || !lfoot_des || !F_leg_ref)
     return fail(h, GO1MPC_E_INVALID, "grf_force_distribution_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
   const size_t d = (size_t)B * sizeof(double);
-  const double* src[5] = {com_des, leg_des, F_force_des, rfoot_des, lfoot_des};
-  const int rows[5] = {3, 12, 6, 3, 3};
-  void* dev[6];
-  int rc;
-  cudaStream_t st = h->stream;
-  for (int k = 0; k < 5; k++) {
-    if ((rc = stage_buf(h, k, rows[k] * d, &dev[k]))) return rc;
-    CU(h, cudaMemcpyAsync(dev[k], src[k], rows[k] * d, cudaMemcpyHostToDevice, st));
-  }
-  if ((rc = stage_buf(h, 5, 12 * d, &dev[5]))) return rc;
-  rc = go1mpc_grf_force_distribution_batch(h, B, gait_mode, y_coefficient, (const double*)dev[0], (const double*)dev[1],
-                                           (const double*)dev[2], (const double*)dev[3], (const double*)dev[4], (double*)dev[5], st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(F_leg_ref, dev[5], 12 * d, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  Staging S(h, h->stage, h->stream);
+  const double* dcom = S.up(com_des, 3 * d);
+  const double* dleg = S.up(leg_des, 12 * d);
+  const double* dF = S.up(F_force_des, 6 * d);
+  const double* drf = S.up(rfoot_des, 3 * d);
+  const double* dlf = S.up(lfoot_des, 3 * d);
+  double* dref = S.out(F_leg_ref, 12 * d);
+  return S.run(true, [&] {
+    return go1mpc_grf_force_distribution_batch(h, B, gait_mode, y_coefficient, dcom, dleg, dF, drf, dlf, dref, S.st);
+  });
 }
 int go1mpc_grf_joint_torques_batch_host(go1mpc_t* h, int B, const double* jac, const int* swing, const double* p_des,
                                         const double* p_est, const double* pv_des, const double* pv_est,
@@ -992,26 +1016,20 @@ int go1mpc_grf_joint_torques_batch_host(go1mpc_t* h, int B, const double* jac, c
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!jac || !swing || !p_des || !p_est || !pv_des || !pv_est || !F_leg_ref || !tau || F_elem_stride < 0 || F_robot_stride < 0)
     return fail(h, GO1MPC_E_INVALID, "grf_joint_torques_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
   const size_t d = (size_t)B * sizeof(double);
   const size_t fdoubles = (size_t)(11 * F_elem_stride + (B - 1) * F_robot_stride + 1);   // extent the strides address
-  const void* src[7] = {jac, swing, p_des, p_est, pv_des, pv_est, F_leg_ref};
-  const size_t bytes[7] = {36 * d, 4 * (size_t)B * sizeof(int), 12 * d, 12 * d, 12 * d, 12 * d, fdoubles * sizeof(double)};
-  void* dev[8];
-  int rc;
-  cudaStream_t st = h->stream;
-  for (int k = 0; k < 7; k++) {
-    if ((rc = stage_buf(h, k, bytes[k], &dev[k]))) return rc;
-    CU(h, cudaMemcpyAsync(dev[k], src[k], bytes[k], cudaMemcpyHostToDevice, st));
-  }
-  if ((rc = stage_buf(h, 7, 12 * d, &dev[7]))) return rc;
-  rc = go1mpc_grf_joint_torques_batch(h, B, (const double*)dev[0], (const int*)dev[1], (const double*)dev[2], (const double*)dev[3],
-                                      (const double*)dev[4], (const double*)dev[5], (const double*)dev[6], F_elem_stride,
-                                      F_robot_stride, (double*)dev[7], st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(tau, dev[7], 12 * d, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  Staging S(h, h->stage, h->stream);
+  const double* djac = S.up(jac, 36 * d);
+  const int* dsw = S.up(swing, 4 * (size_t)B * sizeof(int));
+  const double* dpd = S.up(p_des, 12 * d);
+  const double* dpe = S.up(p_est, 12 * d);
+  const double* dvd = S.up(pv_des, 12 * d);
+  const double* dve = S.up(pv_est, 12 * d);
+  const double* dF = S.up(F_leg_ref, fdoubles * sizeof(double));
+  double* dtau = S.out(tau, 12 * d);
+  return S.run(true, [&] {
+    return go1mpc_grf_joint_torques_batch(h, B, djac, dsw, dpd, dpe, dvd, dve, dF, F_elem_stride, F_robot_stride, dtau, S.st);
+  });
 }
 
 // ------------------------------------------------------------------ 40 Hz -> 100 Hz reference interpolation
@@ -1237,21 +1255,15 @@ int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d
     CU(h, cudaMalloc((void**)&h->squat_d, sizeof tab));
     CU(h, cudaMemcpy(h->squat_d, tab, sizeof tab, cudaMemcpyHostToDevice));
   }
-  // per-stream workspace: tick | in | out38 | out18 | right_support | hz_co | lipm
-  if (h->nlp_ws.size() >= 256 && h->nlp_ws.find(st) == h->nlp_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "nlp_node_tick_batch: more than 256 distinct streams used with one handle");
-  go1mpc::NlpWs& W = h->nlp_ws[st];
-  const size_t need[7] = {(size_t)B * sizeof(int), (size_t)B * STEP_IN_DOUBLES * sizeof(double), (size_t)B * STEP_OUT_DOUBLES * sizeof(double),
-                          (size_t)B * FOOT_OUT_DOUBLES * sizeof(double), (size_t)B * sizeof(int), (size_t)B * 8 * sizeof(double),
-                          (size_t)B * 6 * sizeof(double)};
-  for (int k = 0; k < 7; k++)
-    if (W.b[k].cap < need[k]) {
-      CU(h, cudaStreamSynchronize(st));
-      if (W.b[k].p) CU(h, cudaFree(W.b[k].p));
-      W.b[k].p = nullptr; W.b[k].cap = 0;
-      CU(h, cudaMalloc(&W.b[k].p, need[k]));
-      W.b[k].cap = need[k];
-    }
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  auto& ws = W->nlp;
+  const size_t b = (size_t)B, d = b * sizeof(double);
+  if ((rc = grow(h, ws.tick, b * sizeof(int), st)) || (rc = grow(h, ws.in, STEP_IN_DOUBLES * d, st)) ||
+      (rc = grow(h, ws.out38, STEP_OUT_DOUBLES * d, st)) || (rc = grow(h, ws.out18, FOOT_OUT_DOUBLES * d, st)) ||
+      (rc = grow(h, ws.right_support, b * sizeof(int), st)) || (rc = grow(h, ws.hz_co, 8 * d, st)) || (rc = grow(h, ws.lipm, 6 * d, st)))
+    return rc;
   NlpKParams P;
   P.B = B;
   nlp_limits(h, &P.t_end, &P.walkdtime_max);
@@ -1261,13 +1273,13 @@ int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d
   for (int q = 0; q < NLP_NTD_MAX; q++) { const double w = c.Wn * c.dt * (q + 1); P.sh_w[q] = sinh(w); P.ch_w[q] = cosh(w); }
   P.squat = h->squat_d; P.squat_n = kSquatN;
   P.node = state_d; P.walkdtime = walkdtime_d; P.start = start_d; P.cmd = cmd_d; P.rfoot_fb = rfoot_fb_d; P.lfoot_fb = lfoot_fb_d;
-  P.tick = (int*)W.b[0].p; P.in = (double*)W.b[1].p; P.out38 = (double*)W.b[2].p; P.out18 = (double*)W.b[3].p;
-  P.right_support = (int*)W.b[4].p; P.hz_co = (double*)W.b[5].p; P.lipm = (double*)W.b[6].p; P.msg = msg_d;
+  P.tick = (int*)ws.tick.p; P.in = (double*)ws.in.p; P.out38 = (double*)ws.out38.p; P.out18 = (double*)ws.out18.p;
+  P.right_support = (int*)ws.right_support.p; P.hz_co = (double*)ws.hz_co.p; P.lipm = (double*)ws.lipm.p; P.msg = msg_d;
   P.active = active_d;
   CU(h, nlp_pre_launch(P, st));
   h->launches++;
   // the planner state is rows [0, 202) of the node, the swing-foot window rows [202, 234): same SoA stride B
-  int rc = step_tick_enqueue(h, 3, B, P.tick, state_d, state_d, P.in, P.out38, nullptr, st, P.hz_co, P.lipm);
+  rc = step_tick_enqueue(h, 3, B, P.tick, state_d, state_d, P.in, P.out38, nullptr, st, P.hz_co, P.lipm);
   if (rc) return rc;
   rc = foot_enqueue(h, B, P.tick, state_d, P.out38, state_d + (size_t)STEP_STATE_DOUBLES * B, P.out18, P.right_support, st,
                     state_d + (size_t)kNlpLift0 * B, state_d + (size_t)kNlpStop * B, P.t_end);
@@ -1285,31 +1297,16 @@ int go1mpc_nlp_node_tick_batch_host(go1mpc_t* h, int B, double* state, const int
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!state || !walkdtime || !msg) return fail(h, GO1MPC_E_INVALID, "nlp_node_tick_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  const size_t b = (size_t)B, ib = b * sizeof(int), sb = b * NLP_NODE_DOUBLES * sizeof(double), fb = b * 3 * sizeof(double), mb = b * 100 * sizeof(double);
-  void *ds, *dw, *dst_ = nullptr, *dc = nullptr, *drf = nullptr, *dlf = nullptr, *dm;
-  int rc;
-  if ((rc = stage_buf(h, 0, sb, &ds))) return rc;
-  if ((rc = stage_buf(h, 1, ib, &dw))) return rc;
-  if (start && (rc = stage_buf(h, 2, ib, &dst_))) return rc;
-  if (cmd && (rc = stage_buf(h, 3, ib, &dc))) return rc;
-  if (rfoot_fb && (rc = stage_buf(h, 4, fb, &drf))) return rc;
-  if (lfoot_fb && (rc = stage_buf(h, 5, fb, &dlf))) return rc;
-  if ((rc = stage_buf(h, 6, mb, &dm))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(ds, state, sb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dw, walkdtime, ib, cudaMemcpyHostToDevice, st));
-  if (start) CU(h, cudaMemcpyAsync(dst_, start, ib, cudaMemcpyHostToDevice, st));
-  if (cmd) CU(h, cudaMemcpyAsync(dc, cmd, ib, cudaMemcpyHostToDevice, st));
-  if (rfoot_fb) CU(h, cudaMemcpyAsync(drf, rfoot_fb, fb, cudaMemcpyHostToDevice, st));
-  if (lfoot_fb) CU(h, cudaMemcpyAsync(dlf, lfoot_fb, fb, cudaMemcpyHostToDevice, st));
-  rc = go1mpc_nlp_node_tick_batch(h, B, (double*)ds, (const int*)dw, (const int*)dst_, (const int*)dc, (const double*)drf,
-                                  (const double*)dlf, (double*)dm, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(state, ds, sb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaMemcpyAsync(msg, dm, mb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  const size_t b = (size_t)B, ib = b * sizeof(int), fb = b * 3 * sizeof(double);
+  Staging S(h, h->stage, h->stream);
+  double* ds = S.inout(state, b * NLP_NODE_DOUBLES * sizeof(double));
+  const int* dw = S.up(walkdtime, ib);
+  const int* dst_ = S.up(start, ib);
+  const int* dc = S.up(cmd, ib);
+  const double* drf = S.up(rfoot_fb, fb);
+  const double* dlf = S.up(lfoot_fb, fb);
+  double* dm = S.out(msg, b * 100 * sizeof(double));
+  return S.run(true, [&] { return go1mpc_nlp_node_tick_batch(h, B, ds, dw, dst_, dc, drf, dlf, dm, S.st); });
 }
 
 // ------------------------------------------------------------------ the 100 Hz node (message in, message out)
@@ -1396,33 +1393,16 @@ int go1mpc_rt_node_tick_batch_host(go1mpc_t* h, int nh, int B, double* state, co
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!state || !msg || !body_out || !out100) return fail(h, GO1MPC_E_INVALID, "rt_node_tick_batch_host: bad argument");
   if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "rt_node_tick_batch_host: 3 <= nh <= 40");
-  CU(h, cudaSetDevice(h->device));
-  const size_t b = (size_t)B, sb = b * go1mpc_rt_node_state_doubles(nh) * sizeof(double), mb = b * 100 * sizeof(double);
-  const size_t ib = b * sizeof(int), ab = b * 4 * sizeof(double), bib = b * go1mpc_body_in_stride(nh) * sizeof(double);
-  const size_t bob = b * go1mpc_body_out_stride(nh) * sizeof(double);
-  void *ds, *dm, *dc = nullptr, *da = nullptr, *dbi, *dbo, *dout;
-  int rc;
-  if ((rc = stage_buf(h, 0, sb, &ds))) return rc;
-  if ((rc = stage_buf(h, 1, mb, &dm))) return rc;
-  if (ctrl && (rc = stage_buf(h, 2, ib, &dc))) return rc;
-  if (bodyangle_state && (rc = stage_buf(h, 3, ab, &da))) return rc;
-  if ((rc = stage_buf(h, 4, bib, &dbi))) return rc;
-  if ((rc = stage_buf(h, 5, bob, &dbo))) return rc;
-  if ((rc = stage_buf(h, 6, mb, &dout))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(ds, state, sb, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dm, msg, mb, cudaMemcpyHostToDevice, st));
-  if (ctrl) CU(h, cudaMemcpyAsync(dc, ctrl, ib, cudaMemcpyHostToDevice, st));
-  if (bodyangle_state) CU(h, cudaMemcpyAsync(da, bodyangle_state, ab, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dbo, body_out, bob, cudaMemcpyHostToDevice, st));
-  rc = go1mpc_rt_node_tick_batch(h, nh, B, (double*)ds, (const double*)dm, (const int*)dc, (const double*)da, (double*)dbi,
-                                 (double*)dbo, nullptr, (double*)dout, nullptr, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(state, ds, sb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaMemcpyAsync(body_out, dbo, bob, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaMemcpyAsync(out100, dout, mb, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
+  const size_t b = (size_t)B, mb = b * 100 * sizeof(double);
+  Staging S(h, h->stage, h->stream);
+  double* ds = S.inout(state, b * go1mpc_rt_node_state_doubles(nh) * sizeof(double));
+  const double* dm = S.up(msg, mb);
+  const int* dc = S.up(ctrl, b * sizeof(int));
+  const double* da = S.up(bodyangle_state, b * 4 * sizeof(double));
+  double* dbi = S.out_always((double*)nullptr, b * go1mpc_body_in_stride(nh) * sizeof(double), 0);   // the node writes the records
+  double* dbo = S.inout(body_out, b * go1mpc_body_out_stride(nh) * sizeof(double));
+  double* dout = S.out(out100, mb);
+  return S.run(true, [&] { return go1mpc_rt_node_tick_batch(h, nh, B, ds, dm, dc, da, dbi, dbo, nullptr, dout, nullptr, S.st); });
 }
 
 // ------------------------------------------------------------------ gait stack tick: both nodes behind one host call
@@ -1488,52 +1468,49 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
   }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-  go1mpc::StackWs& W = h->stack_ws[st];
-  const size_t b = (size_t)B;
-  const int nbuf = clock_d ? 7 : 6;
-  const size_t bytes[7] = {b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), b * 25 * sizeof(double), b * sizeof(int), b * sizeof(int),
-                           b * sizeof(int), b * go1mpc_body_in_stride(nh) * sizeof(double), b * sizeof(int)};
-  void* d[7] = {};
-  int rc;
-  for (int k = 0; k < nbuf; k++) {
-    const bool grow = bytes[k] > W.b[k].cap;
-    if (grow) CU(h, cudaStreamSynchronize(st));     // growing: earlier work on this stream may still use the old buffer
-    if ((rc = stage_buf2(h, W.b[k], bytes[k], &d[k]))) return rc;
-    if (grow && k == 1) W.zero_B = -1;
-  }
-  double* ctl = (double*)d[1];
-  if (W.zero_B != B) {
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  auto& ws = W->stack;
+  const size_t b = (size_t)B, sb = b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), cb = b * 25 * sizeof(double), ib = b * sizeof(int);
+  bool fresh = false;   // the control message buffer was (re)allocated
+  if ((rc = grow(h, ws.sensor, sb, st)) || (rc = grow(h, ws.ctl_msg, cb, st, &fresh)) || (rc = grow(h, ws.walkdtime, ib, st)) ||
+      (rc = grow(h, ws.cmd, ib, st)) || (rc = grow(h, ws.start, ib, st)) ||
+      (rc = grow(h, ws.body_in, b * go1mpc_body_in_stride(nh) * sizeof(double), st)) || (clock_d && (rc = grow(h, ws.plan, ib, st))))
+    return rc;
+  if (fresh) ws.zero_B = -1;
+  double* ctl = (double*)ws.ctl_msg.p;
+  int* walkdtime = (int*)ws.walkdtime.p;
+  if (ws.zero_B != B) {
     // the 14 slots of /control2rtmpc/state the stack does not upload read as zero: cleared once per batch size
-    CU(h, cudaMemsetAsync(ctl, 0, bytes[1], st));
-    W.zero_B = B;
+    CU(h, cudaMemsetAsync(ctl, 0, cb, st));
+    ws.zero_B = B;
   }
   double* state = t->state_d;
   // device inputs are read in place; host inputs go up into the stream's staging buffers
   const double* sensor = t->sensor_d;
-  if (!sensor) { CU(h, cudaMemcpyAsync(d[0], t->sensor, bytes[0], cudaMemcpyHostToDevice, st)); sensor = (const double*)d[0]; }
+  if (!sensor) { CU(h, cudaMemcpyAsync(ws.sensor.p, t->sensor, sb, cudaMemcpyHostToDevice, st)); sensor = (const double*)ws.sensor.p; }
   // with per-robot clocks some robot may plan in any call, so cmd / start go up whenever they are given
   const bool planner = clock_d || t->planner;
   const int* cmd_d = t->cmd_d;
   const int* start_d = t->start_d;
-  if (planner && t->cmd) { CU(h, cudaMemcpyAsync(d[3], t->cmd, bytes[3], cudaMemcpyHostToDevice, st)); cmd_d = (const int*)d[3]; }
-  if (planner && t->start) { CU(h, cudaMemcpyAsync(d[4], t->start, bytes[4], cudaMemcpyHostToDevice, st)); start_d = (const int*)d[4]; }
-  int* plan_d = (int*)d[6];
+  if (planner && t->cmd) { CU(h, cudaMemcpyAsync(ws.cmd.p, t->cmd, ib, cudaMemcpyHostToDevice, st)); cmd_d = (const int*)ws.cmd.p; }
+  if (planner && t->start) { CU(h, cudaMemcpyAsync(ws.start.p, t->start, ib, cudaMemcpyHostToDevice, st)); start_d = (const int*)ws.start.p; }
+  int* plan_d = (int*)ws.plan.p;
   if (clock_d)
-    CU(h, gait_stack_clocked_pre_launch(B, clock_d, plan_d, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], sensor, ctl, h->sms, st));
+    CU(h, gait_stack_clocked_pre_launch(B, clock_d, plan_d, state + GO1MPC_STACK_ROW_WALKDTIME * b, walkdtime, sensor, ctl, h->sms, st));
   else
-    CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, (int*)d[2], sensor, ctl, h->sms, st));
+    CU(h, gait_stack_pre_launch(B, t->planner ? 1 : 0, state + GO1MPC_STACK_ROW_WALKDTIME * b, walkdtime, sensor, ctl, h->sms, st));
   h->launches++;
   double* gait = state + GO1MPC_STACK_ROW_GAIT * b;
   double* rt2nrt = state + GO1MPC_STACK_ROW_RT2NRT * b;
   double* traj = state + GO1MPC_STACK_ROW_TRAJ * b;
   if (planner &&
-      (rc = nlp_node_enqueue(h, B, state + GO1MPC_STACK_ROW_NLP * b, (const int*)d[2], start_d, cmd_d, rt2nrt + 22 * b, rt2nrt + 19 * b,
+      (rc = nlp_node_enqueue(h, B, state + GO1MPC_STACK_ROW_NLP * b, walkdtime, start_d, cmd_d, rt2nrt + 22 * b, rt2nrt + 19 * b,
                              gait, clock_d ? plan_d : nullptr, st)))
     return rc;
-  if ((rc = rt_node_enqueue(h, nh, B, state + GO1MPC_STACK_ROW_RT * b, gait, nullptr, nullptr, ctl, (double*)d[5], t->body_out_d, nullptr,
-                            traj, rt2nrt, nullptr, st)))
+  if ((rc = rt_node_enqueue(h, nh, B, state + GO1MPC_STACK_ROW_RT * b, gait, nullptr, nullptr, ctl, (double*)ws.body_in.p, t->body_out_d,
+                            nullptr, traj, rt2nrt, nullptr, st)))
     return rc;
   CU(h, gait_stack_pack_launch(S, B, gait, traj, t->rows_d, h->sms, st));
   h->launches++;
@@ -1590,18 +1567,14 @@ int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r
     if (e != cudaSuccess) { cudaFree(p); return cuda_fail(h, e, "cudaMemcpy(default gait stack column)"); }
     it = h->stack_col_d.emplace(nh, p).first;
   }
-  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-  go1mpc::StackWs& W = h->stack_ws[st];
-  // {count, 3 pad, flags[B], list[B]}
-  const size_t b = (size_t)B, bytes = (4 + 2 * b) * sizeof(int);
-  if (bytes > W.b[7].cap) CU(h, cudaStreamSynchronize(st));
-  void* ws;
-  int rc;
-  if ((rc = stage_buf2(h, W.b[7], bytes, &ws))) return rc;
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  const size_t b = (size_t)B;
+  if ((rc = grow(h, W->reset_list, (4 + 2 * b) * sizeof(int), st))) return rc;
   StackResetParams P;
   P.B = B; P.rows = rows; P.out_stride = go1mpc_body_out_stride(nh);
-  P.count = (int*)ws; P.reset = r->reset_d ? r->reset_d : P.count + 4; P.list = P.count + 4 + B;
+  P.count = (int*)W->reset_list.p; P.reset = r->reset_d ? r->reset_d : P.count + 4; P.list = P.count + 4 + B;
   P.clock = r->clock_d; P.state = r->state_d; P.column = it->second; P.body_out = r->body_out_d; P.servo = r->servo_state_d;
   memcpy(P.q0, r->servo_q0, sizeof P.q0);
   if (r->reset) CU(h, cudaMemcpyAsync((void*)P.reset, r->reset, b * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -1645,15 +1618,10 @@ int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
         return fail(h, GO1MPC_E_INVALID, "farm_copy_async: a destination block overlaps a source block");
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  if (h->stack_ws.size() >= 256 && h->stack_ws.find(st) == h->stack_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-  go1mpc::StackWs& W = h->stack_ws[st];
-  // {count, 3 pad, destination list[dst.B], source list[dst.B]}
-  const size_t bytes = (4 + 2 * (size_t)D.B) * sizeof(int);
-  if (bytes > W.b[8].cap) CU(h, cudaStreamSynchronize(st));
-  void* ws;
-  int rc;
-  if ((rc = stage_buf2(h, W.b[8], bytes, &ws))) return rc;
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  if ((rc = grow(h, W->copy_list, (4 + 2 * (size_t)D.B) * sizeof(int), st))) return rc;
   FarmCopyParams P;
   P.dst_B = D.B; P.src_B = S.B;
   P.rows = rows;
@@ -1665,7 +1633,7 @@ int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
   P.src_state = S.state_d; P.src_servo = S.servo_state_d; P.src_force = S.force_state_d;
   P.dst_body = reinterpret_cast<double2*>(D.body_out_d); P.src_body = reinterpret_cast<const double2*>(S.body_out_d);
   P.dst_clock = D.clock_d; P.src_clock = S.clock_d;
-  P.count = (int*)ws; P.dlist = P.count + 4; P.slist = P.count + 4 + D.B;
+  P.count = (int*)W->copy_list.p; P.dlist = P.count + 4; P.slist = P.count + 4 + D.B;
   CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
   CU(h, farm_copy_launch(P, h->sms, st));
   h->launches += 2;
@@ -1686,20 +1654,9 @@ int go1mpc_servo_stack_tick_async(go1mpc_t* h, int B, const Go1ServoStackTick* t
   if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, "servo_stack_tick_async: gait_mode 101, 102 or 103");
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  const size_t b = (size_t)B;
-  ServoStackKParams P;
-  P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
-  P.half_hip_width = h->cfg.step.half_hip_width; P.y_offset = t->y_offset;
-  double k6[6];
-  go1mpc_lpf_coefficients(1000.0, 3.0, k6);                     // the servo loop's 3 Hz filters at 1 kHz
-  P.coef = LpfCoef{k6[0], k6[1], k6[2], k6[3], k6[4], k6[5]};
-  P.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
-  P.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
-  P.state = t->servo_state_d; P.q_out = t->q_d;
-  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d; P.ch = nullptr;
-  CU(h, servo_stack_launch(P, st));
+  CU(h, servo_stack_launch(servo_stack_params(h, B, t, nullptr), st));
   h->launches++;
-  if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, b * 12 * t->K * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, (size_t)B * 12 * t->K * sizeof(double), cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
 }
 
@@ -1726,35 +1683,21 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
   }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  if (h->servo_ws.size() >= 256 && h->servo_ws.find(st) == h->servo_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-  go1mpc::ServoWs& W = h->servo_ws[st];
-  const size_t b = (size_t)B;
-  // sized for K = GO1MPC_SERVO_TICKS_MAX, so that K changes do not reallocate; a growing buffer may still be read by the
-  // stream's previous call
-  const size_t chb = b * SERVO_TICKS_MAX * SERVO_LPF_CHANNELS * sizeof(double), rb = b * sizeof(int);
-  if (chb > W.ch.cap || (t->reset && rb > W.reset.cap)) CU(h, cudaStreamSynchronize(st));
-  void *ch, *rst = nullptr;
-  int rc;
-  if ((rc = stage_buf2(h, W.ch, chb, &ch))) return rc;
-  if (t->reset && (rc = stage_buf2(h, W.reset, rb, &rst))) return rc;
-  ServoStackKParams S;
-  S.B = B; S.K = t->K; S.gait_mode = t->gait_mode;
-  S.half_hip_width = h->cfg.step.half_hip_width; S.y_offset = t->y_offset;
-  double k6[6];
-  go1mpc_lpf_coefficients(1000.0, 3.0, k6);
-  S.coef = LpfCoef{k6[0], k6[1], k6[2], k6[3], k6[4], k6[5]};
-  S.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
-  S.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
-  S.state = t->servo_state_d; S.q_out = t->q_d;
-  S.jac = t->jac_d; S.foot_des = t->foot_des_d; S.iters = t->iters_d; S.ch = (double*)ch;
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  const size_t b = (size_t)B, rb = b * sizeof(int);
+  // sized for K = GO1MPC_SERVO_TICKS_MAX, so that K changes do not reallocate
+  if ((rc = grow(h, W->servo_ch, b * SERVO_TICKS_MAX * SERVO_LPF_CHANNELS * sizeof(double), st)) ||
+      (t->reset && (rc = grow(h, W->servo_reset, rb, st))))
+    return rc;
+  void* rst = t->reset ? W->servo_reset.p : nullptr;
+  const ServoStackKParams S = servo_stack_params(h, B, t, (double*)W->servo_ch.p);
   ServoTorqueKParams P;
-  P.g.B = B; P.g.cap = h->cfg.qp_iter_cap_scale * (12 + 12 + 24) + 50; P.g.warp_doubles = 0;
-  P.g.qp_alpha = 10000; P.g.qp_beta = 1000; P.g.qp_gama = 10; P.g.fz_max = 160; P.g.mu = 0.25;   // as go1mpc_grf_force_opt_batch
-  P.g.in = nullptr; P.g.out = nullptr; P.g.diag = nullptr;
+  P.g = grf_params(h, B, nullptr, nullptr, nullptr);
   P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
   P.half_hip_width = S.half_hip_width; P.y_offset = t->y_offset; P.y_coefficient = t->y_coefficient;
-  P.swing_kp = 1; P.swing_kd = 0.01;                                                               // as go1mpc_grf_joint_torques_batch
+  P.swing_kp = kSwingKp; P.swing_kd = kSwingKd;
   P.gait = S.gait; P.traj = S.traj; P.homing = t->servo_state_d + SERVO_ROW_HOMING * b; P.ch = S.ch; P.q = t->q_d;
   P.meas = t->meas_d; P.reset = t->reset_d ? t->reset_d : (const int*)rst; P.force = t->force_state_d; P.tau = t->tau_d;
   P.grf = t->grf_d; P.grf_diag = t->grf_diag_d;
@@ -1780,28 +1723,21 @@ int go1mpc_body_mpc_step_batch_host_async(go1mpc_t* h, int nh, int B, const doub
   BodyModel* M;
   int rc = get_body_model(h, nh, &M);
   if (rc) return rc;
-  const int is = go1mpc_body_in_stride(nh), os = go1mpc_body_out_stride(nh);
-  const size_t ib = (size_t)B * is * sizeof(double), ob = (size_t)B * os * sizeof(double);
-  const size_t db = (size_t)B * go1mpc_body_diag_stride(nh) * sizeof(int);
-  go1mpc::Lane& L = h->lanes[h->lane_next++ % go1mpc::kLanes];
-  void *din, *dout, *ddiag = nullptr;
-  if ((rc = stage_buf2(h, L.stage[0], ib, &din))) return rc;
-  if ((rc = stage_buf2(h, L.stage[1], ob, &dout))) return rc;
-  if (diag && (rc = stage_buf2(h, L.stage[2], db, &ddiag))) return rc;
+  const int is = go1mpc_body_in_stride(nh);
+  const size_t b = (size_t)B, ob = b * go1mpc_body_out_stride(nh) * sizeof(double);
   // the previous outputs are only read by gated ticks (the reference returns its stale members):
   // upload them only when the batch has one
   bool gated = false;
-  for (int b = 0; b < B && !gated; b++) {
-    const int t = (int)in[(size_t)b * is + 27];
+  for (int k = 0; k < B && !gated; k++) {
+    const int t = (int)in[(size_t)k * is + 27];
     gated = (t < M->gate) || !(t - M->gate < M->nsum_mpc - nh);
   }
-  CU(h, cudaMemcpyAsync(din, in, ib, cudaMemcpyHostToDevice, L.stream));
-  if (gated) CU(h, cudaMemcpyAsync(dout, out, ob, cudaMemcpyHostToDevice, L.stream));
-  rc = go1mpc_body_mpc_step_batch(h, nh, B, (const double*)din, (double*)dout, (int*)ddiag, L.stream);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(out, dout, ob, cudaMemcpyDeviceToHost, L.stream));
-  if (diag) CU(h, cudaMemcpyAsync(diag, ddiag, db, cudaMemcpyDeviceToHost, L.stream));
-  return GO1MPC_OK;
+  go1mpc::Lane& L = h->lanes[h->lane_next++ % go1mpc::kLanes];
+  Staging S(h, L.body, L.stream);
+  const double* din = S.up(in, b * is * sizeof(double));
+  double* dout = gated ? S.inout(out, ob) : S.out(out, ob);
+  int* ddiag = S.out(diag, b * go1mpc_body_diag_stride(nh) * sizeof(int));
+  return S.run(false, [&] { return go1mpc_body_mpc_step_batch(h, nh, B, din, dout, ddiag, S.st); });
 }
 
 // Same tick with tx and the previous output record resident on the device (body_resident.cu): per instance
@@ -1814,38 +1750,32 @@ int go1mpc_body_mpc_step_batch_resident_host_async(go1mpc_t* h, int nh, int B, c
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!tx_d || !out_d || !tick_in || !tick_out) return fail(h, GO1MPC_E_INVALID, "body_mpc_step_batch_resident_host_async: bad argument");
   if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "body_mpc_step_batch_resident_host_async: 3 <= nh <= 40");
-  CU(h, cudaSetDevice(h->device));
   const int is = go1mpc_body_in_stride(nh), os = go1mpc_body_out_stride(nh), ts = go1mpc_body_tick_in_stride(nh);
-  const size_t ib = (size_t)B * is * sizeof(double), tb = (size_t)B * ts * sizeof(double);
-  const size_t tob = (size_t)B * GO1MPC_BODY_TICK_OUT * sizeof(double);
-  const size_t db = (size_t)B * go1mpc_body_diag_stride(nh) * sizeof(int);
+  const size_t b = (size_t)B;
   go1mpc::Lane& L = h->lanes[h->lane_next++ % go1mpc::kLanes];
-  void *drec, *dtick, *dto, *ddiag = nullptr;
-  int rc;
-  if ((rc = stage_buf2(h, L.stage[0], ib, &drec))) return rc;
-  if ((rc = stage_buf2(h, L.stage[8], tb, &dtick))) return rc;
-  if ((rc = stage_buf2(h, L.stage[9], tob, &dto))) return rc;
-  if (diag && (rc = stage_buf2(h, L.stage[2], db, &ddiag))) return rc;
-  CU(h, cudaMemcpyAsync(dtick, tick_in, tb, cudaMemcpyHostToDevice, L.stream));
+  Staging S(h, L.resident, L.stream);
+  double* drec = S.out_always((double*)nullptr, b * is * sizeof(double), 0);   // the expand kernel writes the records
+  const double* dtick = S.up(tick_in, b * ts * sizeof(double));
+  double* dto = S.out(tick_out, b * GO1MPC_BODY_TICK_OUT * sizeof(double));
+  int* ddiag = S.out(diag, b * go1mpc_body_diag_stride(nh) * sizeof(int));
+  if (S.rc) return S.rc;
   // consecutive ticks of the same instances sit on different lanes: order them through the resident records
   {
     auto it = h->last_writer.find((const void*)out_d);
     if (it != h->last_writer.end()) CU(h, cudaStreamWaitEvent(L.stream, it->second, 0));
   }
-  CU(h, body_record_expand_launch(B, nh, is, ts, os, tx_d, (const double*)dtick, out_d, (double*)drec, h->sms, L.stream));
+  CU(h, body_record_expand_launch(B, nh, is, ts, os, tx_d, dtick, out_d, drec, h->sms, L.stream));
   h->launches++;
-  rc = go1mpc_body_mpc_step_batch(h, nh, B, (const double*)drec, out_d, (int*)ddiag, L.stream);
+  int rc = go1mpc_body_mpc_step_batch(h, nh, B, drec, out_d, ddiag, L.stream);
   if (rc) return rc;
-  CU(h, body_record_pack_launch(B, nh, os, out_d, (double*)dto, h->sms, L.stream));
+  CU(h, body_record_pack_launch(B, nh, os, out_d, dto, h->sms, L.stream));
   h->launches++;
   {
     cudaEvent_t& ev = h->last_writer[(const void*)out_d];
     if (!ev) CU(h, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
     CU(h, cudaEventRecord(ev, L.stream));
   }
-  CU(h, cudaMemcpyAsync(tick_out, dto, tob, cudaMemcpyDeviceToHost, L.stream));
-  if (diag) CU(h, cudaMemcpyAsync(diag, ddiag, db, cudaMemcpyDeviceToHost, L.stream));
-  return GO1MPC_OK;
+  return S.finish(false);
 }
 
 int go1mpc_step_timing_step_batch_host_async(go1mpc_t* h, int n_sqp, int B, const int* tick, const double* state_d,
@@ -1856,23 +1786,19 @@ int go1mpc_step_timing_step_batch_host_async(go1mpc_t* h, int n_sqp, int B, cons
   if (!tick || !state_d || !state_out_d || !in || !out) return fail(h, GO1MPC_E_INVALID, "step_timing_step_batch_host_async: bad argument");
   CU(h, cudaSetDevice(h->device));
   const size_t b = (size_t)B;
-  const size_t tb = b * sizeof(int), ib = b * STEP_IN_DOUBLES * sizeof(double);
-  const size_t ob = b * STEP_OUT_DOUBLES * sizeof(double), db = b * STEP_DIAG_INTS * sizeof(int);
   go1mpc::Lane& L = h->lanes[h->lane_next++ % go1mpc::kLanes];
-  void *dt_, *di, *do_, *dd = nullptr;
-  int rc;
-  if ((rc = stage_buf2(h, L.stage[3], tb, &dt_))) return rc;
-  if ((rc = stage_buf2(h, L.stage[4], ib, &di))) return rc;
-  if ((rc = stage_buf2(h, L.stage[5], ob, &do_))) return rc;
-  if (diag && (rc = stage_buf2(h, L.stage[6], db, &dd))) return rc;
   // consecutive ticks of the same planners sit on different lanes: order them through the state buffers
   for (const void* key : {(const void*)state_d, (const void*)state_out_d}) {
     auto it = h->last_writer.find(key);
     if (it != h->last_writer.end()) CU(h, cudaStreamWaitEvent(L.stream, it->second, 0));
   }
-  CU(h, cudaMemcpyAsync(dt_, tick, tb, cudaMemcpyHostToDevice, L.stream));
-  CU(h, cudaMemcpyAsync(di, in, ib, cudaMemcpyHostToDevice, L.stream));
-  rc = go1mpc_step_timing_step_batch(h, n_sqp, B, (const int*)dt_, state_d, state_out_d, (const double*)di, (double*)do_, (int*)dd, L.stream);
+  Staging S(h, L.step, L.stream);
+  const int* dt_ = S.up(tick, b * sizeof(int));
+  const double* di = S.up(in, b * STEP_IN_DOUBLES * sizeof(double));
+  double* do_ = S.out(out, b * STEP_OUT_DOUBLES * sizeof(double));
+  int* dd = S.out(diag, b * STEP_DIAG_INTS * sizeof(int));
+  if (S.rc) return S.rc;
+  int rc = go1mpc_step_timing_step_batch(h, n_sqp, B, dt_, state_d, state_out_d, di, do_, dd, L.stream);
   if (rc) return rc;
   // the buffer read and the buffer written: a later call on another lane that WRITES the state this call read must come after
   // it too (write-after-read when state_out_d != state_d)
@@ -1882,9 +1808,7 @@ int go1mpc_step_timing_step_batch_host_async(go1mpc_t* h, int n_sqp, int B, cons
     CU(h, cudaEventRecord(ev, L.stream));
     if (state_out_d == state_d) break;
   }
-  CU(h, cudaMemcpyAsync(out, do_, ob, cudaMemcpyDeviceToHost, L.stream));
-  if (diag) CU(h, cudaMemcpyAsync(diag, dd, db, cudaMemcpyDeviceToHost, L.stream));
-  return GO1MPC_OK;
+  return S.finish(false);
 }
 
 // The pipelined entries order calls that share a device-resident buffer through an event kept per buffer address; a caller that
@@ -1977,43 +1901,21 @@ int go1mpc_fused_tick_batch(go1mpc_t* h, int B, const Go1FusedTick* t, void* str
                                         GRF_OUT_DOUBLES, t->tau_d, st);
 }
 
-namespace {
-// shared host staging for the two leg entries: ins[k] (bytes) up, outs[k] down
-int leg_host(go1mpc* h, int B, bool ik, const double* a3, const double* b3, const int* leg, const double* bp, const double* br,
-             double* o3, double* jac, int* iters) {
-  const size_t b = (size_t)B, v3 = b * 3 * sizeof(double), v9 = b * 9 * sizeof(double), vi = b * sizeof(int);
-  void *da, *db = nullptr, *dl, *dbp = nullptr, *dbr = nullptr, *do3, *dj = nullptr, *dit = nullptr;
-  int rc;
-  if ((rc = stage_buf(h, 0, v3, &da))) return rc;
-  if (ik && (rc = stage_buf(h, 1, v3, &db))) return rc;
-  if ((rc = stage_buf(h, 2, vi, &dl))) return rc;
-  if (bp) { if ((rc = stage_buf(h, 3, v3, &dbp))) return rc; if ((rc = stage_buf(h, 4, v3, &dbr))) return rc; }
-  if ((rc = stage_buf(h, 5, v3, &do3))) return rc;
-  if (jac && (rc = stage_buf(h, 6, v9, &dj))) return rc;
-  if (iters && (rc = stage_buf(h, 7, vi, &dit))) return rc;
-  cudaStream_t st = h->stream;
-  CU(h, cudaMemcpyAsync(da, a3, v3, cudaMemcpyHostToDevice, st));
-  if (ik) CU(h, cudaMemcpyAsync(db, b3, v3, cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(dl, leg, vi, cudaMemcpyHostToDevice, st));
-  if (bp) { CU(h, cudaMemcpyAsync(dbp, bp, v3, cudaMemcpyHostToDevice, st)); CU(h, cudaMemcpyAsync(dbr, br, v3, cudaMemcpyHostToDevice, st)); }
-  if (ik) rc = go1mpc_leg_ik_batch(h, B, (double*)da, (double*)db, (int*)dl, (double*)dbp, (double*)dbr, (double*)do3, (double*)dj, (int*)dit, st);
-  else rc = go1mpc_leg_fk_batch(h, B, (double*)da, (int*)dl, (double*)dbp, (double*)dbr, (double*)do3, (double*)dj, st);
-  if (rc) return rc;
-  CU(h, cudaMemcpyAsync(o3, do3, v3, cudaMemcpyDeviceToHost, st));
-  if (jac) CU(h, cudaMemcpyAsync(jac, dj, v9, cudaMemcpyDeviceToHost, st));
-  if (iters) CU(h, cudaMemcpyAsync(iters, dit, vi, cudaMemcpyDeviceToHost, st));
-  CU(h, cudaStreamSynchronize(st));
-  return GO1MPC_OK;
-}
-}  // namespace
 int go1mpc_leg_fk_batch_host(go1mpc_t* h, int B, const double* q, const int* leg, const double* body_p, const double* body_r,
                              double* pos, double* jac) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!q || !leg || !pos || ((body_p == nullptr) != (body_r == nullptr))) return fail(h, GO1MPC_E_INVALID, "leg_fk_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  return leg_host(h, B, false, q, nullptr, leg, body_p, body_r, pos, jac, nullptr);
+  const size_t v3 = (size_t)B * 3 * sizeof(double);
+  Staging S(h, h->stage, h->stream);
+  const double* dq = S.up(q, v3);
+  const int* dl = S.up(leg, (size_t)B * sizeof(int));
+  const double* dbp = S.up(body_p, v3);
+  const double* dbr = S.up(body_r, v3);
+  double* dpos = S.out(pos, v3);
+  double* dj = S.out(jac, 3 * v3);
+  return S.run(true, [&] { return go1mpc_leg_fk_batch(h, B, dq, dl, dbp, dbr, dpos, dj, S.st); });
 }
 int go1mpc_leg_ik_batch_host(go1mpc_t* h, int B, const double* pdes, const double* qini, const int* leg, const double* body_p,
                              const double* body_r, double* q, double* jac, int* iters) {
@@ -2021,8 +1923,17 @@ int go1mpc_leg_ik_batch_host(go1mpc_t* h, int B, const double* pdes, const doubl
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!pdes || !qini || !leg || !q || ((body_p == nullptr) != (body_r == nullptr))) return fail(h, GO1MPC_E_INVALID, "leg_ik_batch_host: bad argument");
-  CU(h, cudaSetDevice(h->device));
-  return leg_host(h, B, true, pdes, qini, leg, body_p, body_r, q, jac, iters);
+  const size_t v3 = (size_t)B * 3 * sizeof(double), vi = (size_t)B * sizeof(int);
+  Staging S(h, h->stage, h->stream);
+  const double* dpdes = S.up(pdes, v3);
+  const double* dqini = S.up(qini, v3);
+  const int* dl = S.up(leg, vi);
+  const double* dbp = S.up(body_p, v3);
+  const double* dbr = S.up(body_r, v3);
+  double* dq = S.out(q, v3);
+  double* dj = S.out(jac, 3 * v3);
+  int* dit = S.out(iters, vi);
+  return S.run(true, [&] { return go1mpc_leg_ik_batch(h, B, dpdes, dqini, dl, dbp, dbr, dq, dj, dit, S.st); });
 }
 
 // ------------------------------------------------------------------ control tick with host inputs and compact results
@@ -2051,48 +1962,54 @@ int go1mpc_control_tick_host_async(go1mpc_t* h, int B, const Go1ControlTick* t, 
   if (nh < 3 || nh > GO1MPC_BODY_NH_MAX) return fail(h, GO1MPC_E_UNSUPPORTED, "control_tick_host_async: 3 <= nh <= 40");
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-  if (h->tick_ws.size() >= 256 && h->tick_ws.find(st) == h->tick_ws.end())
-    return fail(h, GO1MPC_E_UNSUPPORTED, "more than 256 distinct streams used with one handle");
-  go1mpc::TickWs& W = h->tick_ws[st];
+  StreamWs* W;
+  int rc = stream_ws(h, st, &W);
+  if (rc) return rc;
+  auto& ws = W->control;
   const size_t b = (size_t)B;
   const int is = go1mpc_body_in_stride(nh), os = go1mpc_body_out_stride(nh), ts = go1mpc_body_tick_in_stride(nh), ds = go1mpc_body_diag_stride(nh);
-  const size_t bytes[7] = {b * sizeof(int), b * STEP_IN_DOUBLES * sizeof(double), b * ts * sizeof(double), b * is * sizeof(double),
-                           b * STEP_OUT_DOUBLES * sizeof(double), b * STEP_DIAG_INTS * sizeof(int), b * ds * sizeof(int)};
-  void* d[7];
-  int rc;
+  const size_t tb = b * sizeof(int), tib = b * ts * sizeof(double), ob = b * STEP_OUT_DOUBLES * sizeof(double);
+  const size_t sdb = b * STEP_DIAG_INTS * sizeof(int), bdb = b * ds * sizeof(int);
   const int in_rows = (t->step_in_rows > 0 && t->step_in_rows < STEP_IN_DOUBLES) ? t->step_in_rows : STEP_IN_DOUBLES;
   if (in_rows < STEP_IN_DOUBLES && (in_rows < 10 || h->cfg.step.ext_height))
     return fail(h, GO1MPC_E_INVALID, "control_tick_host_async: step_in_rows must cover the 10 sensor rows, and all 20 with cfg.step.ext_height");
-  for (int k = 0; k < 7; k++) {
-    const bool grow = bytes[k] > W.b[k].cap;
-    if (grow) CU(h, cudaStreamSynchronize(st));     // growing: earlier work on this stream may still use the old buffer
-    if ((rc = stage_buf2(h, W.b[k], bytes[k], &d[k]))) return rc;
-    if (grow && k == 1) W.zero_B = -1;
-  }
+  bool fresh = false;   // the planner input buffer was (re)allocated
+  if ((rc = grow(h, ws.tick, tb, st)) || (rc = grow(h, ws.step_in, b * STEP_IN_DOUBLES * sizeof(double), st, &fresh)) ||
+      (rc = grow(h, ws.body_tick_in, tib, st)) || (rc = grow(h, ws.body_in, b * is * sizeof(double), st)) ||
+      (rc = grow(h, ws.out38, ob, st)) || (rc = grow(h, ws.step_diag, sdb, st)) || (rc = grow(h, ws.body_diag, bdb, st)))
+    return rc;
+  if (fresh) ws.zero_B = -1;
+  int* tick = (int*)ws.tick.p;
+  double* step_in = (double*)ws.step_in.p;
+  double* body_tick_in = (double*)ws.body_tick_in.p;
+  double* body_in = (double*)ws.body_in.p;
+  double* out38 = (double*)ws.out38.p;
+  int* step_diag = (int*)ws.step_diag.p;
+  int* body_diag = (int*)ws.body_diag.p;
   if (in_rows < STEP_IN_DOUBLES) {
     // rows a partial upload does not carry read as zero (flat ground, no external heights): cleared once per batch size
-    if (W.zero_B != B) {
-      CU(h, cudaMemsetAsync((double*)d[1] + b * in_rows, 0, b * (STEP_IN_DOUBLES - in_rows) * sizeof(double), st));
-      W.zero_B = B;
+    if (ws.zero_B != B) {
+      CU(h, cudaMemsetAsync(step_in + b * in_rows, 0, b * (STEP_IN_DOUBLES - in_rows) * sizeof(double), st));
+      ws.zero_B = B;
     }
   } else {
-    W.zero_B = -1;
+    ws.zero_B = -1;
   }
-  CU(h, cudaMemcpyAsync(d[0], t->tick, bytes[0], cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(d[1], t->step_in, b * in_rows * sizeof(double), cudaMemcpyHostToDevice, st));
-  CU(h, cudaMemcpyAsync(d[2], t->body_tick_in, bytes[2], cudaMemcpyHostToDevice, st));
+  CU(h, cudaMemcpyAsync(tick, t->tick, tb, cudaMemcpyHostToDevice, st));
+  CU(h, cudaMemcpyAsync(step_in, t->step_in, b * in_rows * sizeof(double), cudaMemcpyHostToDevice, st));
+  CU(h, cudaMemcpyAsync(body_tick_in, t->body_tick_in, tib, cudaMemcpyHostToDevice, st));
   // planner tick: out of place from the pristine state when the caller gives one (replays of the same tick), else in place
   const double* src = t->step_state_src_d ? t->step_state_src_d : t->step_state_d;
-  if ((rc = go1mpc_step_timing_step_batch(h, t->n_sqp, B, (const int*)d[0], src, t->step_state_d, (const double*)d[1], (double*)d[4], (int*)d[5], st))) return rc;
+  if ((rc = go1mpc_step_timing_step_batch(h, t->n_sqp, B, tick, src, t->step_state_d, step_in, out38, step_diag, st))) return rc;
   // body tick on the resident records
-  CU(h, body_record_expand_launch(B, nh, is, ts, os, t->tx_d, (const double*)d[2], t->body_out_d, (double*)d[3], h->sms, st));
+  CU(h, body_record_expand_launch(B, nh, is, ts, os, t->tx_d, body_tick_in, t->body_out_d, body_in, h->sms, st));
   h->launches++;
-  if ((rc = go1mpc_body_mpc_step_batch(h, nh, B, (const double*)d[3], t->body_out_d, (int*)d[6], st))) return rc;
-  CU(h, compact_pack_launch(B, nh, os, ds, (const double*)d[4], (const int*)d[5], t->body_out_d, (const int*)d[6], t->compact_d, h->sms, st));
+  if ((rc = go1mpc_body_mpc_step_batch(h, nh, B, body_in, t->body_out_d, body_diag, st))) return rc;
+  CU(h, compact_pack_launch(B, nh, os, ds, out38, step_diag, t->body_out_d, body_diag, t->compact_d, h->sms, st));
   h->launches++;
-  if (t->out38) CU(h, cudaMemcpyAsync(t->out38, d[4], bytes[4], cudaMemcpyDeviceToHost, st));
-  if (t->step_diag) CU(h, cudaMemcpyAsync(t->step_diag, d[5], bytes[5], cudaMemcpyDeviceToHost, st));
-  if (t->body_diag) CU(h, cudaMemcpyAsync(t->body_diag, d[6], bytes[6], cudaMemcpyDeviceToHost, st));
+  if (t->out38) CU(h, cudaMemcpyAsync(t->out38, out38, ob, cudaMemcpyDeviceToHost, st));
+  if (t->step_diag) CU(h, cudaMemcpyAsync(t->step_diag, step_diag, sdb, cudaMemcpyDeviceToHost, st));
+  if (t->body_diag) CU(h, cudaMemcpyAsync(t->body_diag, body_diag, bdb, cudaMemcpyDeviceToHost, st));
   if (t->compact) CU(h, cudaMemcpyAsync(t->compact, t->compact_d, b * GO1MPC_COMPACT_DOUBLES * sizeof(double), cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
 }
