@@ -772,7 +772,11 @@ int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r
  * index_d[i] = 0 for the robots that fork and -1 elsewhere.  A bank column holding a freshly reset robot (snapshot right after
  * go1mpc_gait_stack_reset_async, force column zero) restarts robots as that reset plus the torque tick's reset flag do, except
  * that the homing rows come from the bank column.
- * clock_d, servo_state_d and force_state_d are each given on both sides or on neither; both sides share nh.
+ * clock_d, servo_state_d, force_state_d and health_d are each given on both sides or on neither; both sides share nh.
+ * health_d (the farm's health counters, see go1mpc_gait_stack_tick_clocked_health_async) travels with the clock: a copied
+ * column takes the source's counters, so a snapshot and restore continues counting bit-identically.  A restore given no health
+ * block leaves the destination's old counters in place; they restart anyway when the restored clock is 0 (the next health-enabled
+ * clocked tick zeroes them).
  * Two kernel launches of a fixed shape after a memset of a device counter: the first lists the copied destinations (one
  * atomic per warp) and copies their clocks, the second copies the listed columns, reading the count on the device.  The index
  * never changes what is enqueued, and the work grows with the number of columns copied.  A workspace of 8 B per destination
@@ -780,7 +784,7 @@ int go1mpc_gait_stack_reset_async(go1mpc_t *h, int B, const Go1GaitStackReset *r
  * restore -> go1mpc_gait_stack_tick_clocked_async -> go1mpc_servo_torque_tick_async can be captured once with
  * go1mpc_graph_capture_* and replayed, the caller (or a device kernel) rewriting index_d between replays.  dst.B = 0 is a no-op.
  * Errors (nothing is enqueued): GO1MPC_E_INVALID for a NULL c, state_d, body_out_d or index_d, an optional block given on one
- * side only, body_out_d not 16-byte aligned on either side, a negative B, src.B < 1 while dst.B > 0, or any destination block
+ * side only, body_out_d not 16-byte or health_d not 4-byte aligned on either side, a negative B, src.B < 1 while dst.B > 0, or any destination block
  * whose address range overlaps any source block; GO1MPC_E_UNSUPPORTED for nh outside 3..40.  index_d is device memory and is
  * not checked on the host: an out-of-range entry never causes an out-of-bounds access.
  * ------------------------------------------------------------------------ */
@@ -791,6 +795,7 @@ typedef struct {
   int *clock_d;             /* [B] or NULL */
   double *servo_state_d;    /* [GO1MPC_SERVO_STATE_ROWS][B] or NULL */
   double *force_state_d;    /* [GO1MPC_SERVO_FORCE_ROWS][B] or NULL */
+  int *health_d;            /* [GO1MPC_HEALTH_ROWS][B] ints, 4-byte aligned, or NULL */
 } Go1FarmColumns;
 typedef struct {
   int nh;                   /* 3..40, shared by both sides */
@@ -912,6 +917,59 @@ typedef struct {
   const int *reset_d;           /* device [B] or NULL, same flags as `reset`; at most one of reset / reset_d */
 } Go1ServoTorqueTick;
 int go1mpc_servo_torque_tick_async(go1mpc_t *h, int B, const Go1ServoTorqueTick *t, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * Farm health counters: per robot, how its solvers ended since the robot's reset, counted on the device by the farm's own kernels,
+ * so that a Monte-Carlo or RL study can tell which robots drove a QP infeasible and how often, and restart robots whose controller
+ * failed (go1mpc_farm_copy_async with an index computed on the device from the EVENTS row) with no host round trip.
+ *
+ * health_d: caller-owned device ints [GO1MPC_HEALTH_ROWS][B], SoA like every other farm block, zero-initialised; row r of robot b at
+ * health_d[r * B + b].  Each row counts:
+ *   PLAN_OK / _INFEASIBLE / _FAILED   planner SQP QPs (3 per planner tick) with status GO1MPC_QP_OK, GO1MPC_QP_INFEASIBLE, any other
+ *                                     status >= 1 (NOT_PD, ITER_CAP, NAN, EQ_DEPENDENT); iterations that ran no solve count nowhere
+ *   BODY_OK / _INFEASIBLE / _FAILED   the same split for body-MPC solves, one per clocked tick; a gated tick (status -1) counts nowhere
+ *   GRF_OK / GRF_FAILED               servo ticks whose force QP returned GO1MPC_QP_OK / any other status (x = 0 is always feasible
+ *                                     for that QP, so there is no infeasible row)
+ *   GRF_FALLBACK                      servo ticks whose QP solution held a NaN, so the torque map used F_leg_guess (diag word 6 = 0)
+ *   IK_CAP                            leg-ticks whose Inverse_kinematics_g applied all 15 updates (its stop test never passed)
+ *   NONFINITE                         clocked ticks whose rows_d row of the robot holds a non-finite value, plus servo ticks whose
+ *                                     12 q or 12 tau of the robot hold one
+ *   EVENTS                            bit r (r = 0..10) set when row r grew during the current period: the clocked tick overwrites
+ *                                     this row, the torque tick ORs into it
+ * Counters restart with the robot's episode: a robot whose clock is 0 at the start of a health-enabled clocked tick starts that
+ * call from zero (a fresh batch, a robot flagged by go1mpc_gait_stack_reset_async, a robot restored from a freshly reset bank
+ * column).  clock_d counts the periods since that reset.  int32 is enough: IK_CAP, the fastest row, grows by at most 40 per period,
+ * which takes more than 600 days of 100 Hz periods to overflow.
+ *
+ * go1mpc_gait_stack_tick_clocked_health_async: go1mpc_gait_stack_tick_clocked_async plus the counting.  The planner writes its step
+ *   diag and the body MPC its diag records into a per-stream workspace (allocated with the other workspaces on the first call with
+ *   a given (stream, B, nh)), and one more kernel after the pack updates health_d: planner rows for the robots that planned in this
+ *   call, body rows for every robot, NONFINITE, the clock-0 restart and EVENTS.
+ * go1mpc_servo_torque_tick_health_async: go1mpc_servo_torque_tick_async plus the counting of IK_CAP (in the servo stack kernel),
+ *   the force-QP rows, GRF_FALLBACK and NONFINITE (in the force-stage kernel), tick by tick over the K ticks.  Same two launches.
+ * With health, every output of both calls is bit-identical to the same call without it; the entries without health enqueue the
+ * same work as before.  A warmed-up period restore -> clocked health tick -> torque health tick captures and replays as the plain one.
+ * Errors (nothing is enqueued): those of the entry without health, and GO1MPC_E_INVALID for a NULL health_d, health_d not 4-byte
+ * aligned, or a health_d range that overlaps a block the call reads or writes -- clocked tick: state_d, body_out_d, rows_d,
+ * clock_d, sensor_d, cmd_d, start_d; torque tick: stack_state_d (its rows before GO1MPC_STACK_ROW_RT), servo_state_d,
+ * force_state_d, meas_d, q_d, tau_d, reset_d, grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.
+ * Not covered: the position-mode farm entries go1mpc_gait_stack_tick_host_async and go1mpc_servo_stack_tick_async.
+ * ------------------------------------------------------------------------ */
+#define GO1MPC_HEALTH_ROWS 12
+#define GO1MPC_HEALTH_PLAN_OK 0
+#define GO1MPC_HEALTH_PLAN_INFEASIBLE 1
+#define GO1MPC_HEALTH_PLAN_FAILED 2
+#define GO1MPC_HEALTH_BODY_OK 3
+#define GO1MPC_HEALTH_BODY_INFEASIBLE 4
+#define GO1MPC_HEALTH_BODY_FAILED 5
+#define GO1MPC_HEALTH_GRF_OK 6
+#define GO1MPC_HEALTH_GRF_FAILED 7
+#define GO1MPC_HEALTH_GRF_FALLBACK 8
+#define GO1MPC_HEALTH_IK_CAP 9
+#define GO1MPC_HEALTH_NONFINITE 10
+#define GO1MPC_HEALTH_EVENTS 11
+int go1mpc_gait_stack_tick_clocked_health_async(go1mpc_t *h, int B, const Go1GaitStackClockedTick *t, int *health_d, void *stream);
+int go1mpc_servo_torque_tick_health_async(go1mpc_t *h, int B, const Go1ServoTorqueTick *t, int *health_d, void *stream);
 
 /* Per-kernel timing of the three-launch body tick (measurement aid for bench.py's roofline): while enabled, each
  * go1mpc_body_mpc_step_batch call on that path records CUDA events around its setup / solve / merge launches;

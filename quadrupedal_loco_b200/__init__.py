@@ -13,6 +13,8 @@ from .binding import (  # noqa: F401
     STACK_ROW_GAIT, STACK_ROW_RT2NRT, STACK_ROW_WALKDTIME, STACK_ROW_TRAJ, STACK_ROW_RT,
     ServoStackTick, SERVO_TICKS_MAX, SERVO_STATE_ROWS, SERVO_ROW_Q, SERVO_ROW_HOMING, SERVO_ROW_LPF, SERVO_LPF_SLOTS,
     GaitStackClockedTick, GaitStackReset, ServoTorqueTick, SERVO_FORCE_ROWS, FarmColumns, FarmCopy,
+    HEALTH_ROWS, HEALTH_PLAN_OK, HEALTH_PLAN_INFEASIBLE, HEALTH_PLAN_FAILED, HEALTH_BODY_OK, HEALTH_BODY_INFEASIBLE,
+    HEALTH_BODY_FAILED, HEALTH_GRF_OK, HEALTH_GRF_FAILED, HEALTH_GRF_FALLBACK, HEALTH_IK_CAP, HEALTH_NONFINITE, HEALTH_EVENTS,
 )
 from ._build import build  # noqa: F401
 
@@ -25,4 +27,7 @@ __all__ = [
     "STACK_ROW_WALKDTIME", "STACK_ROW_TRAJ", "STACK_ROW_RT",
     "ServoStackTick", "SERVO_TICKS_MAX", "SERVO_STATE_ROWS", "SERVO_ROW_Q", "SERVO_ROW_HOMING", "SERVO_ROW_LPF", "SERVO_LPF_SLOTS",
     "GaitStackClockedTick", "GaitStackReset", "ServoTorqueTick", "SERVO_FORCE_ROWS", "FarmColumns", "FarmCopy",
+    "HEALTH_ROWS", "HEALTH_PLAN_OK", "HEALTH_PLAN_INFEASIBLE", "HEALTH_PLAN_FAILED", "HEALTH_BODY_OK", "HEALTH_BODY_INFEASIBLE",
+    "HEALTH_BODY_FAILED", "HEALTH_GRF_OK", "HEALTH_GRF_FAILED", "HEALTH_GRF_FALLBACK", "HEALTH_IK_CAP", "HEALTH_NONFINITE",
+    "HEALTH_EVENTS",
 ]

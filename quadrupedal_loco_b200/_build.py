@@ -6,7 +6,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgo1mpc.so")
-SOURCES = ["api.cu", "body_mpc.cu", "body_fast.cu", "body_tri.cu", "body_duo.cu", "body_resident.cu", "qp_dense.cu", "step_timing.cu", "step_sqp.cu", "foot_traj.cu", "leg_kin.cu", "grf_qp.cu", "ref_interp.cu", "rt_chain.cu", "nlp_chain.cu", "filters.cu", "peer_gather.cu", "gait_stack.cu", "servo_stack.cu", "servo_torque.cu"]
+SOURCES = ["api.cu", "body_mpc.cu", "body_fast.cu", "body_tri.cu", "body_duo.cu", "body_resident.cu", "qp_dense.cu", "step_timing.cu", "step_sqp.cu", "foot_traj.cu", "leg_kin.cu", "grf_qp.cu", "ref_interp.cu", "rt_chain.cu", "nlp_chain.cu", "filters.cu", "peer_gather.cu", "gait_stack.cu", "servo_stack.cu", "servo_torque.cu", "farm_health.cu"]
 # A/B variants that `auto` never chooses (body_split.cu: roll / pitch halves side by side in one warp) are only compiled
 # into the library with GO1MPC_BUILD_AB=1 (then GO1MPC_BODY_MODE=split selects it)
 AB_SOURCES = ["body_split.cu"]

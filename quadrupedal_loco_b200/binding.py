@@ -36,6 +36,7 @@ EXPORTED_SYMBOLS = [
     "go1mpc_gait_stack_state_doubles", "go1mpc_gait_stack_default_state", "go1mpc_gait_stack_tick_host_async",
     "go1mpc_servo_stack_tick_async", "go1mpc_gait_stack_tick_clocked_async", "go1mpc_gait_stack_reset_async",
     "go1mpc_servo_torque_tick_async", "go1mpc_farm_copy_async",
+    "go1mpc_gait_stack_tick_clocked_health_async", "go1mpc_servo_torque_tick_health_async",
 ]
 
 
@@ -174,6 +175,8 @@ def load_library():
     lib.go1mpc_gait_stack_reset_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackReset), vp]
     lib.go1mpc_servo_torque_tick_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoTorqueTick), vp]
     lib.go1mpc_farm_copy_async.argtypes = [vp, ctypes.POINTER(FarmCopy), vp]
+    lib.go1mpc_gait_stack_tick_clocked_health_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(GaitStackClockedTick), vp, vp]
+    lib.go1mpc_servo_torque_tick_health_async.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ServoTorqueTick), vp, vp]
     _LIB = lib
     return lib
 
@@ -316,10 +319,16 @@ class ServoTorqueTick(ctypes.Structure):
         ("grf_diag_d", ctypes.c_void_p), ("reset_d", ctypes.c_void_p)]
 
 
+# GO1MPC_HEALTH_*: rows of a farm's health counters, int32 [HEALTH_ROWS][B] (see include/go1mpc.h)
+HEALTH_ROWS = 12
+(HEALTH_PLAN_OK, HEALTH_PLAN_INFEASIBLE, HEALTH_PLAN_FAILED, HEALTH_BODY_OK, HEALTH_BODY_INFEASIBLE, HEALTH_BODY_FAILED,
+ HEALTH_GRF_OK, HEALTH_GRF_FAILED, HEALTH_GRF_FALLBACK, HEALTH_IK_CAP, HEALTH_NONFINITE, HEALTH_EVENTS) = range(HEALTH_ROWS)
+
+
 class FarmColumns(ctypes.Structure):
     """Go1FarmColumns of include/go1mpc.h: one farm-shaped buffer set (device)."""
     _fields_ = [("B", ctypes.c_int), ("state_d", ctypes.c_void_p), ("body_out_d", ctypes.c_void_p), ("clock_d", ctypes.c_void_p),
-                ("servo_state_d", ctypes.c_void_p), ("force_state_d", ctypes.c_void_p)]
+                ("servo_state_d", ctypes.c_void_p), ("force_state_d", ctypes.c_void_p), ("health_d", ctypes.c_void_p)]
 
 
 class FarmCopy(ctypes.Structure):
@@ -657,10 +666,15 @@ class Go1Mpc:
         t.sensor_d, t.cmd_d, t.start_d = _ptr(sensor_d), _ptr(cmd_d), _ptr(start_d)
         return t
 
-    def gait_stack_tick_clocked_async(self, B, t, stream=None):
+    def gait_stack_tick_clocked_async(self, B, t, stream=None, health_d=None):
         """go1mpc_gait_stack_tick_clocked_async with a GaitStackClockedTick: each robot plans on its own clock; returns after
-        enqueueing on `stream` (None = the handle's)."""
-        self._check(self.lib.go1mpc_gait_stack_tick_clocked_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_clocked_async")
+        enqueueing on `stream` (None = the handle's).  health_d (device int32 [HEALTH_ROWS][B]) calls
+        go1mpc_gait_stack_tick_clocked_health_async instead, which also updates the farm's health counters."""
+        if health_d is None:
+            self._check(self.lib.go1mpc_gait_stack_tick_clocked_async(self.h, B, ctypes.byref(t), stream), "gait_stack_tick_clocked_async")
+        else:
+            self._check(self.lib.go1mpc_gait_stack_tick_clocked_health_async(self.h, B, ctypes.byref(t), _ptr(health_d), stream),
+                        "gait_stack_tick_clocked_health_async")
 
     def gait_stack_reset_struct(self, nh, reset, clock_d, state_d, body_out_d, servo_state_d=None, servo_q0=None, reset_d=None):
         """Go1GaitStackReset for the given buffers (host reset [B] int32, pinned for graph capture, or reset = None and device
@@ -702,19 +716,25 @@ class Go1Mpc:
                                _ptr(reset), _ptr(tau_d), _ptr(tau), _ptr(grf_d), _ptr(grf_diag_d), _ptr(reset_d))
 
     def servo_torque_tick(self, B, K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d, q_d,
-                          tau_d, stream=None, **kw):
+                          tau_d, stream=None, health_d=None, **kw):
         """go1mpc_servo_torque_tick_async: K 1 kHz servo ticks (filters, leg IK, force distribution, force QP, joint torques) on
         the gait stack state; joint targets into q_d and torques into tau_d, both [B][12 K].  Keyword arguments: q, tau, reset,
-        reset_d, grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.  Returns after enqueueing on `stream` (None = the handle's)."""
+        reset_d, grf_d, grf_diag_d, jac_d, foot_des_d, iters_d.  health_d (device int32 [HEALTH_ROWS][B]) calls
+        go1mpc_servo_torque_tick_health_async instead.  Returns after enqueueing on `stream` (None = the handle's)."""
         t = self.servo_torque_tick_struct(K, gait_mode, y_offset, y_coefficient, stack_state_d, servo_state_d, force_state_d, meas_d,
                                           q_d, tau_d, **kw)
-        self._check(self.lib.go1mpc_servo_torque_tick_async(self.h, B, ctypes.byref(t), stream), "servo_torque_tick_async")
+        if health_d is None:
+            self._check(self.lib.go1mpc_servo_torque_tick_async(self.h, B, ctypes.byref(t), stream), "servo_torque_tick_async")
+        else:
+            self._check(self.lib.go1mpc_servo_torque_tick_health_async(self.h, B, ctypes.byref(t), _ptr(health_d), stream),
+                        "servo_torque_tick_health_async")
 
     # --- farm column copy: whole robots between two farm-shaped buffer sets, picked by a device index ---
     @staticmethod
-    def farm_columns(B, state_d, body_out_d, clock_d=None, servo_state_d=None, force_state_d=None):
+    def farm_columns(B, state_d, body_out_d, clock_d=None, servo_state_d=None, force_state_d=None, health_d=None):
         """FarmColumns for one buffer set (torch CUDA tensors or raw addresses)."""
-        return FarmColumns(int(B), _ptr(state_d), _ptr(body_out_d), _ptr(clock_d), _ptr(servo_state_d), _ptr(force_state_d))
+        return FarmColumns(int(B), _ptr(state_d), _ptr(body_out_d), _ptr(clock_d), _ptr(servo_state_d), _ptr(force_state_d),
+                           _ptr(health_d))
 
     def farm_copy(self, nh, dst, src, index_d, bad_d=None, stream=None):
         """go1mpc_farm_copy_async: destination column i of every given block <- source column index_d[i] (device int32 [dst.B];

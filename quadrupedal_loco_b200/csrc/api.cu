@@ -59,6 +59,8 @@ struct StreamWs {
   DevBuf reset_list;   // go1mpc_gait_stack_reset_async: {count, 3 pad, flags[B], robot list[B]}
   DevBuf copy_list;    // go1mpc_farm_copy_async: {count, 3 pad, destination list[dst.B], source list[dst.B]}
   DevBuf servo_ch, servo_reset;   // go1mpc_servo_torque_tick_async: filtered channels [SERVO_TICKS_MAX][9][B], reset flags [B]
+  // go1mpc_gait_stack_tick_clocked_health_async: the planner's step diag [STEP_DIAG_INTS][B] and the body MPC's diag records
+  struct { DevBuf step_diag, body_diag; } health;
 };
 
 }  // namespace
@@ -370,7 +372,7 @@ ServoStackKParams servo_stack_params(const go1mpc* h, int B, const Tick* t, doub
   P.gait = t->stack_state_d + GO1MPC_STACK_ROW_GAIT * b;
   P.traj = t->stack_state_d + GO1MPC_STACK_ROW_TRAJ * b;
   P.state = t->servo_state_d; P.q_out = t->q_d;
-  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d; P.ch = ch;
+  P.jac = t->jac_d; P.foot_des = t->foot_des_d; P.iters = t->iters_d; P.ch = ch; P.health = nullptr;
   return P;
 }
 
@@ -1231,16 +1233,19 @@ int go1mpc_nlp_node_default_state(go1mpc_t* h, double* s) {
 
 namespace {
 int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
-                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, void* stream);
+                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, int* step_diag_d,
+                     void* stream);
 }
 int go1mpc_nlp_node_tick_batch(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
                                const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, void* stream) {
-  return nlp_node_enqueue(h, B, state_d, walkdtime_d, start_d, cmd_d, rfoot_fb_d, lfoot_fb_d, msg_d, nullptr, stream);
+  return nlp_node_enqueue(h, B, state_d, walkdtime_d, start_d, cmd_d, rfoot_fb_d, lfoot_fb_d, msg_d, nullptr, nullptr, stream);
 }
 namespace {
-// active_d: [B] ints or null (= all); robots with 0 leave the node untouched (per-robot clocks of the gait stack)
+// active_d: [B] ints or null (= all); robots with 0 leave the node untouched (per-robot clocks of the gait stack).
+// step_diag_d: [STEP_DIAG_INTS][B] or null, the planner tick's diag (written only for robots whose node tick is >= 1)
 int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d, const int* start_d, const int* cmd_d,
-                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, void* stream) {
+                     const double* rfoot_fb_d, const double* lfoot_fb_d, double* msg_d, const int* active_d, int* step_diag_d,
+                     void* stream) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B < 0 || !state_d || !walkdtime_d || !msg_d) return fail(h, GO1MPC_E_INVALID, "nlp_node_tick_batch: bad argument");
@@ -1279,7 +1284,7 @@ int nlp_node_enqueue(go1mpc_t* h, int B, double* state_d, const int* walkdtime_d
   CU(h, nlp_pre_launch(P, st));
   h->launches++;
   // the planner state is rows [0, 202) of the node, the swing-foot window rows [202, 234): same SoA stride B
-  rc = step_tick_enqueue(h, 3, B, P.tick, state_d, state_d, P.in, P.out38, nullptr, st, P.hz_co, P.lipm);
+  rc = step_tick_enqueue(h, 3, B, P.tick, state_d, state_d, P.in, P.out38, step_diag_d, st, P.hz_co, P.lipm);
   if (rc) return rc;
   rc = foot_enqueue(h, B, P.tick, state_d, P.out38, state_d + (size_t)STEP_STATE_DOUBLES * B, P.out18, P.right_support, st,
                     state_d + (size_t)kNlpLift0 * B, state_d + (size_t)kNlpStop * B, P.t_end);
@@ -1435,7 +1440,9 @@ bool overlaps_written(const void* in, size_t bytes, std::initializer_list<Block>
 // The node sequence of both gait stack ticks.  clock_d == null: every robot gets t.planner (go1mpc_gait_stack_tick_host_async);
 // otherwise each robot's planner flag comes from its clock (go1mpc_gait_stack_tick_clocked_async), and the planner node is always
 // enqueued, with the robots that do not plan masked out -- the same launches every period, so one captured graph fits all.
-int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock_d, void* stream, const char* name) {
+// health_d (clocked only, else null): the planner and body MPC write their diag into the stream's workspace, and one more kernel
+// after the pack updates the farm's health counters from it.
+int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock_d, int* health_d, void* stream, const char* name) {
   const std::string nm(name);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!t || !t->sensor == !t->sensor_d || !t->state_d || !t->body_out_d || !t->rows_d) return fail(h, GO1MPC_E_INVALID, nm + ": bad argument");
@@ -1465,6 +1472,15 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
     if (overlaps_written(t->sensor_d, b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double), written) ||
         overlaps_written(t->cmd_d, b * sizeof(int), written) || overlaps_written(t->start_d, b * sizeof(int), written))
       return fail(h, GO1MPC_E_INVALID, nm + ": sensor_d / cmd_d / start_d overlap state_d, body_out_d, rows_d or clock_d");
+    if (health_d) {
+      if ((uintptr_t)health_d & 3) return fail(h, GO1MPC_E_INVALID, nm + ": health_d must be 4-byte aligned");
+      if (overlaps_written(health_d, b * GO1MPC_HEALTH_ROWS * sizeof(int),
+                           {{t->state_d, b * go1mpc_gait_stack_state_doubles(nh) * sizeof(double)},
+                            {t->body_out_d, b * go1mpc_body_out_stride(nh) * sizeof(double)}, {t->rows_d, b * n * sizeof(double)},
+                            {clock_d, b * sizeof(int)}, {t->sensor_d, b * GO1MPC_STACK_SENSOR_ROWS * sizeof(double)},
+                            {t->cmd_d, b * sizeof(int)}, {t->start_d, b * sizeof(int)}}))
+        return fail(h, GO1MPC_E_INVALID, nm + ": health_d overlaps state_d, body_out_d, rows_d, clock_d, sensor_d, cmd_d or start_d");
+    }
   }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
@@ -1478,6 +1494,14 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
       (rc = grow(h, ws.cmd, ib, st)) || (rc = grow(h, ws.start, ib, st)) ||
       (rc = grow(h, ws.body_in, b * go1mpc_body_in_stride(nh) * sizeof(double), st)) || (clock_d && (rc = grow(h, ws.plan, ib, st))))
     return rc;
+  int *step_diag = nullptr, *body_diag = nullptr;
+  if (health_d) {
+    if ((rc = grow(h, W->health.step_diag, STEP_DIAG_INTS * ib, st)) ||
+        (rc = grow(h, W->health.body_diag, b * go1mpc_body_diag_stride(nh) * sizeof(int), st)))
+      return rc;
+    step_diag = (int*)W->health.step_diag.p;
+    body_diag = (int*)W->health.body_diag.p;
+  }
   if (fresh) ws.zero_B = -1;
   double* ctl = (double*)ws.ctl_msg.p;
   int* walkdtime = (int*)ws.walkdtime.p;
@@ -1507,13 +1531,21 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
   double* traj = state + GO1MPC_STACK_ROW_TRAJ * b;
   if (planner &&
       (rc = nlp_node_enqueue(h, B, state + GO1MPC_STACK_ROW_NLP * b, walkdtime, start_d, cmd_d, rt2nrt + 22 * b, rt2nrt + 19 * b,
-                             gait, clock_d ? plan_d : nullptr, st)))
+                             gait, clock_d ? plan_d : nullptr, step_diag, st)))
     return rc;
   if ((rc = rt_node_enqueue(h, nh, B, state + GO1MPC_STACK_ROW_RT * b, gait, nullptr, nullptr, ctl, (double*)ws.body_in.p, t->body_out_d,
-                            nullptr, traj, rt2nrt, nullptr, st)))
+                            body_diag, traj, rt2nrt, nullptr, st)))
     return rc;
   CU(h, gait_stack_pack_launch(S, B, gait, traj, t->rows_d, h->sms, st));
   h->launches++;
+  if (health_d) {
+    FarmHealthStackParams H;
+    H.B = B; H.n_slots = n; H.body_diag_stride = go1mpc_body_diag_stride(nh);
+    H.clock = clock_d; H.node_tick = (const int*)W->nlp.tick.p; H.step_diag = step_diag; H.body_diag = body_diag; H.rows = t->rows_d;
+    H.health = health_d;
+    CU(h, farm_health_stack_launch(H, h->sms, st));
+    h->launches++;
+  }
   if (t->rows) CU(h, cudaMemcpyAsync(t->rows, t->rows_d, b * n * sizeof(double), cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
 }
@@ -1522,20 +1554,33 @@ int gait_stack_enqueue(go1mpc_t* h, int B, const Go1GaitStackTick* t, int* clock
 int go1mpc_gait_stack_tick_host_async(go1mpc_t* h, int B, const Go1GaitStackTick* t, void* stream) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
-  return gait_stack_enqueue(h, B, t, nullptr, stream, "gait_stack_tick_host_async");
+  return gait_stack_enqueue(h, B, t, nullptr, nullptr, stream, "gait_stack_tick_host_async");
 }
 
-int go1mpc_gait_stack_tick_clocked_async(go1mpc_t* h, int B, const Go1GaitStackClockedTick* t, void* stream) {
+namespace {
+int gait_stack_clocked_enqueue(go1mpc_t* h, int B, const Go1GaitStackClockedTick* t, int* health_d, void* stream, const char* name) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
-  if (!t || !t->clock_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_clocked_async: bad argument");
+  if (!t || !t->clock_d) return fail(h, GO1MPC_E_INVALID, std::string(name) + ": bad argument");
   Go1GaitStackTick u;
   u.nh = t->nh; u.planner = 0; u.sensor = t->sensor; u.cmd = t->cmd; u.start = t->start; u.state_d = t->state_d;
   u.body_out_d = t->body_out_d; u.n_slots = t->n_slots; u.rows_d = t->rows_d; u.rows = t->rows;
   u.sensor_d = t->sensor_d; u.cmd_d = t->cmd_d; u.start_d = t->start_d;
   memcpy(u.slots, t->slots, sizeof u.slots);
-  return gait_stack_enqueue(h, B, &u, t->clock_d, stream, "gait_stack_tick_clocked_async");
+  return gait_stack_enqueue(h, B, &u, t->clock_d, health_d, stream, name);
+}
+}  // namespace
+
+int go1mpc_gait_stack_tick_clocked_async(go1mpc_t* h, int B, const Go1GaitStackClockedTick* t, void* stream) {
+  return gait_stack_clocked_enqueue(h, B, t, nullptr, stream, "gait_stack_tick_clocked_async");
+}
+
+int go1mpc_gait_stack_tick_clocked_health_async(go1mpc_t* h, int B, const Go1GaitStackClockedTick* t, int* health_d, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (!health_d) return fail(h, GO1MPC_E_INVALID, "gait_stack_tick_clocked_health_async: health_d must be given");
+  return gait_stack_clocked_enqueue(h, B, t, health_d, stream, "gait_stack_tick_clocked_health_async");
 }
 
 int go1mpc_gait_stack_reset_async(go1mpc_t* h, int B, const Go1GaitStackReset* r, void* stream) {
@@ -1594,8 +1639,11 @@ int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
   if (S.B < 1) return fail(h, GO1MPC_E_INVALID, "farm_copy_async: src.B must be at least 1");
   if (!D.state_d || !D.body_out_d || !S.state_d || !S.body_out_d || !c->index_d)
     return fail(h, GO1MPC_E_INVALID, "farm_copy_async: bad argument");
-  if (!D.clock_d != !S.clock_d || !D.servo_state_d != !S.servo_state_d || !D.force_state_d != !S.force_state_d)
-    return fail(h, GO1MPC_E_INVALID, "farm_copy_async: clock_d, servo_state_d and force_state_d must be given on both sides or neither");
+  if (!D.clock_d != !S.clock_d || !D.servo_state_d != !S.servo_state_d || !D.force_state_d != !S.force_state_d ||
+      !D.health_d != !S.health_d)
+    return fail(h, GO1MPC_E_INVALID,
+                "farm_copy_async: clock_d, servo_state_d, force_state_d and health_d must be given on both sides or neither");
+  if (((uintptr_t)D.health_d | (uintptr_t)S.health_d) & 3) return fail(h, GO1MPC_E_INVALID, "farm_copy_async: health_d must be 4-byte aligned");
   if (((uintptr_t)D.body_out_d | (uintptr_t)S.body_out_d) & 15)
     return fail(h, GO1MPC_E_INVALID, "farm_copy_async: body_out_d must be 16-byte aligned");
   const int nh = c->nh;
@@ -1604,16 +1652,16 @@ int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
   // the kernels read the source while they write the destination: no destination block may share a byte with a source block
   auto blocks = [&](const Go1FarmColumns& F, uintptr_t* lo, uintptr_t* hi) {
     const size_t b = (size_t)F.B;
-    const void* p[5] = {F.state_d, F.body_out_d, F.clock_d, F.servo_state_d, F.force_state_d};
-    const size_t n[5] = {b * rows * sizeof(double), b * out_stride * sizeof(double), b * sizeof(int), b * SERVO_STATE_ROWS * sizeof(double),
-                         b * SERVO_FORCE_ROWS * sizeof(double)};
-    for (int k = 0; k < 5; k++) { lo[k] = (uintptr_t)p[k]; hi[k] = p[k] ? lo[k] + n[k] : lo[k]; }
+    const void* p[6] = {F.state_d, F.body_out_d, F.clock_d, F.servo_state_d, F.force_state_d, F.health_d};
+    const size_t n[6] = {b * rows * sizeof(double), b * out_stride * sizeof(double), b * sizeof(int), b * SERVO_STATE_ROWS * sizeof(double),
+                         b * SERVO_FORCE_ROWS * sizeof(double), b * GO1MPC_HEALTH_ROWS * sizeof(int)};
+    for (int k = 0; k < 6; k++) { lo[k] = (uintptr_t)p[k]; hi[k] = p[k] ? lo[k] + n[k] : lo[k]; }
   };
-  uintptr_t dlo[5], dhi[5], slo[5], shi[5];
+  uintptr_t dlo[6], dhi[6], slo[6], shi[6];
   blocks(D, dlo, dhi);
   blocks(S, slo, shi);
-  for (int i = 0; i < 5; i++)
-    for (int k = 0; k < 5; k++)
+  for (int i = 0; i < 6; i++)
+    for (int k = 0; k < 6; k++)
       if (dlo[i] < shi[k] && slo[k] < dhi[i])
         return fail(h, GO1MPC_E_INVALID, "farm_copy_async: a destination block overlaps a source block");
   CU(h, cudaSetDevice(h->device));
@@ -1633,6 +1681,7 @@ int go1mpc_farm_copy_async(go1mpc_t* h, const Go1FarmCopy* c, void* stream) {
   P.src_state = S.state_d; P.src_servo = S.servo_state_d; P.src_force = S.force_state_d;
   P.dst_body = reinterpret_cast<double2*>(D.body_out_d); P.src_body = reinterpret_cast<const double2*>(S.body_out_d);
   P.dst_clock = D.clock_d; P.src_clock = S.clock_d;
+  P.dst_health = D.health_d; P.src_health = S.health_d;
   P.count = (int*)W->copy_list.p; P.dlist = P.count + 4; P.slist = P.count + 4 + D.B;
   CU(h, cudaMemsetAsync(P.count, 0, sizeof(int), st));
   CU(h, farm_copy_launch(P, h->sms, st));
@@ -1662,24 +1711,44 @@ int go1mpc_servo_stack_tick_async(go1mpc_t* h, int B, const Go1ServoStackTick* t
 
 // ------------------------------------------------------------------ servo torque tick: the servo stack + force QP + torque map
 static_assert(GO1MPC_SERVO_FORCE_ROWS == SERVO_FORCE_ROWS, "servo force state layout");
-int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick* t, void* stream) {
+static_assert(GO1MPC_HEALTH_ROWS == FARM_HEALTH_ROWS && GO1MPC_HEALTH_PLAN_OK == FH_PLAN_OK && GO1MPC_HEALTH_PLAN_INFEASIBLE == FH_PLAN_INF &&
+              GO1MPC_HEALTH_PLAN_FAILED == FH_PLAN_FAIL && GO1MPC_HEALTH_BODY_OK == FH_BODY_OK && GO1MPC_HEALTH_BODY_INFEASIBLE == FH_BODY_INF &&
+              GO1MPC_HEALTH_BODY_FAILED == FH_BODY_FAIL && GO1MPC_HEALTH_GRF_OK == FH_GRF_OK && GO1MPC_HEALTH_GRF_FAILED == FH_GRF_FAIL &&
+              GO1MPC_HEALTH_GRF_FALLBACK == FH_GRF_FALLBACK && GO1MPC_HEALTH_IK_CAP == FH_IK_CAP && GO1MPC_HEALTH_NONFINITE == FH_NONFINITE &&
+              GO1MPC_HEALTH_EVENTS == FH_EVENTS && GO1MPC_QP_OK == 0 && GO1MPC_QP_INFEASIBLE == 2, "farm health rows");
+namespace {
+// health_d: null, or the farm's health counters, which the health instantiations of both kernels update
+int servo_torque_enqueue(go1mpc_t* h, int B, const Go1ServoTorqueTick* t, int* health_d, void* stream, const char* name) {
   if (!h) return GO1MPC_E_INVALID;
   std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  const std::string nm(name);
   if (B <= 0) return B == 0 ? GO1MPC_OK : GO1MPC_E_INVALID;
   if (!t || !t->stack_state_d || !t->servo_state_d || !t->q_d || !t->force_state_d || !t->meas_d || !t->tau_d)
-    return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: bad argument");
-  if (t->K < 1 || t->K > GO1MPC_SERVO_TICKS_MAX) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: 1 <= K <= 10");
+    return fail(h, GO1MPC_E_INVALID, nm + ": bad argument");
+  if (t->K < 1 || t->K > GO1MPC_SERVO_TICKS_MAX) return fail(h, GO1MPC_E_INVALID, nm + ": 1 <= K <= 10");
   if (((uintptr_t)t->q_d | (uintptr_t)t->tau_d) & 7)
-    return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: q_d and tau_d must be 8-byte aligned");
-  if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, "servo_torque_tick_async: gait_mode 101, 102 or 103");
-  if (t->reset && t->reset_d) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: at most one of reset / reset_d");
-  if ((uintptr_t)t->reset_d & 3) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: reset_d must be 4-byte aligned");
+    return fail(h, GO1MPC_E_INVALID, nm + ": q_d and tau_d must be 8-byte aligned");
+  if (t->gait_mode < 101 || t->gait_mode > 103) return fail(h, GO1MPC_E_UNSUPPORTED, nm + ": gait_mode 101, 102 or 103");
+  if (t->reset && t->reset_d) return fail(h, GO1MPC_E_INVALID, nm + ": at most one of reset / reset_d");
+  if ((uintptr_t)t->reset_d & 3) return fail(h, GO1MPC_E_INVALID, nm + ": reset_d must be 4-byte aligned");
   {
     const size_t b = (size_t)B, kb = b * 12 * t->K * sizeof(double);
     if (overlaps_written(t->reset_d, b * sizeof(int),
                          {{t->force_state_d, b * SERVO_FORCE_ROWS * sizeof(double)}, {t->servo_state_d, b * SERVO_STATE_ROWS * sizeof(double)},
                           {t->q_d, kb}, {t->tau_d, kb}}))
-      return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_async: reset_d overlaps force_state_d, servo_state_d, q_d or tau_d");
+      return fail(h, GO1MPC_E_INVALID, nm + ": reset_d overlaps force_state_d, servo_state_d, q_d or tau_d");
+    if (health_d) {
+      if ((uintptr_t)health_d & 3) return fail(h, GO1MPC_E_INVALID, nm + ": health_d must be 4-byte aligned");
+      // the stack state's size depends on nh, which this call does not take: its rows before the 100 Hz node's are checked
+      if (overlaps_written(health_d, b * GO1MPC_HEALTH_ROWS * sizeof(int),
+                           {{t->stack_state_d, b * GO1MPC_STACK_ROW_RT * sizeof(double)},
+                            {t->servo_state_d, b * SERVO_STATE_ROWS * sizeof(double)},
+                            {t->force_state_d, b * SERVO_FORCE_ROWS * sizeof(double)}, {t->meas_d, b * SERVO_MEAS_ROWS * sizeof(double)},
+                            {t->q_d, kb}, {t->tau_d, kb}, {t->reset_d, b * sizeof(int)},
+                            {t->grf_d, b * GRF_OUT_DOUBLES * sizeof(double)}, {t->grf_diag_d, b * GRF_DIAG_INTS * sizeof(int)},
+                            {t->jac_d, b * 36 * sizeof(double)}, {t->foot_des_d, b * 12 * sizeof(double)}, {t->iters_d, b * 4 * sizeof(int)}}))
+        return fail(h, GO1MPC_E_INVALID, nm + ": health_d overlaps a block the call reads or writes");
+    }
   }
   CU(h, cudaSetDevice(h->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
@@ -1692,7 +1761,8 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
       (t->reset && (rc = grow(h, W->servo_reset, rb, st))))
     return rc;
   void* rst = t->reset ? W->servo_reset.p : nullptr;
-  const ServoStackKParams S = servo_stack_params(h, B, t, (double*)W->servo_ch.p);
+  ServoStackKParams S = servo_stack_params(h, B, t, (double*)W->servo_ch.p);
+  S.health = health_d;
   ServoTorqueKParams P;
   P.g = grf_params(h, B, nullptr, nullptr, nullptr);
   P.B = B; P.K = t->K; P.gait_mode = t->gait_mode;
@@ -1700,7 +1770,7 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
   P.swing_kp = kSwingKp; P.swing_kd = kSwingKd;
   P.gait = S.gait; P.traj = S.traj; P.homing = t->servo_state_d + SERVO_ROW_HOMING * b; P.ch = S.ch; P.q = t->q_d;
   P.meas = t->meas_d; P.reset = t->reset_d ? t->reset_d : (const int*)rst; P.force = t->force_state_d; P.tau = t->tau_d;
-  P.grf = t->grf_d; P.grf_diag = t->grf_diag_d;
+  P.grf = t->grf_d; P.grf_diag = t->grf_diag_d; P.health = health_d;
   if (rst) CU(h, cudaMemcpyAsync(rst, t->reset, rb, cudaMemcpyHostToDevice, st));
   CU(h, servo_stack_launch(S, st));
   h->launches++;
@@ -1710,6 +1780,18 @@ int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick*
   if (t->q) CU(h, cudaMemcpyAsync(t->q, t->q_d, kb, cudaMemcpyDeviceToHost, st));
   if (t->tau) CU(h, cudaMemcpyAsync(t->tau, t->tau_d, kb, cudaMemcpyDeviceToHost, st));
   return GO1MPC_OK;
+}
+}  // namespace
+
+int go1mpc_servo_torque_tick_async(go1mpc_t* h, int B, const Go1ServoTorqueTick* t, void* stream) {
+  return servo_torque_enqueue(h, B, t, nullptr, stream, "servo_torque_tick_async");
+}
+
+int go1mpc_servo_torque_tick_health_async(go1mpc_t* h, int B, const Go1ServoTorqueTick* t, int* health_d, void* stream) {
+  if (!h) return GO1MPC_E_INVALID;
+  std::lock_guard<std::recursive_mutex> lk_(h->mu);
+  if (!health_d) return fail(h, GO1MPC_E_INVALID, "servo_torque_tick_health_async: health_d must be given");
+  return servo_torque_enqueue(h, B, t, health_d, stream, "servo_torque_tick_health_async");
 }
 
 // ------------------------------------------------------------------ pipelined host entries

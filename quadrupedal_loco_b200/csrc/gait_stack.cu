@@ -9,6 +9,7 @@
 //                            call, into a mask the planner node reads; walkdtime += 1 for those robots; clock += 1; the sensor scatter
 //   gait_stack_reset_mark_kernel / gait_stack_reset_column_kernel : robot resets, see below
 //   farm_copy_list_kernel / farm_copy_column_kernel : whole robot columns copied between two farms (go1mpc_farm_copy_async)
+//                            (the health rows of farm_health.cu travel with the clock, in the list kernel)
 // Thread per robot (pre) / per output double (pack): every warp access is coalesced over B.
 #include "kernels.h"
 
@@ -114,7 +115,7 @@ __global__ void __launch_bounds__(256) gait_stack_reset_column_kernel(StackReset
 }
 
 // ---- farm column copy.  Thread per destination column: the columns with a valid source are listed with one atomic per warp, with
-// their source beside them, and get their clock here.  Entries outside -1..src_B-1 are counted (one atomic per warp) and never read
+// their source beside them, and get their clock and health counters here.  Entries outside -1..src_B-1 are counted (one atomic per warp) and never read
 // through.  Every lane reaches the ballots: lanes past dst_B hold -1.
 __global__ void __launch_bounds__(256) farm_copy_list_kernel(FarmCopyParams P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -129,6 +130,10 @@ __global__ void __launch_bounds__(256) farm_copy_list_kernel(FarmCopyParams P) {
   P.dlist[slot] = i;
   P.slist[slot] = s;
   if (P.dst_clock) P.dst_clock[i] = P.src_clock[s];
+  if (P.dst_health) {
+#pragma unroll
+    for (int r = 0; r < FARM_HEALTH_ROWS; r++) P.dst_health[(size_t)r * P.dst_B + i] = P.src_health[(size_t)r * P.src_B + s];
+  }
 }
 
 constexpr int FARM_TASK_ROWS = 32;   // SoA rows per warp task

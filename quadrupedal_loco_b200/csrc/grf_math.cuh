@@ -75,10 +75,14 @@ __device__ __forceinline__ void grf_ci_build(double* CI, double fz_max, double m
   __syncthreads();
 }
 
+// What one force QP ended with, in registers on every lane: its status (diag word 0) and whether x held a NaN, so that the
+// closed-form guess was returned (diag word 6 = 0)
+struct GrfQpOutcome { int status; bool nan; };
+
 // force_opt (:265-373) + solve_grf_opt (:387-427) for one robot, one warp.  recs: the robot's 48-double record in the layout of
 // GrfKParams::in (shared memory); A (6 x 12), g0, CE, ce0: the warp's scratch; w: its QP workspace.  Writes out[0..16) in
-// GrfKParams::out's layout and, when dg is non-null, the 32 diagnostic ints.
-__device__ __forceinline__ void grf_force_opt_warp(const GrfKParams& P, const double* CI, const GiWs& w, double* A, double* g0,
+// GrfKParams::out's layout and, when dg is non-null, the 32 diagnostic ints; returns the outcome.
+__device__ __forceinline__ GrfQpOutcome grf_force_opt_warp(const GrfKParams& P, const double* CI, const GiWs& w, double* A, double* g0,
                                                    double* CE, double* ce0, const double* recs, double* out, int* dg, int lane) {
   const double* ci0 = CI + GN * GM;
   auto field = [&](int k) -> double { return recs[k]; };
@@ -153,6 +157,7 @@ __device__ __forceinline__ void grf_force_opt_warp(const GrfKParams& P, const do
     if (lane == 0) { dg[0] = res.status; dg[1] = pd ? res.iq : 0; dg[2] = res.it_outer; dg[3] = res.it_add; dg[4] = res.it_drop; dg[5] = res.it_degen; dg[6] = nan ? 0 : 1; dg[7] = 0; }
     if (lane < 24) dg[8 + lane] = (pd && lane < res.iq) ? w.A[lane] : -99;
   }
+  return GrfQpOutcome{res.status, nan};
 }
 
 // force_distribution (:141-261) for one robot: com [3], leg [12] (FR, FL, RR, RL xyz), F [6] (L xyz, R xyz), rf / lf [3]

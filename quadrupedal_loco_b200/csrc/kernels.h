@@ -276,6 +276,22 @@ struct StackResetParams {
   int* list;                  // [B]
 };
 cudaError_t gait_stack_reset_launch(const StackResetParams& P, int sms, cudaStream_t st);
+// farm health counters (farm_health.cu): int [FARM_HEALTH_ROWS][B] per farm, rows as GO1MPC_HEALTH_* of include/go1mpc.h
+constexpr int FARM_HEALTH_ROWS = 12;
+enum { FH_PLAN_OK = 0, FH_PLAN_INF = 1, FH_PLAN_FAIL = 2, FH_BODY_OK = 3, FH_BODY_INF = 4, FH_BODY_FAIL = 5, FH_GRF_OK = 6,
+       FH_GRF_FAIL = 7, FH_GRF_FALLBACK = 8, FH_IK_CAP = 9, FH_NONFINITE = 10, FH_EVENTS = 11 };
+// After a clocked gait stack tick: per robot, restart at clock 0 (clock after the call == 1), count the planner statuses of the
+// robots whose node tick is >= 1, the body status, a non-finite rows_d row, and overwrite EVENTS
+struct FarmHealthStackParams {
+  int B, n_slots, body_diag_stride;
+  const int* clock;           // [B] after the call
+  const int* node_tick;       // [B] the planner node's tick index of this call (0: no planner tick)
+  const int* step_diag;       // [STEP_DIAG_INTS][B]
+  const int* body_diag;       // [B][body_diag_stride]
+  const double* rows;         // [B][n_slots]
+  int* health;                // [FARM_HEALTH_ROWS][B]
+};
+cudaError_t farm_health_stack_launch(const FarmHealthStackParams& P, int sms, cudaStream_t st);
 // farm column copy: ws = {count, 3 pad, dst list[dst_B], src list[dst_B]} ints, count zero on entry.  The list kernel lists the
 // destinations with a valid index and copies their clocks; the column kernel copies the listed columns' SoA rows (state | servo |
 // force as one row range) and body records
@@ -293,6 +309,8 @@ struct FarmCopyParams {
   const int* src_clock;
   int* count;
   int *dlist, *slist;               // [dst_B]
+  int* dst_health;                  // [FARM_HEALTH_ROWS][dst_B] or null (then src_health too): copied by the list kernel
+  const int* src_health;            // [FARM_HEALTH_ROWS][src_B]
 };
 cudaError_t farm_copy_launch(const FarmCopyParams& P, int sms, cudaStream_t st);
 
@@ -311,6 +329,7 @@ struct ServoStackKParams {
   double* foot_des;             // [12][B] or null (last tick)
   int* iters;                   // [4][B] or null (last tick)
   double* ch;                   // [K][9][B] or null: each tick's filtered channels
+  int* health;                  // [FARM_HEALTH_ROWS][B] or null: IK_CAP and EVENTS (servo_stack_kernel<true, true> only)
 };
 cudaError_t servo_stack_launch(const ServoStackKParams& P, cudaStream_t st);
 
@@ -331,6 +350,7 @@ struct ServoTorqueKParams {
   double* tau;                  // [B][12 K]
   double* grf;                  // [B][16] or null (last tick)
   int* grf_diag;                // [B][32] or null (last tick)
+  int* health;                  // [FARM_HEALTH_ROWS][B] or null: force-QP rows, NONFINITE and EVENTS (servo_torque_kernel<4, true>)
 };
 cudaError_t servo_torque_launch(ServoTorqueKParams P, int sms, cudaStream_t st);
 

@@ -19,8 +19,10 @@ namespace {
 __device__ __forceinline__ constexpr int lpf_slot(int c) { return c < 3 ? c : c + 3; }
 }  // namespace
 
-// CH: also store each tick's nine filtered channels to P.ch [K][9][B] (the servo torque tick's second kernel reads them)
-template <bool CH>
+// CH: also store each tick's nine filtered channels to P.ch [K][9][B] (the servo torque tick's second kernel reads them).
+// H: also count the leg-ticks whose IK applied all 15 updates into the robot's health row FH_IK_CAP (the group's four legs summed
+// by shuffle, lane 0 of the group writes) and mark the row in FH_EVENTS.
+template <bool CH, bool H = false>
 __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const size_t B = (size_t)P.B;
@@ -60,7 +62,7 @@ __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
 
   double* qo = P.q_out + b * (size_t)(12 * P.K) + 3 * leg;
   double pdes[3], J[9];
-  int it = 0;
+  int it = 0, capped = 0;
   for (int k = 0; k < P.K; k++) {
     double f[3];
 #pragma unroll
@@ -77,6 +79,7 @@ __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
     const double vf[3] = {right ? ch[6] : ch[3], right ? ch[7] : ch[4], right ? ch[8] : ch[5]};
     servo_leg_target(hom, vf, right, P.half_hip_width, pdes);
     it = servo_leg_ik(lc, bd, pdes, q, J);
+    if constexpr (H) capped += (it == 15);
     qo[12 * k] = q[0]; qo[12 * k + 1] = q[1]; qo[12 * k + 2] = q[2];
   }
 
@@ -93,11 +96,20 @@ __global__ void __launch_bounds__(256) servo_stack_kernel(ServoStackKParams P) {
   if (P.jac) for (int k = 0; k < 9; k++) P.jac[(size_t)(9 * leg + k) * B + b] = J[k];
   if (P.foot_des) for (int k = 0; k < 3; k++) P.foot_des[(size_t)(3 * leg + k) * B + b] = pdes[k];
   if (P.iters) P.iters[(size_t)leg * B + b] = it;
+  if constexpr (H) {
+    capped += __shfl_xor_sync(live, capped, 1, 4);
+    capped += __shfl_xor_sync(live, capped, 2, 4);
+    if (leg == 0 && capped) {
+      P.health[(size_t)FH_IK_CAP * B + b] += capped;
+      P.health[(size_t)FH_EVENTS * B + b] |= 1 << FH_IK_CAP;
+    }
+  }
 }
 
 cudaError_t servo_stack_launch(const ServoStackKParams& P, cudaStream_t st) {
   const size_t threads = 4 * (size_t)P.B;
-  if (P.ch) servo_stack_kernel<true><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
+  if (P.health) servo_stack_kernel<true, true><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
+  else if (P.ch) servo_stack_kernel<true><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
   else servo_stack_kernel<false><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(P);
   return cudaGetLastError();
 }

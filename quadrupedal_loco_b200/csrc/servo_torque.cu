@@ -19,8 +19,10 @@ constexpr int TQ_EXTRA = GRF_OUT_DOUBLES + 36 + 12 + 12 + 12 + 12 + 36 + 9 + 6 +
 }
 
 // The per-call leg data lives in shared memory, not in registers across the QP, so that 4 CTAs (16 warps) fit an SM without
-// spills: the QP is latency-bound and wants as many warps per SM as the registers allow
-template <int WPC>
+// spills: the QP is latency-bound and wants as many warps per SM as the registers allow.
+// H: also count, per tick, the force QP's outcome (FH_GRF_OK / FH_GRF_FAILED, FH_GRF_FALLBACK on a NaN solution) and a non-finite
+// q or tau of the robot (FH_NONFINITE) in registers of lane 0, which adds them to the health rows and ORs FH_EVENTS once per robot.
+template <int WPC, bool H = false>
 __global__ void __launch_bounds__(WPC * 32, 4) servo_torque_kernel(ServoTorqueKParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* smem = reinterpret_cast<double*>(smem_raw);
@@ -78,7 +80,9 @@ __global__ void __launch_bounds__(WPC * 32, 4) servo_torque_kernel(ServoTorqueKP
     }
     if (lane < 6) Fd[lane] = G[(size_t)(15 + lane) * B];
     __syncwarp();
+    int n_ok = 0, n_fail = 0, n_fallback = 0, n_nonfinite = 0;   // H only
     for (int k = 0; k < K; k++) {
+      bool nonfinite = false;                                   // H only: this tick's q or tau of the robot
       double ch[SERVO_LPF_CHANNELS];
       if (lane < 4) {
 #pragma unroll
@@ -94,6 +98,7 @@ __global__ void __launch_bounds__(WPC * 32, 4) servo_torque_kernel(ServoTorqueKP
         servo_leg_target(hom, vf, right, P.half_hip_width, pdes);
         const double* qk = P.q + b * (size_t)(12 * K) + 12 * k + 3 * leg;
         const double qq[3] = {qk[0], qk[1], qk[2]};
+        if constexpr (H) nonfinite = !isfinite(qq[0]) || !isfinite(qq[1]) || !isfinite(qq[2]);
         fk_any(qq, lc, bd, pos, J);
         for (int j = 0; j < 9; j++) Jq[9 * leg + j] = J[j];
         fk_any(qm, lc, bd, pos, J);
@@ -114,8 +119,13 @@ __global__ void __launch_bounds__(WPC * 32, 4) servo_torque_kernel(ServoTorqueKP
       __syncwarp();
       if (lane < 12) recs[21 + lane] = fref[lane];            // F_leg_guess
       __syncwarp();
-      grf_force_opt_warp(P.g, CI, w, A, g0, CE, ce0, recs, out, (k == K - 1 && P.grf_diag) ? P.grf_diag + b * GRF_DIAG_INTS : nullptr,
-                         lane);
+      const GrfQpOutcome qo = grf_force_opt_warp(P.g, CI, w, A, g0, CE, ce0, recs, out,
+                                                 (k == K - 1 && P.grf_diag) ? P.grf_diag + b * GRF_DIAG_INTS : nullptr, lane);
+      if constexpr (H) {
+        n_ok += qo.status == ST_OK;
+        n_fail += qo.status != ST_OK;
+        n_fallback += qo.nan;
+      }
       __syncwarp();
       if (lane < 12) {
         const int l = lane / 3, i = lane - 3 * l;
@@ -126,10 +136,24 @@ __global__ void __launch_bounds__(WPC * 32, 4) servo_torque_kernel(ServoTorqueKP
           wv[r] = sw ? grf_swing_w(P.swing_kp, P.swing_kd, recs[3 + e], pest[e], pvdes[e], pvest[e]) : out[e];
           jc[r] = Jq[9 * l + 3 * r + i];
         }
-        P.tau[b * (size_t)(12 * K) + 12 * k + lane] = grf_tau(l, i, jc, wv);
+        const double tq = grf_tau(l, i, jc, wv);
+        P.tau[b * (size_t)(12 * K) + 12 * k + lane] = tq;
+        if constexpr (H) nonfinite = nonfinite || !isfinite(tq);
         recs[33 + lane] = out[lane];                          // grf_opt -> the next tick's previous solution
       }
+      if constexpr (H) n_nonfinite += __any_sync(FULL_MASK, nonfinite) ? 1 : 0;
       __syncwarp();
+    }
+    if constexpr (H) {
+      if (lane == 0) {
+        const int add[4] = {n_ok, n_fail, n_fallback, n_nonfinite};
+        const int row[4] = {FH_GRF_OK, FH_GRF_FAIL, FH_GRF_FALLBACK, FH_NONFINITE};
+        int ev = 0;
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+          if (add[j]) { P.health[(size_t)row[j] * B + b] += add[j]; ev |= 1 << row[j]; }
+        if (ev) P.health[(size_t)FH_EVENTS * B + b] |= ev;
+      }
     }
     if (lane < 12) {
       P.force[(size_t)lane * B + b] = recs[33 + lane];
@@ -144,13 +168,14 @@ cudaError_t servo_torque_launch(ServoTorqueKParams P, int sms, cudaStream_t st) 
   constexpr int WPC = 4;
   P.g.warp_doubles = grf_warp_doubles() + TQ_EXTRA;
   const size_t smem = (size_t)(GN * GM + GM + WPC * P.g.warp_doubles) * sizeof(double);
-  cudaError_t e = cudaFuncSetAttribute(servo_torque_kernel<WPC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  auto kern = P.health ? servo_torque_kernel<WPC, true> : servo_torque_kernel<WPC>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   int per_sm = 0;
-  if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, servo_torque_kernel<WPC>, WPC * 32, smem)) != cudaSuccess) return e;
+  if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WPC * 32, smem)) != cudaSuccess) return e;
   int grid = (P.B + WPC - 1) / WPC;                 // one wave of resident CTAs, grid-stride over the robots
   if (grid > sms * per_sm) grid = sms * per_sm;
-  servo_torque_kernel<WPC><<<grid, WPC * 32, smem, st>>>(P);
+  kern<<<grid, WPC * 32, smem, st>>>(P);
   return cudaGetLastError();
 }
 
